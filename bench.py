@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: fused gray -> 5x5 Gaussian -> Sobel on 4K RGB frames.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--no-extras]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--no-extras] [--dump-outputs DIR]
 
 One process per GPU (the driver launches N > 1 with torch.distributed.run).  Frames are
 independent, so each rank owns whole frames (BASELINE config 4: 256 frames of 3840x2160 RGB8 over 8
@@ -23,6 +23,9 @@ the informational keys (so nothing spins in an NCCL barrier while the CPU oracle
             a 16-frame batch sharded over the same N devices (rip_process_host), and the resident kernel
   e2e_nv12  the end-to-end leg with NV12 input (1.5 B/px in instead of 3)
   cpu_baseline  the oracle on the headline workload, all host threads, bounded sample
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs), so that two builds can be compared
+output for output: the inputs are seeded and the same from run to run.
 """
 from __future__ import annotations
 
@@ -39,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only and is left as it was: no __pycache__ from this run
 
 W, H, CN = 3840, 2160, 3
 FRAMES_PER_GPU = 32
@@ -46,6 +50,7 @@ KSIZE, SIGMA = 5, 1.0
 ALGO_BYTES_PER_PX = 4  # 3 in (RGB8) + 1 out (u8)   -- SURVEY.md 8(d)
 WORKLOAD = (f"fused gray->gauss{KSIZE}x{KSIZE}(sigma={SIGMA})->sobel, synthetic RGB8 {W}x{H}, "
             f"{FRAMES_PER_GPU} frames per GPU per step (BASELINE config 4 shard: 256 frames over 8 GPUs)")
+DUMP_ROWS = 64  # rows per frame in --dump-outputs: 32 frames x 64 rows x 3840 px in float32 = 31.5 MB
 
 
 def synth_batch(n: int, seed0: int) -> np.ndarray:
@@ -54,6 +59,18 @@ def synth_batch(n: int, seed0: int) -> np.ndarray:
     for i in range(n):
         out[i] = np.random.default_rng(seed0 + i).integers(0, 256, (H, W, CN), dtype=np.uint8)
     return out
+
+
+def dump_outputs(path: str, out: np.ndarray) -> None:
+    """Write the fused output of the last timed step, (N, H, W) u8 as the caller receives it, to path/fused_rows.npy
+    in float32.  A whole step is 265 MB of u8, so the file holds a fixed sample: the same DUMP_ROWS rows of every
+    frame, namely the three top and three bottom rows (where the 5x5 blur and the Sobel clamp to the border) and rows
+    drawn with a fixed seed."""
+    h = out.shape[1]
+    inner = np.random.default_rng(0xB200 + 99).choice(np.arange(3, h - 3), DUMP_ROWS - 6, replace=False)
+    rows = np.sort(np.concatenate([[0, 1, 2, h - 3, h - 2, h - 1], inner]))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "fused_rows.npy"), out[:, rows].astype(np.float32))
 
 
 def content_frame(kind: str, h: int = H, w: int = W) -> np.ndarray:
@@ -207,9 +224,10 @@ def run_reference(args, rank: int) -> None:
         O.fused(frames[0], KSIZE, weights=w, threads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        for i in range(per_step):
-            O.fused(frames[i], KSIZE, weights=w, threads=cores)
+        outs = [O.fused(frames[i], KSIZE, weights=w, threads=cores) for i in range(per_step)]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.stack(outs))
     mpx = args.steps * per_step * W * H / dt / 1e6
     line = {"impl": "reference", "metric": "fused_4k_throughput", "value": mpx, "unit": "Mpixel/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True,
@@ -403,8 +421,13 @@ def main() -> None:
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline + e2e legs only (no content / configs / config5 keys)")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer leg (default: min(steps, 10))")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer legs (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the last step's output as DIR/fused_rows.npy "
+                         "(float32; rank 0's frames when there are several ranks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -488,10 +511,12 @@ def main() -> None:
 
     # correctness spot check outside the timed region: first frame of the resident output vs oracle
     out0 = d_out.download((H, W))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out.download((n, H, W)))
 
     # ---- end-to-end leg: public host-buffer API, pinned host frames, H2D + kernel + D2H per step ----
     ctx = rip.Context([dev])
-    e2e_steps = args.e2e_steps or min(args.steps, 10)
+    e2e_steps = args.e2e_steps or args.steps
     out_host = pin_out.array.reshape(n, H, W)
     for _ in range(2):
         ctx.process(frames, rip.OP_FUSED, rip.FMT_RGB8, ksize=KSIZE, weights=weights, out=out_host)
