@@ -143,17 +143,19 @@ int rip_gauss(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out
 int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int in_format);
 
-/* Fused gray -> K x K Gaussian -> Sobel, one HBM round trip per frame (ksize 5; other sizes run the
- * three stages through d_workspace).  Processes output rows [out_row0, out_row0 + out_rows) of
+/* Fused gray -> K x K Gaussian -> Sobel in one kernel, one HBM round trip per frame, for every
+ * shape and kernel size.  Processes output rows [out_row0, out_row0 + out_rows) of
  * frames whose true height is `height`; d_in holds input rows [in_row0, in_row0 + in_rows) of each
  * frame (a row band with halo: it must cover out rows extended by ksize/2 + 1 rows each side, clipped to
  * the image).  For whole frames pass in_row0 = out_row0 = 0 and in_rows = out_rows = height.
- * d_out holds out_rows * width bytes per frame. */
+ * d_out holds out_rows * width bytes per frame.  d_workspace and workspace_bytes are unused (pass
+ * NULL, 0); they stay in the signature for ABI compatibility. */
 int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int in_format, int ksize, const float *weights,
               int in_row0, int in_rows, int out_row0, int out_rows, void *d_workspace,
               size_t workspace_bytes);
-/* bytes of d_workspace rip_fused needs for this shape (0 on the single-kernel path) */
+/* bytes of d_workspace rip_fused needs for this shape: always 0 (rip_fused needs no workspace);
+ * still rejects a non-positive shape */
 int rip_fused_workspace_bytes(int width, int in_rows, int n_frames, int ksize, size_t *bytes);
 
 /* counters: kernels launched by this library in this process (all threads) */
@@ -167,7 +169,7 @@ int rip_debug_slow_path_stats(int device, int enable, uint64_t *slow_pixels);
  * triples) against the plain exact formulations.  mismatches must come back 0. */
 int rip_debug_selftest(int device, uint64_t *checked, uint64_t *mismatches);
 /* diagnostics: experiment switches (kernel selection for A/B runs and for the tests that compare kernels).  They are
- * read from the environment once, at first use (RIP_DISABLE_FUSED, RIP_FUSED_SEG, RIP_FUSED_NPX, RIP_FUSED_GENERIC,
+ * read from the environment once, at first use (RIP_FUSED_SEG, RIP_FUSED_NPX, RIP_FUSED_GENERIC,
  * RIP_BLUR_EXACT, RIP_BLUR_TILED, RIP_BLUR_STREAM); afterwards only this call changes them, so no launch path calls
  * getenv().  `name` is the variable name with or without the RIP_ prefix.  The reference has no counterpart (its
  * switches are file-scope globals, RealtimeImageProcessing.cpp:10-30). */

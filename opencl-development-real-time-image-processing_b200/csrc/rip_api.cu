@@ -50,9 +50,8 @@ void count_launch(uint64_t n) { g_launches.fetch_add(n, std::memory_order_relaxe
 static Options g_options;
 static std::once_flag g_options_once;
 static const struct { const char *name; int Options::*field; } kOptionTable[] = {
-    {"RIP_DISABLE_FUSED", &Options::disable_fused}, {"RIP_FUSED_SEG", &Options::fused_seg}, {"RIP_FUSED_NPX", &Options::fused_npx},
-    {"RIP_FUSED_GENERIC", &Options::fused_generic}, {"RIP_FUSED_STAGED", &Options::fused_staged}, {"RIP_BLUR_EXACT", &Options::blur_exact}, {"RIP_BLUR_TILED", &Options::blur_tiled},
-    {"RIP_BLUR_STREAM", &Options::blur_stream},
+    {"RIP_FUSED_SEG", &Options::fused_seg}, {"RIP_FUSED_NPX", &Options::fused_npx}, {"RIP_FUSED_GENERIC", &Options::fused_generic},
+    {"RIP_BLUR_EXACT", &Options::blur_exact}, {"RIP_BLUR_TILED", &Options::blur_tiled}, {"RIP_BLUR_STREAM", &Options::blur_stream},
 };
 
 static void load_options_from_env()
@@ -137,8 +136,8 @@ struct Part;
 
 struct BufSet {
     cudaStream_t stream = nullptr;
-    void *d_in = nullptr, *d_out = nullptr, *d_ws = nullptr;
-    size_t in_cap = 0, out_cap = 0, ws_cap = 0;
+    void *d_in = nullptr, *d_out = nullptr;
+    size_t in_cap = 0, out_cap = 0;
     // pinned staging for callers that hand in pageable memory (std::vector, cv::Mat): allocated on first need
     void *stage_in = nullptr, *stage_out = nullptr;
     size_t stage_in_cap = 0, stage_out_cap = 0;
@@ -377,7 +376,6 @@ extern "C" int rip_ctx_destroy(rip_ctx *ctx)
             }
             if (b.d_in) cudaFree(b.d_in);
             if (b.d_out) cudaFree(b.d_out);
-            if (b.d_ws) cudaFree(b.d_ws);
             if (b.stage_in) cudaFreeHost(b.stage_in);
             if (b.stage_out) cudaFreeHost(b.stage_out);
             for (int j = 0; j < 4; j++)
@@ -695,20 +693,18 @@ extern "C" int rip_fused_workspace_bytes(int width, int in_rows, int n_frames, i
 {
     if (!bytes) return fail(RIP_EINVAL, "rip_fused_workspace_bytes: NULL");
     if (width <= 0 || in_rows <= 0 || n_frames <= 0) return fail(RIP_EINVAL, "rip_fused_workspace_bytes: bad shape");
-    // staged path (any ksize but 5, or shapes the single-kernel path rejects): gray band + blurred band
     (void)ksize;
-    *bytes = (size_t)2 * width * in_rows * n_frames;
+    *bytes = 0;   // every shape and kernel size runs as a single kernel
     return RIP_OK;
 }
 
 extern "C" int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
                          int n_frames, int in_format, int ksize, const float *weights, int in_row0, int in_rows,
-                         int out_row0, int out_rows, void *d_workspace, size_t workspace_bytes)
+                         int out_row0, int out_rows, void * /* d_workspace: unused */, size_t /* workspace_bytes: unused */)
 {
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_fused", d_in, d_out, width, height, n_frames)) return rc;
-    const int cn = channels_of(in_format);
-    if (cn == 0) return fail(RIP_EINVAL, "rip_fused: unsupported input format %d", in_format);
+    if (channels_of(in_format) == 0) return fail(RIP_EINVAL, "rip_fused: unsupported input format %d", in_format);
     Weights wts;
     if (int rc = load_weights(wts, ksize, weights, "rip_fused")) return rc;
     const int half = ksize / 2;
@@ -728,26 +724,8 @@ extern "C" int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uin
         if (ksize == 5 && !options().fused_generic && fused_supported(width, height, in_format, 5, d_in, d_out) && fused_plan_weights(wts.w, g3, &thr))
             return launch_fused(s, d_in, d_out, width, height, n_frames, in_format, true, wts.w, in_row0, in_rows, out_row0, out_rows, device);
     }
-    // every other shape, kernel size and weight set: still one kernel (no workspace), the reference's arithmetic throughout
-    if (!options().fused_staged)
-        return launch_fused_tile(s, d_in, d_out, width, height, n_frames, in_format, ksize, wts, in_row0, in_rows, out_row0, out_rows);
-
-    // staged path: gray band -> exact KxK blur -> Sobel, through the caller's workspace
-    size_t need = 0;
-    rip_fused_workspace_bytes(width, in_rows, n_frames, ksize, &need);
-    if (!d_workspace || workspace_bytes < need)
-        return fail(RIP_EINVAL, "rip_fused: this shape runs the staged path and needs %zu bytes of workspace (got %zu)", need, workspace_bytes);
-    uint8_t *ws_gray = (uint8_t *)d_workspace;
-    uint8_t *ws_blur = ws_gray + (size_t)width * in_rows * n_frames;
-    if (cn == 1) {   // the input is the gray image already
-        if (in_format == RIP_FMT_NV12 && n_frames > 1)
-            return fail(RIP_EUNSUPPORTED, "rip_fused: NV12 batches run the single-kernel path only (5x5 weights, width %% 4 == 0, aligned buffers)");
-        ws_gray = const_cast<uint8_t *>(d_in);
-    } else if (int rc = launch_gray(s, d_in, ws_gray, (long long)width * in_rows * n_frames, in_format, RIP_GRAY_OUT_U8, device)) {
-        return rc;
-    }
-    if (int rc = launch_blur(s, ws_gray, ws_blur, width, height, n_frames, 1, ksize, wts, in_row0, in_rows, b0, b1 - b0)) return rc;
-    return launch_sobel(s, ws_blur, d_out, width, height, n_frames, RIP_FMT_GRAY8, b0, b1 - b0, out_row0, out_rows);
+    // every other shape, kernel size and weight set: still one kernel, the reference's arithmetic throughout
+    return launch_fused_tile(s, d_in, d_out, width, height, n_frames, in_format, ksize, wts, in_row0, in_rows, out_row0, out_rows);
 }
 
 // ============================================================================================
@@ -826,13 +804,6 @@ extern "C" int rip_out_bytes_per_frame(const rip_op_desc *desc, int width, int h
 
 namespace {
 
-bool fused_single_kernel(int W, int H, int fmt, int ksize, const float *weights, const void *d_in, const void *d_out)
-{
-    float g3[3], thr;
-    return ksize == 5 && weights && fused_supported(W, H, fmt, 5, (const uint8_t *)d_in, (const uint8_t *)d_out) &&
-           fused_plan_weights(weights, g3, &thr);
-}
-
 int validate_desc(const rip_op_desc *desc, int *cn_out)
 {
     if (!desc) return fail(RIP_EINVAL, "rip_process_host: NULL descriptor");
@@ -881,7 +852,7 @@ int enqueue_op(const rip_ticket &t, int device, const BufSet &b, int n_frames, c
     if (band) {
         if (d.op == RIP_OP_FUSED)
             return rip_fused(device, s, in, out, t.W, t.H, 1, d.in_format, d.ksize, d.weights, band->in_row0, band->in_rows,
-                             band->out_row0, band->out_rows, b.d_ws, b.ws_cap);
+                             band->out_row0, band->out_rows, nullptr, 0);
         return rip_sobel_rows(device, s, in, out, t.W, t.H, d.in_format, band->in_row0, band->in_rows, band->out_row0, band->out_rows);
     }
     switch (d.op) {
@@ -892,7 +863,7 @@ int enqueue_op(const rip_ticket &t, int device, const BufSet &b, int n_frames, c
     case RIP_OP_GAUSSIAN:
         return rip_gauss(device, s, in, out, t.W, t.H, n_frames, t.cn, d.ksize, d.weights);
     case RIP_OP_FUSED:
-        return rip_fused(device, s, in, out, t.W, t.H, n_frames, d.in_format, d.ksize, d.weights, 0, t.H, 0, t.H, b.d_ws, b.ws_cap);
+        return rip_fused(device, s, in, out, t.W, t.H, n_frames, d.in_format, d.ksize, d.weights, 0, t.H, 0, t.H, nullptr, 0);
     default:
         return fail(RIP_EINVAL, "unknown op %d", d.op);
     }
@@ -966,12 +937,6 @@ void issue_part(DevState &dev, Part *p)
         uint8_t *dst = band ? t.h_out + (size_t)t.W * p->out_row0 : t.h_out + (size_t)(p->f0 + c0) * t.out_frame_bytes;
         if ((rc = ensure(&b.d_in, &b.in_cap, in_bytes))) break;
         if ((rc = ensure(&b.d_out, &b.out_cap, out_bytes))) break;
-        if (t.desc.op == RIP_OP_FUSED &&
-            !fused_single_kernel(t.W, t.H, t.desc.in_format, t.desc.ksize, t.desc.weights, b.d_in, b.d_out)) {
-            size_t ws_need = 0;  // staged path only
-            rip_fused_workspace_bytes(t.W, band ? p->in_rows : t.H, cf, t.desc.ksize, &ws_need);
-            if ((rc = ensure(&b.d_ws, &b.ws_cap, ws_need))) break;
-        }
         if (!t.in_pinned) {   // pageable source: stage through pinned memory (the copy overlaps the DMA of the previous chunk)
             if ((rc = ensure_pinned(&b.stage_in, &b.stage_in_cap, in_bytes))) break;
             memcpy(b.stage_in, src, in_bytes);

@@ -49,11 +49,9 @@ constexpr int kMaxGridZ = 65535;   // frames per launch of the kernels that inde
 // Debug / experiment switches.  Read from the environment ONCE (first use), then only changed through
 // rip_debug_set_option(): no getenv() on any launch path.
 struct Options {
-    int disable_fused = 0;   // RIP_DISABLE_FUSED: never take the single-kernel fused path
     int fused_seg = 0;       // RIP_FUSED_SEG:     rows per segment of the fused kernel (0 = automatic)
     int fused_npx = 0;       // RIP_FUSED_NPX:     4 = force the 4-pixel-per-lane kernel (0 / 8 = automatic)
     int fused_generic = 0;   // RIP_FUSED_GENERIC: rip_fused always runs the any-shape tile kernel (rip_fused_tile.cu)
-    int fused_staged = 0;    // RIP_FUSED_STAGED:  shapes the streaming kernel rejects run gray / blur / Sobel as three kernels (round 1's path)
     int blur_exact = 0;      // RIP_BLUR_EXACT:    always run the reference-order blur kernel
     int blur_tiled = 0;      // RIP_BLUR_TILED:    never run the streaming blur kernels
     int blur_stream = 0;     // RIP_BLUR_STREAM:   run the streaming blur kernels on small inputs too

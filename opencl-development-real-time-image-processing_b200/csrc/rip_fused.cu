@@ -1,15 +1,15 @@
 // rip_fused.cu -- gray -> 5x5 Gaussian -> 3x3 Sobel in ONE kernel (one HBM round trip per frame), and the
 // same kernel without the blur stage (gray -> Sobel, BASELINE config 3): host side (weight planning, grid
-// shaping, launch) and the on-device self-test.  The kernel itself is rip_fused_x2.cuh.
+// shaping, launch) and the on-device self-test.  The kernel itself is rip_fused_x3.cuh.
 //
 // Design (sm_100a, an FMA-pipe/issue-bound integer+fp32 stencil; no tensor cores by design):
 //   * every WARP is independent.  A lane owns NPX = 8 (or 4) horizontally adjacent pixels; a warp covers
 //     32*NPX pixels of which the middle 30*NPX (lanes 1..30) are outputs and the outer lanes are halo.
 //     The warp slides DOWN a segment of rows, so the vertical halo costs 6 warm-up rows per segment and
 //     the horizontal halo 2/32 of the lanes.  One block-level barrier at start-up, none afterwards.
-//   * per image row a lane loads its 3*NPX (RGB) or 4*NPX (RGBA) bytes with 64/128-bit loads issued
-//     three rows ahead (plus an L2 prefetch further down), converts them to the reference's exact gray,
-//     and keeps the vertical blur accumulators and two rows of Sobel input in registers.
+//   * per image row a lane fetches its 3*NPX (RGB) or 4*NPX (RGBA) bytes into shared memory with cp.async
+//     three (with the blur stage) or six rows ahead, converts them to the reference's exact gray, and keeps
+//     the vertical blur accumulators and two rows of Sobel input in registers.
 //   * the horizontal neighbours (2 per side for the blur, 1 per side for Sobel) come from the adjacent
 //     lanes with warp shuffles.
 //   * exactness: the blurred value must equal the reference's sequential, unfused, 25-tap fp32 sum
@@ -30,25 +30,15 @@
 #include "rip_common.cuh"
 #include "rip_internal.h"
 
-// x2 kernel (rip_fused_x2.cuh): resident blocks per SM for 8 / 4 pixels per lane, L2 prefetch distance
-#ifndef RIP_X2_MINB8
-#define RIP_X2_MINB8 4
-#endif
-#ifndef RIP_X2_MINB8_NOBLUR
-#define RIP_X2_MINB8_NOBLUR 6   // colour -> gray -> Sobel: six blocks (24 warps) per SM since the row buffers left the registers (76 registers; config 3: 121 -> 117 us; five before: 127 -> 123 us; gray input is better off with 4)
-#endif
-#ifndef RIP_X2_MINB4
-#define RIP_X2_MINB4 6
-#endif
-#ifndef RIP_X2_L2PF
-#define RIP_X2_L2PF 0   // rows ahead of the register loads that prefetch.global.L2 runs (0 = off: round 2 measured 431 us without against 436 us with 6)
-#endif
-
 namespace rip {
 
 namespace {
 
 constexpr int kWarpsPerBlock = 4;
+// x2 kernel (rip_fused_x3.cuh): resident blocks per SM for 8 / 4 pixels per lane
+constexpr int kMinBlocks8 = 4;
+constexpr int kMinBlocks8NoBlur = 6;   // colour -> gray -> Sobel: six blocks (24 warps) per SM since the row buffers left the registers (76 registers; config 3: 121 -> 117 us; five before: 127 -> 123 us; gray input is better off with 4)
+constexpr int kMinBlocks4 = 6;
 constexpr unsigned FULL = 0xffffffffu;
 
 struct FusedParams {
@@ -91,7 +81,6 @@ bool fused_supported(int W, int H, int fmt, int ksize, const uint8_t *d_in, cons
     if (fmt == RIP_FMT_NV12 && (H & 1)) return false;
     const uintptr_t in_align = cn == 4 ? 15u : 3u;
     if ((reinterpret_cast<uintptr_t>(d_in) & in_align) || (reinterpret_cast<uintptr_t>(d_out) & 3u)) return false;
-    if (options().disable_fused) return false;
     return true;
 }
 
@@ -204,7 +193,7 @@ static int launch_fused_x2_n(cudaStream_t s, FusedParams p, int n_frames, int fm
     memset(&xp, 0, sizeof(xp));
     p.n_bands = (p.W + kBand - 1) / kBand;
     p.n_band_groups = (p.n_bands + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    p.seg_rows = pick_seg_rows(p.out_rows, n_frames, p.n_band_groups, device, NPX == 8 ? RIP_X2_MINB8 : RIP_X2_MINB4);
+    p.seg_rows = pick_seg_rows(p.out_rows, n_frames, p.n_band_groups, device, NPX == 8 ? kMinBlocks8 : kMinBlocks4);
     p.n_segs = (p.out_rows + p.seg_rows - 1) / p.seg_rows;
     xp.f = p;
     if (with_blur) {
@@ -327,7 +316,7 @@ __global__ void selftest_gray_x2_kernel(unsigned long long *bad)
         u64 Q[NP], E[NP];
         const uint32_t any = gray_x2<NPX, CN, BGR>(w, Q, E);
         if (__any_sync(FULL, any & 1u)) {
-            if (any & 1u) gray_fix_x2<NPX, CN, BGR>(w, Q, E);
+            if (any & 1u) gray_fix_pairs<NPX, CN, BGR>(w, Q, E);
         }
 #pragma unroll
         for (int j = 0; j < NPX; j++) {

@@ -44,13 +44,6 @@
 
 typedef unsigned long long u64;
 
-#ifndef RIP_REPLAY_FN
-#define RIP_REPLAY_FN __forceinline__
-#endif
-#ifndef RIP_COLD_FN
-#define RIP_COLD_FN __forceinline__
-#endif
-
 __device__ __forceinline__ u64 pk2(float lo, float hi) { u64 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
 __device__ __forceinline__ u64 pk2u(uint32_t lo, uint32_t hi) { u64 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "r"(lo), "r"(hi)); return r; }
 __device__ __forceinline__ float lo2(u64 v) { float lo, hi; asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); return lo; }
@@ -146,12 +139,10 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t addr) { uint32_t v; asm vola
 
 // ---- the gray ring ------------------------------------------------------------------------------------------------
 // Every warp keeps the last kRing = 6 gray rows of its band in shared memory, as integer bit patterns (= q * 2^-149 read
-// as floats).  It serves two readers: the VERTICAL BLUR PASS of the hot path, which loads rows r-1 .. r-4 back instead of
-// carrying four rows of partial sums in registers (32 registers less than round 1's accumulate form, and no register
-// shift between rows -- ptxas turned that shift into ~28 moves per three rows at the loop's back edge), and the exact
-// replay of guard-band pixels.  Layout of a row (kRowB = 128 * NPX bytes): NP/2 planes of 512 bytes; plane p holds, for
-// lane L at byte 16 L, the pairs 2p and 2p+1 of that lane (pair k = (pixel k, pixel k + NP)): a lane stores and
-// reloads its row with NP/2 conflict-free 128-bit accesses.
+// as floats).  Only the cold paths read it: the constant-window test and the exact replay of guard-band pixels (the
+// vertical blur pass of the hot path carries its partial sums in registers, WarpX).  Layout of a row (kRowB = 128 * NPX
+// bytes): NP/2 planes of 512 bytes; plane p holds, for lane L at byte 16 L, the pairs 2p and 2p+1 of that lane (pair k =
+// (pixel k, pixel k + NP)): a lane stores and reloads its row with NP/2 conflict-free 128-bit accesses.
 constexpr int kRing = 6;
 
 // byte offset inside a ring row of band column c (column 0 = pixel 0 of lane 0)
@@ -233,56 +224,19 @@ __device__ __forceinline__ void apply_dec(u64 *V, uint32_t dec)
     }
 }
 
-// register-in / register-out gray fix for the self-test
-template <int NPX, int CN, bool BGR>
-__device__ __forceinline__ void gray_fix_x2(const uint32_t *w, u64 *Q, const u64 *E)
-{
-    gray_fix_pairs<NPX, CN, BGR>(w, Q, E);
-}
-
+// this lane's raw bytes of one input row
 template <int NPX, int CN>
 struct RawX {
     uint32_t w[NPX * CN / 4];
 };
 
-// Unpredicated: lanes outside the image read the start of the row (their pointer has x offset 0) and
-// their pixels are never consumed.  A predicated load would tie each destination register to its
-// previous value and turn the rotation of the prefetch registers into moves.
-template <int NPX, int CN>
-__device__ __forceinline__ void load_row_x2(RawX<NPX, CN> &r, const uint8_t *p)
-{
-    constexpr int NW = NPX * CN / 4;
-    if constexpr (NW == 1) {
-        r.w[0] = __ldg(reinterpret_cast<const uint32_t *>(p));
-    } else if constexpr (NW == 2) {
-        const uint2 a = __ldg(reinterpret_cast<const uint2 *>(p));
-        r.w[0] = a.x; r.w[1] = a.y;
-    } else if constexpr (NW == 3) {
-        const uint32_t *q = reinterpret_cast<const uint32_t *>(p);
-        r.w[0] = __ldg(q); r.w[1] = __ldg(q + 1); r.w[2] = __ldg(q + 2);
-    } else if constexpr (NW == 4) {
-        const uint4 v = __ldg(reinterpret_cast<const uint4 *>(p));
-        r.w[0] = v.x; r.w[1] = v.y; r.w[2] = v.z; r.w[3] = v.w;
-    } else if constexpr (NW == 6) {
-        const uint2 *q = reinterpret_cast<const uint2 *>(p);
-        const uint2 a = __ldg(q), b = __ldg(q + 1), c = __ldg(q + 2);
-        r.w[0] = a.x; r.w[1] = a.y; r.w[2] = b.x; r.w[3] = b.y; r.w[4] = c.x; r.w[5] = c.y;
-    } else {
-        const uint4 *q = reinterpret_cast<const uint4 *>(p);
-        const uint4 a = __ldg(q), b = __ldg(q + 1);
-        r.w[0] = a.x; r.w[1] = a.y; r.w[2] = a.z; r.w[3] = a.w; r.w[4] = b.x; r.w[5] = b.y; r.w[6] = b.z; r.w[7] = b.w;
-    }
-}
-
-// RIP_X3_CPASYNC = 1 (the default): input rows travel global -> shared with cp.async, NB rows ahead of their use (one commit
-// group per row, the step of row r waits until at most NB - 1 groups are pending), and each lane reads its own bytes back with
-// LDS.  0: register loads NB rows ahead (rounds 1-2).  With register loads the first consumer of a loaded row in ONE of the
-// unrolled steps held 8.5 % of the kernel's stall samples (profiles/r2m_fused_x3_hotspots.txt) whatever the distance -- a wait
-// on a load's scoreboard also waits for every younger load that shares it (seen and fixed first in the streaming blur,
-// rip_blur_stream.cuh) -- and the three row buffers occupied 18 registers.
-#ifndef RIP_X3_CPASYNC
-#define RIP_X3_CPASYNC 1
-#endif
+// Input rows travel global -> shared with cp.async, NB rows ahead of their use (one commit group per row, the step of row r
+// waits until at most NB - 1 groups are pending), and each lane reads its own bytes back with LDS.  Rounds 1-2 used register
+// loads NB rows ahead: the first consumer of a loaded row in ONE of the unrolled steps then held 8.5 % of the kernel's stall
+// samples (profiles/r2m_fused_x3_hotspots.txt) whatever the distance -- a wait on a load's scoreboard also waits for every
+// younger load that shares it (seen and fixed first in the streaming blur, rip_blur_stream.cuh) -- and the three row buffers
+// occupied 18 registers.  Lanes outside the image fetch the start of the row (their pointer has x offset 0); their pixels are
+// never consumed.
 
 // this lane's NW words of a row: global -> shared (asynchronous), shared -> registers
 template <int NPX, int CN>
@@ -331,19 +285,13 @@ __device__ __forceinline__ void lds_row_x3(RawX<NPX, CN> &r, uint32_t a)
     }
 }
 
-// RIP_X3_ACC = 1 (the default): the vertical pass carries four rows of partial sums in registers (accumulate form, five
-// packed FMAs per pixel pair and row, no shared-memory reads on the hot path); 0: it re-reads gray rows r-1 .. r-4 from the
-// ring (eight LDS.128 per lane and row, 32 registers of state less).  Measured on 32 4K frames with the round's final cold
-// paths: 418 us against 436 us (122 against 114 registers, both four blocks per SM, neither spills).
-#ifndef RIP_X3_ACC
-#define RIP_X3_ACC 1
-#endif
-
+// The vertical blur pass carries four rows of partial sums in registers (accumulate form, five packed FMAs per pixel pair and
+// row, no shared-memory reads on the hot path).  Re-reading gray rows r-1 .. r-4 from the ring instead (eight LDS.128 per lane
+// and row, 32 registers of state less) was measured on 32 4K frames with the round's final cold paths: 436 us against 418 us
+// (114 against 122 registers, both four blocks per SM, neither spills).
 template <int NPX, int CN>
 struct WarpX {
-#if RIP_X3_ACC
     u64 a0[NPX / 2], a1[NPX / 2], a2[NPX / 2], a3[NPX / 2];  // pending vertical sums of blurred rows r-2 .. r+1
-#endif
     u64 F1[NPX / 2], F2[NPX / 2];   // rows yb-1 and yb-2 of the image the Sobel stage reads
 };
 
@@ -353,10 +301,9 @@ struct GeoX {
     uint32_t ring_lane;      // shared-memory byte address of this lane's 16 bytes in plane 0 of slot 0 of the warp's gray ring
     uint32_t ringA, ringB;   // main loop: ring_lane + the half (slots 0-2 / 3-5) this trip writes / wrote last trip
     uint32_t slot;           // head / tail rows: slot of the newest gray row
-    uint32_t raw_lane, rs;   // RIP_X3_CPASYNC: shared-memory byte address of this lane's bytes in slot 0 of the warp's raw-row ring; head / tail rows: slot of the row in use
+    uint32_t raw_lane, rs;   // shared-memory byte address of this lane's bytes in slot 0 of the warp's raw-row ring; head / tail rows: slot of the row in use
     uint32_t in_pitch;
     int adv_lo, adv_n;       // the source pointer advances before the load of step r iff 0 <= r - adv_lo < adv_n
-    uint32_t pf_off;         // byte offset from src of the line this lane prefetches into L2 (0: none)
     int lane;
     uint32_t need;           // pixels of this lane whose blurred value feeds an output (bit j = pixel j): all of lanes 1..30,
                              // only the pixel next to the band in the two halo lanes, none in lanes outside the image
@@ -390,7 +337,7 @@ constexpr int kLaneTabWords = 16;
 __shared__ uint32_t s_lane_tab[kWarpsPerBlock * 32 * kLaneTabWords];
 
 template <int NPX>
-__device__ RIP_REPLAY_FN uint32_t blur_flat_lane(uint32_t ring_lane, uint32_t newest, uint32_t tab, const uint32_t *flat_dec, int r)
+__device__ __forceinline__ uint32_t blur_flat_lane(uint32_t ring_lane, uint32_t newest, uint32_t tab, const uint32_t *flat_dec, int r)
 {
     constexpr uint32_t kRowB = 32 * NPX * 4;
     const uint32_t ol2 = lds_u32(tab), ol1 = lds_u32(tab + 4u), or0 = lds_u32(tab + 4u * (NPX + 2)), or1 = lds_u32(tab + 4u * (NPX + 3));
@@ -465,7 +412,7 @@ __constant__ RingRel<4> c_ring_rel4;
 // (Out of line -- one __noinline__ copy for all row bodies, main loop 1126 instead of 1693 instructions -- was measured:
 // 445 us against 431 us; the call sequence and the run-time ring slots cost more than the smaller loop gains.)
 template <int NPX>
-__device__ RIP_REPLAY_FN uint32_t blur_replay_lane(uint32_t my, const uint32_t (&rowaddr)[5], uint32_t tab, const BlurFixConst &cst)
+__device__ __forceinline__ uint32_t blur_replay_lane(uint32_t my, const uint32_t (&rowaddr)[5], uint32_t tab, const BlurFixConst &cst)
 {
     uint32_t dec = 0;
 #pragma unroll 1
@@ -489,29 +436,24 @@ __device__ RIP_REPLAY_FN uint32_t blur_replay_lane(uint32_t my, const uint32_t (
     return dec;
 }
 
-// One image row of the sliding window: consumes the input row held in `buf` (row r, clamped to the
-// rows of the band), refills `buf` with row r + NB (NB = row buffers, see X2Cfg), and -- for r_store <= r <= r_last -- stores output
-// row r - HALO.  The border rules are applied at run time (per-lane selects in x, two rare uniform
-// branches in y), so this is the only copy of the row body; the caller unrolls it by three with three
-// row buffers, which makes the buffer rotation and the two-row Sobel delay line register renames.
+// One image row of the sliding window: consumes input row r (clamped to the rows of the band) from the raw-ring slot at
+// `raw_addr`, where it was fetched NB steps earlier, fetches row r + NB into the same slot, and -- for r_store <= r <= r_last --
+// stores output row r - HALO.  The border rules are applied at run time (per-lane selects in x, two rare uniform branches in
+// y), so this is the only copy of the row body; the caller's main loop unrolls it by NB, which makes the two-row Sobel delay
+// line register renames.
 // What a copy of the row body has to check at run time:
-//   SPECIAL  head and tail rows of a segment: does this row store, do the next input row and the prefetched
-//            line exist, BORDER_REFLECT_101 in y.  The main loop's copies check none of that.
-//   EDGE     the warp's band holds image column 0 and/or W-1: per-lane border selects in x.
+//   SPECIAL  head and tail rows of a segment: does this row store, does the next input row exist, BORDER_REFLECT_101 in y.
+//            The main loop's copies check none of that.
 //   KS       position of the row inside a main-loop trip (0, 1, 2): the ring slots of rows r .. r-4 are then compile-time
 //            offsets from the two half-ring bases geo.ringA / geo.ringB.  KS = -1 (head / tail rows): run-time slots.
-template <int NPX, int CN, bool BGR, bool BLUR, bool SPECIAL, bool EDGE, bool STATS, int KS, int NB>
-#if RIP_X3_CPASYNC
+// Every copy takes the per-lane border selects in x behind one warp-uniform branch (geo.edge_warp: the band holds image
+// column 0 and/or W-1).
+template <int NPX, int CN, bool BGR, bool BLUR, bool SPECIAL, bool STATS, int KS, int NB>
 __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, const uint32_t raw_addr, const X2Params &xp, GeoX &geo, int r)
-#else
-__device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, const X2Params &xp, GeoX &geo, int r)
-#endif
 {
-#if RIP_X3_CPASYNC
     RawX<NPX, CN> buf;   // row r: fetched NB steps ago
     asm volatile("cp.async.wait_group %0;" ::"n"(NB - 1) : "memory");
     lds_row_x3<NPX, CN>(buf, raw_addr);
-#endif
     constexpr int NP = NPX / 2;
     constexpr int kRowB = 32 * NPX * 4;  // bytes per ring row
     static_assert(SPECIAL == (KS < 0), "head / tail rows use run-time ring slots");
@@ -519,30 +461,18 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
     const int W = p.W, H = p.H;
     (void)H;
 
-    // ---- 1. gray of row r; refill the buffer with row r + NB --------------------------------------
+    // ---- 1. gray of row r; fetch row r + NB --------------------------------------------------------
     u64 Q[NP];
     uint32_t rowaddr[5];   // this lane's 16 bytes (plane 0) of the ring rows holding gray rows r, r-1, .. r-4
     {
         u64 E[NP];
         const uint32_t flagged = gray_x2<NPX, CN, BGR>(buf.w, Q, E) & 1u;
-#if !defined(RIP_X2_NOCOLD) && !defined(RIP_X3_NOGRAYCOLD)   // (experiment switches: hot path only, wrong results)
-#ifdef RIP_X3_NEVERCOLD   // (experiment: the cold code is present but never runs -- what does its mere presence cost?)
-        if (CN != 1 && __builtin_expect(__any_sync(FULL, flagged && xp.zthr == 0xdeadbeefu), 0)) {
-#else
         if (CN != 1 && __builtin_expect(__any_sync(FULL, flagged), 0)) {
-#endif
-            if (flagged) {
-#ifdef RIP_X3_EMPTYCOLD   // (experiment: the branches without their work -- what does the control structure alone cost?)
-                asm volatile("" : "+l"(Q[0]));
-#else
-                gray_fix_pairs<NPX, CN, BGR>(buf.w, Q, E);
-#endif
-            }
+            if (flagged) gray_fix_pairs<NPX, CN, BGR>(buf.w, Q, E);
         }
-#endif
         if constexpr (BLUR) {
-            // park the integer gray row in the shared ring (the vertical pass of the next four rows and the exact
-            // replay read it back); rows r-1 .. r-4 sit in the slots before it
+            // park the integer gray row in the shared ring (the blur's cold paths of this and the next four rows read it
+            // back); rows r-1 .. r-4 sit in the slots before it
             if constexpr (KS < 0) {
                 geo.slot = geo.slot == (uint32_t)kRing - 1u ? 0u : geo.slot + 1u;
                 uint32_t s4 = geo.slot;
@@ -567,17 +497,7 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
         } else {
             geo.src += geo.in_pitch;   // (the main loop stops short of the rows where the band ends)
         }
-#if RIP_X3_CPASYNC
         cp_row_x3<NPX, CN>(raw_addr, geo.src);   // row r + NB into the slot row r just left
-#else
-        load_row_x2<NPX, CN>(buf, geo.src);
-#endif
-#if RIP_X2_L2PF > 0
-        // pull the warp's bytes of a row further down into L2 (one 128-byte line per lane; pf_off is 0 in
-        // the lanes that have no line to fetch and at the rows the band does not hold)
-        if (geo.pf_off != 0 && (!SPECIAL || (unsigned)(r - geo.adv_lo) + RIP_X2_L2PF < (unsigned)geo.adv_n))
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(geo.src + geo.pf_off));
-#endif
     }
 
     // F[j] = (f[j], f[j + NP]): the row the Sobel stage consumes (blurred row yb, biased by kBias, or
@@ -587,7 +507,6 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
     if constexpr (BLUR) {
         const u64 GV0 = pk2(xp.gv0, xp.gv0), GV1 = pk2(xp.gv1, xp.gv1), GV2 = pk2(xp.gv2, xp.gv2);
         u64 V[NP];
-#if RIP_X3_ACC
         // vertical pass, accumulate form: row r completes blurred row r-2
 #pragma unroll
         for (int j = 0; j < NP; j++) {
@@ -597,7 +516,6 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
             st.a2[j] = fma2(GV1, Q[j], st.a3[j]);
             st.a3[j] = mul2(GV2, Q[j]);
         }
-#endif
         if constexpr (SPECIAL) {
             // warm-up rows of a segment: the first blurred row any stored output reads (ys - 1) completes at step
             // r_store - 2; before that only the gray ring is filled (the vote tells the compiler that the whole
@@ -607,29 +525,12 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
                 return;
             }
         }
-#if !RIP_X3_ACC
-        // vertical pass: blurred row r-2 from gray rows r-4 .. r, the four older ones read back from the ring (this lane's
-        // own stores: no synchronisation), symmetric form: g0 q(r-2) + g1 (q(r-3) + q(r-1)) + g2 (q(r-4) + q(r))
-#pragma unroll
-        for (int pl = 0; pl < NP / 2; pl++) {
-            u64 m1[2], m2[2], m3[2], m4[2];
-            asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];" : "=l"(m1[0]), "=l"(m1[1]) : "r"(rowaddr[1] + 512 * pl));
-            asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];" : "=l"(m2[0]), "=l"(m2[1]) : "r"(rowaddr[2] + 512 * pl));
-            asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];" : "=l"(m3[0]), "=l"(m3[1]) : "r"(rowaddr[3] + 512 * pl));
-            asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];" : "=l"(m4[0]), "=l"(m4[1]) : "r"(rowaddr[4] + 512 * pl));
-#pragma unroll
-            for (int k = 0; k < 2; k++) {
-                const u64 s1 = add2(m3[k], m1[k]), s2 = add2(m4[k], Q[2 * pl + k]);   // (integer-valued denormals: exact)
-                V[2 * pl + k] = fma2(GV2, s2, fma2(GV1, s1, mul2(GV0, m2[k])));
-            }
-        }
-#endif
         // horizontal pass.  c[m] = V of pixel m (pixel m lives in pair m % NP, half m / NP); e2 = c[m-2] + c[m+2],
         // e1 = c[m-1] + c[m+1].  Clamp-to-edge columns (GaussianBlur.cpp:240): V is linear in the gray column, so the
         // clamp applies to V: left of column 0 / right of column W-1 repeat it.
         float Vm2 = __shfl_up_sync(FULL, hi2(V[NP - 2]), 1), Vm1 = __shfl_up_sync(FULL, hi2(V[NP - 1]), 1);
         float Vp0 = __shfl_down_sync(FULL, lo2(V[0]), 1), Vp1 = __shfl_down_sync(FULL, lo2(V[1]), 1);
-        if (EDGE && geo.edge_warp) {   // (interior bands skip the selects where ptxas keeps the branch)
+        if (geo.edge_warp) {   // (interior bands skip the selects where ptxas keeps the branch)
             Vm2 = geo.e_left ? lo2(V[0]) : Vm2;
             Vm1 = geo.e_left ? lo2(V[0]) : Vm1;
             Vp0 = geo.e_right ? hi2(V[NP - 1]) : Vp0;
@@ -663,18 +564,9 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
         for (int j = 0; j < NP; j++)
             zmin = __vimin3_u32(zmin, lo2u(F[j]) << (32 - kFracBits), hi2u(F[j]) << (32 - kFracBits));
         const uint32_t flagged = zmin < xp.zthr ? 1u : 0u;
-#if !defined(RIP_X2_NOCOLD) && !defined(RIP_X3_NOBLURCOLD)
-#ifdef RIP_X3_NEVERCOLD
-        if (__builtin_expect(__any_sync(FULL, flagged && xp.bias == 12345.0f), 0)) {
-#else
         if (__builtin_expect(__any_sync(FULL, flagged), 0)) {
-#endif
             __syncwarp();  // the newest ring row was just stored by the other lanes
-#ifdef RIP_X3_EMPTYCOLD
-            if (flagged) asm volatile("" : "+l"(F[0]));
-#else
             if (flagged) {
-                // which pixels are inside the band ... and feed an output
                 // Which pixels are inside the band and feed an output?  A pixel whose masked value is n = 0 needs no fix at all: the
                 // reference's result is n or n - 1 and cannot be negative (black bars and frames leave here).
                 const uint32_t zero_bits = __float_as_uint(kBias);
@@ -709,12 +601,8 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
                     if (dec) apply_dec<NPX, kFracBits>(F, dec);   // 256 + n + fraction -> 256 + (n - 1) + fraction
                 }
             }
-#endif
             __syncwarp();  // every lane is done with the ring before the next step overwrites its oldest slot
         }
-#else
-        if (flagged == 77u) F[0] = 0;
-#endif
 #pragma unroll
         for (int j = 0; j < NP; j++) F[j] = pk2u(lo2u(F[j]) & kBiasMask, hi2u(F[j]) & kBiasMask);   // kBias + floor(S)
     } else {
@@ -748,7 +636,7 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
     // horizontal pass, BORDER_REFLECT_101 in x: gx = Vs[x+1] - Vs[x-1],  gy = Vd[x-1] + 2 Vd[x] + Vd[x+1]
     float sl = __shfl_up_sync(FULL, hi2(Vs[NP - 1]), 1), sr = __shfl_down_sync(FULL, lo2(Vs[0]), 1);
     float dl = __shfl_up_sync(FULL, hi2(Vd[NP - 1]), 1), dr = __shfl_down_sync(FULL, lo2(Vd[0]), 1);
-    if (EDGE && geo.edge_warp) {
+    if (geo.edge_warp) {
         sl = geo.e_left ? lo2(Vs[1]) : sl;             // x = -1 -> x = 1
         dl = geo.e_left ? lo2(Vd[1]) : dl;
         sr = geo.e_right ? hi2(Vs[NP - 2]) : sr;       // x = W  -> x = W-2
@@ -797,19 +685,12 @@ __device__ __forceinline__ void step_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> &buf, 
 }
 
 // The rows of one segment.  Head: the warm-up rows and the first storing row (it may be frame row 0), one row
-// per trip with the SPECIAL copy of the row body and an explicit rotation of the three row buffers.  Main loop:
-// NB rows per trip with the plain copy; the buffer rotation and the Sobel delay line are register renames
-// there.  Tail: the remaining rows (the last may be frame row H-1), SPECIAL again.  Only the main loop is hot,
-// so only its three copies of the row body need to stay in the instruction cache.
-// NB = row buffers = how many rows ahead of their use the register loads run (and the unroll of the main loop:
-// 3 with the blur stage; 6 without it, where a row is consumed twice as fast and load latency is the top stall).
-template <int NPX, int CN, bool BGR, bool BLUR>
-struct X2Cfg {
-    static constexpr int NB = BLUR ? 3 : 6;
-};
-
-#if RIP_X3_CPASYNC
-template <int NPX, int CN, bool BGR, bool BLUR, bool EDGE, int NB, bool STATS>
+// per trip with the SPECIAL copy of the row body and a run-time slot of the raw-row ring.  Main loop: NB rows per
+// trip with the plain copy and compile-time slots.  Tail: the remaining rows (the last may be frame row H-1), SPECIAL
+// again.  Only the main loop is hot, so only its copies of the row body need to stay in the instruction cache.
+// NB = rows in flight in the raw-row ring = the unroll of the main loop: 3 with the blur stage; 6 without it, where a
+// row is consumed twice as fast and load latency is the top stall.
+template <int NPX, int CN, bool BGR, bool BLUR, int NB, bool STATS>
 __device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, const X2Params &xp, GeoX &geo, int r)
 {
     constexpr uint32_t kRowB = 32 * NPX * 4;
@@ -819,10 +700,12 @@ __device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, const X2Params &
     // half ring (slot 2 or 5), so that the main loop's trips write whole halves
 #pragma unroll 1
     for (; (r <= geo.r_store || (BLUR && (geo.slot != 2u && geo.slot != 5u))) && r < geo.r_last; r++) {
-        step_x2<NPX, CN, BGR, BLUR, true, EDGE, STATS, -1, NB>(st, geo.raw_lane + geo.rs * kRawB, xp, geo, r);
+        step_x2<NPX, CN, BGR, BLUR, true, STATS, -1, NB>(st, geo.raw_lane + geo.rs * kRawB, xp, geo, r);
         geo.rs = geo.rs == (uint32_t)NB - 1u ? 0u : geo.rs + 1u;
     }
-    const int r_main_last = min(geo.r_last - 1, p.in_row0 + p.in_rows - 1 - NB - RIP_X2_L2PF);
+    // the main loop runs while all rows of a trip store and the row they fetch (NB ahead) lies inside the band: step s
+    // advances freely iff s + NB - 1 < in_row0 + in_rows - 1
+    const int r_main_last = min(geo.r_last - 1, p.in_row0 + p.in_rows - 1 - NB);
     static_assert(!BLUR || NB == 3, "the half-ring addressing assumes three rows per trip");
     if constexpr (BLUR) {
         geo.ringA = geo.ring_lane + (geo.slot == 2u ? 3u * kRowB : 0u);
@@ -841,94 +724,40 @@ __device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, const X2Params &
 #pragma unroll 1
     for (; r + NB - 1 <= r_main_last; r += NB) {
         if constexpr (BLUR) {
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 0, NB>(st, ra[0], xp, geo, r);
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 1, NB>(st, ra[1], xp, geo, r + 1);
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 2, NB>(st, ra[2], xp, geo, r + 2);
+            step_x2<NPX, CN, BGR, BLUR, false, STATS, 0, NB>(st, ra[0], xp, geo, r);
+            step_x2<NPX, CN, BGR, BLUR, false, STATS, 1, NB>(st, ra[1], xp, geo, r + 1);
+            step_x2<NPX, CN, BGR, BLUR, false, STATS, 2, NB>(st, ra[2], xp, geo, r + 2);
             const uint32_t t = geo.ringA;   // the half just written becomes "last trip's"
             geo.ringA = geo.ringB;
             geo.ringB = t;
         } else {
 #pragma unroll
-            for (int k = 0; k < NB; k++) step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 0, NB>(st, ra[k], xp, geo, r + k);
+            for (int k = 0; k < NB; k++) step_x2<NPX, CN, BGR, BLUR, false, STATS, 0, NB>(st, ra[k], xp, geo, r + k);
         }
     }
     if constexpr (BLUR) geo.slot = (geo.ringB - geo.ring_lane) / kRowB + 2u;   // newest row: last slot of the half written last
 #pragma unroll 1
     for (; r <= geo.r_last; r++) {
-        step_x2<NPX, CN, BGR, BLUR, true, EDGE, STATS, -1, NB>(st, geo.raw_lane + geo.rs * kRawB, xp, geo, r);
+        step_x2<NPX, CN, BGR, BLUR, true, STATS, -1, NB>(st, geo.raw_lane + geo.rs * kRawB, xp, geo, r);
         geo.rs = geo.rs == (uint32_t)NB - 1u ? 0u : geo.rs + 1u;
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");   // (rows fetched past the segment's end)
 }
-#else
-template <int NPX, int CN, bool BGR, bool BLUR, bool EDGE, int NB, bool STATS>
-__device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, RawX<NPX, CN> (&b)[NB], const X2Params &xp, GeoX &geo, int r)
-{
-    constexpr uint32_t kRowB = 32 * NPX * 4;
-    const FusedParams &p = xp.f;
-    // head: up to the first storing row -- and, with the blur stage, until the newest gray row sits in the last slot of a
-    // half ring (slot 2 or 5), so that the main loop's trips write whole halves (geo.slot starts such that the usual
-    // seven head rows end there without extra ones).  (One shared copy of the head / tail body inside a two-phase loop
-    // was tried: ptxas made the whole kernel larger, 3328 instead of 3264 instructions.)
-#pragma unroll 1
-    for (; (r <= geo.r_store || (BLUR && (geo.slot != 2u && geo.slot != 5u))) && r < geo.r_last; r++) {
-        step_x2<NPX, CN, BGR, BLUR, true, EDGE, STATS, -1, NB>(st, b[0], xp, geo, r);
-        const RawX<NPX, CN> t = b[0];
-#pragma unroll
-        for (int k = 0; k + 1 < NB; k++) b[k] = b[k + 1];
-        b[NB - 1] = t;
-    }
-    // the main loop runs while all rows of a trip store, and the row they load (NB ahead) as well as the line
-    // they prefetch (RIP_X2_L2PF further) lie inside the band: step s advances freely iff
-    // s + NB - 1 + RIP_X2_L2PF < in_row0 + in_rows - 1
-    const int r_main_last = min(geo.r_last - 1, p.in_row0 + p.in_rows - 1 - NB - RIP_X2_L2PF);
-    static_assert(!BLUR || NB == 3, "the half-ring addressing assumes three rows per trip");
-    if constexpr (BLUR) {
-        geo.ringA = geo.ring_lane + (geo.slot == 2u ? 3u * kRowB : 0u);
-        geo.ringB = geo.ring_lane + (geo.slot == 2u ? 0u : 3u * kRowB);
-    }
-#pragma unroll 1
-    for (; r + NB - 1 <= r_main_last; r += NB) {
-        if constexpr (BLUR) {
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 0, NB>(st, b[0], xp, geo, r);
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 1, NB>(st, b[1], xp, geo, r + 1);
-            step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 2, NB>(st, b[2], xp, geo, r + 2);
-            const uint32_t t = geo.ringA;   // the half just written becomes "last trip's"
-            geo.ringA = geo.ringB;
-            geo.ringB = t;
-        } else {
-#pragma unroll
-            for (int k = 0; k < NB; k++) step_x2<NPX, CN, BGR, BLUR, false, EDGE, STATS, 0, NB>(st, b[k], xp, geo, r + k);
-        }
-    }
-    if constexpr (BLUR) geo.slot = (geo.ringB - geo.ring_lane) / kRowB + 2u;   // newest row: last slot of the half written last
-#pragma unroll 1
-    for (; r <= geo.r_last; r++) {
-        step_x2<NPX, CN, BGR, BLUR, true, EDGE, STATS, -1, NB>(st, b[0], xp, geo, r);
-        const RawX<NPX, CN> t = b[0];
-#pragma unroll
-        for (int k = 0; k + 1 < NB; k++) b[k] = b[k + 1];
-        b[NB - 1] = t;
-    }
-}
-
-#endif
 
 template <int NPX, int CN, bool BGR, bool BLUR, bool STATS = false>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, NPX == 8 ? ((BLUR || CN == 1) ? RIP_X2_MINB8 : RIP_X2_MINB8_NOBLUR) : RIP_X2_MINB4)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, NPX == 8 ? ((BLUR || CN == 1) ? kMinBlocks8 : kMinBlocks8NoBlur) : kMinBlocks4)
 fused_x2_kernel(const __grid_constant__ X2Params xp)
 {
     constexpr int HALO = BLUR ? 3 : 1;  // input rows above/below an output row
     constexpr int kRowW = 32 * NPX;     // words per ring row
     constexpr int kBand = 30 * NPX;
     constexpr int NW = NPX * CN / 4;
+    constexpr int NB = BLUR ? 3 : 6;    // rows in flight in the raw-row ring (run_rows_x2)
     const FusedParams &p = xp.f;
 
     __shared__ __align__(16) uint32_t ring[BLUR ? kWarpsPerBlock * kRing * kRowW : 4];
-#if RIP_X3_CPASYNC
     constexpr int kRawW = 32 * NPX * CN / 4;   // words of one raw row of a warp's band
-    __shared__ __align__(16) uint32_t raw_ring[kWarpsPerBlock * X2Cfg<NPX, CN, BGR, BLUR>::NB * kRawW];
-#endif
+    __shared__ __align__(16) uint32_t raw_ring[kWarpsPerBlock * NB * kRawW];
     // no block-level barrier: the warps are independent from the first instruction on
 
     GeoX geo;
@@ -979,9 +808,7 @@ fused_x2_kernel(const __grid_constant__ X2Params xp)
 #pragma unroll
     for (int j = 0; j < NPX / 2; j++) {
         st.F1[j] = st.F2[j] = 0ull;
-#if RIP_X3_ACC
         st.a0[j] = st.a1[j] = st.a2[j] = st.a3[j] = 0ull;
-#endif
     }
 
     // Rows are clamped to the rows the input band holds.  The host guarantees the band covers every
@@ -989,8 +816,6 @@ fused_x2_kernel(const __grid_constant__ X2Params xp)
     // (GaussianBlur.cpp:241) is actually exercised; other clamped rows are read-ahead only.
     int r = ys - HALO;
     const uint32_t xoff = in_img ? (uint32_t)x * CN : 0u;
-    constexpr int NB = X2Cfg<NPX, CN, BGR, BLUR>::NB;
-#if RIP_X3_CPASYNC
     geo.raw_lane = (uint32_t)__cvta_generic_to_shared(raw_ring + warp * NB * kRawW) + (uint32_t)(NPX * CN) * (uint32_t)geo.lane;
     geo.rs = 0u;
 #pragma unroll
@@ -999,30 +824,11 @@ fused_x2_kernel(const __grid_constant__ X2Params xp)
         geo.src = in_base + (size_t)i * geo.in_pitch + xoff;
         cp_row_x3<NPX, CN>(geo.raw_lane + (uint32_t)k * (uint32_t)(kRawW * 4), geo.src);
     }
-#else
-    RawX<NPX, CN> b[NB];   // rows r .. r + NB - 1
-#pragma unroll
-    for (int k = 0; k < NB; k++) {
-        const int i = min(max(r + k - p.in_row0, 0), p.in_rows - 1);
-        geo.src = in_base + (size_t)i * geo.in_pitch + xoff;
-        load_row_x2<NPX, CN>(b[k], geo.src);
-    }
-#endif
-    // step r loads row r + NB = one past the row src points at: advance iff in_row0 <= r + NB - 1 < in_row0 + in_rows - 1
+    // step r fetches row r + NB = one past the row src points at: advance iff in_row0 <= r + NB - 1 < in_row0 + in_rows - 1
     geo.adv_lo = p.in_row0 - (NB - 1);
     geo.adv_n = p.in_rows - 1;
-    {   // lanes 0..n-1 fetch the n consecutive 128-byte lines that hold the warp's NPX*CN*32 bytes of a row
-        constexpr int kLines = (32 * NPX * CN + 127) / 128 + 1;
-        const uint32_t lane0_to_me = (uint32_t)(NPX * CN) * (uint32_t)geo.lane;   // src points at this lane's pixels
-        geo.pf_off = (in_img && geo.lane < kLines) ? (uint32_t)RIP_X2_L2PF * geo.in_pitch + 128u * (uint32_t)geo.lane - lane0_to_me : 0u;
-        if (x - NPX * geo.lane < 0) geo.pf_off = 0u;   // (left-most band: lane 0 sits before the row; keep it simple)
-    }
     // output row produced by the step of input row r is r - HALO
     geo.dst = p.out + (size_t)frame * p.out_rows * W + (ptrdiff_t)(r - HALO - p.out_row0) * W + x;
 
-#if RIP_X3_CPASYNC
-    run_rows_x2<NPX, CN, BGR, BLUR, true, NB, STATS>(st, xp, geo, r);
-#else
-    run_rows_x2<NPX, CN, BGR, BLUR, true, NB, STATS>(st, b, xp, geo, r);
-#endif
+    run_rows_x2<NPX, CN, BGR, BLUR, NB, STATS>(st, xp, geo, r);
 }

@@ -54,6 +54,15 @@ def test_weights_generator_rejects_bad_arguments():
             rip.gauss_weights(k, s)
 
 
+def test_fused_needs_no_workspace():
+    """rip_fused runs every shape and kernel size as one kernel: the workspace query answers 0 and still validates."""
+    for w, in_rows, n, k in ((3840, 2160, 32, 5), (683, 1023, 1, 17), (75, 75, 4, 3), (1, 1, 1, 31), (1922, 7, 2, 9)):
+        assert rip.fused_workspace_bytes(w, in_rows, n, k) == 0, (w, in_rows, n, k)
+    for w, in_rows, n in ((0, 16, 1), (16, 0, 1), (16, 16, 0), (-4, 16, 1)):
+        with pytest.raises(rip.RipError):
+            rip.fused_workspace_bytes(w, in_rows, n, 5)
+
+
 @pytest.mark.skipif(rip.device_count() > 0, reason="only meaningful on a box without a GPU")
 def test_compute_fails_loudly_without_gpu():
     with pytest.raises(rip.RipError, match="no CUDA device|no CPU fallback"):

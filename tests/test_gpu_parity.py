@@ -434,17 +434,14 @@ def test_fused_formats_and_sigmas(ctx, oracle, fmt, cn, order, sigma, npx, opt):
 
 
 @pytest.mark.parametrize("shape", [(1, 1), (1, 9), (9, 1), (5, 5), (75, 75), (33, 241), (40, 683), (2, 2), (17, 33), (16, 32), (49, 97)])
-@pytest.mark.parametrize("staged", [0, 1])
-def test_fused_odd_shapes_tile_kernel_and_staged_path(ctx, oracle, shape, staged, opt):
-    """Shapes the streaming kernel rejects: one any-shape tile kernel (rip_fused_tile.cu); round 1's three-kernel path stays
-    reachable behind a switch and must agree."""
-    opt("RIP_FUSED_STAGED", staged)
+def test_fused_odd_shapes_tile_kernel(ctx, oracle, shape):
+    """Shapes the streaming kernel rejects run as one any-shape tile kernel (rip_fused_tile.cu); the streaming kernel takes
+    the others, also in one launch."""
     img = synth_frame("uniform", shape[0], shape[1], 51)
     w = rip.gauss_weights(5, 1.0)
     before = rip.launch_count()
     _eq(ctx.process(img, rip.OP_FUSED, rip.FMT_RGB8, ksize=5, weights=w), oracle.fused(img, 5, weights=w), f"fused odd shape {shape}")
-    streaming = shape[1] % 4 == 0 and shape[0] >= 2   # (the streaming kernel takes this one: one launch either way)
-    assert rip.launch_count() - before == (3 if staged and not streaming else 1)
+    assert rip.launch_count() - before == 1
 
 
 def test_fused_reference_image_sizes_run_one_kernel(ctx, oracle, golden_images):
