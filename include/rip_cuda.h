@@ -48,11 +48,17 @@ typedef struct rip_event rip_event;    /* cudaEvent_t wrapper;  replaces cl_even
 typedef struct rip_ticket rip_ticket;  /* one job in flight in the host-buffer pipeline (rip_submit / rip_collect) */
 
 /* pixel formats of the interleaved u8 images */
-enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5, RIP_FMT_BGRA8 = 6, RIP_FMT_NV12 = 7 };
+enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5, RIP_FMT_BGRA8 = 6, RIP_FMT_NV12 = 7,
+       RIP_FMT_NV12_COLOR = 8 };
 /* RIP_FMT_NV12 (the reference's camera format, RT/RealtimeImageProcessing.cpp:153): per frame a W*H luma plane
  * followed by the W*H/2 interleaved chroma plane (frame = W*H*3/2 bytes, H even).  Accepted by the EDGE and FUSED
  * operations only; the luma plane is the gray image (one byte per pixel leaves HBM instead of three or four),
- * the chroma plane is never read.  Row bands of an NV12 frame are passed as plain luma rows. */
+ * the chroma plane is never read.  Row bands of an NV12 frame are passed as plain luma rows.
+ * RIP_FMT_NV12_COLOR: the same bytes (W and H even), decoded to colour first, exactly as OpenCV's
+ * cvtColor(COLOR_YUV2RGB_NV12) does (BT.601 limited range, 20-bit fixed point, one U,V pair per 2x2 block); every
+ * operation then gives the reference's result on that colour image: GRAYSCALE its gray, GAUSSIAN the blur of the
+ * RGBA image with alpha 255 (W*H*4 bytes out), EDGE / FUSED their result on its gray.  Whole frames only (no row bands);
+ * rip_gray and rip_convert take it on device buffers, rip_sobel / rip_fused do not (decode with rip_gray first). */
 
 /* operations (the reference's METHOD strings "GRAYSCALE" / "GAUSSIAN" / "EDGE", plus "FUSED") */
 enum { RIP_OP_GRAY = 0, RIP_OP_EDGE = 1, RIP_OP_GAUSSIAN = 2, RIP_OP_FUSED = 3 };
@@ -126,9 +132,16 @@ int rip_gauss_weights(int ksize, float sigma, float *weights /* ksize*ksize, hos
  *      All asynchronous on `stream` of `device`. ---- */
 
 /* d_out[i] = (uchar)(0.299*r + 0.587*g + 0.114*b) (double, truncation).  in_format: RGB8 / RGBA8 /
- * BGR8 / BGRA8.  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or RIP_GRAY_OUT_RGBA (w*h*4). */
+ * BGR8 / BGRA8, or NV12_COLOR (decoded in the same kernel).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
+ * RIP_GRAY_OUT_RGBA (w*h*4). */
 int rip_gray(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
              int height, int n_frames, int in_format, int out_mode);
+
+/* Colour conversion of whole frames: in_format RIP_FMT_NV12_COLOR (width and height even), out_format RGB8 / BGR8 / RGBA8
+ * (alpha 255) / BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _BGR / _RGBA / _BGRA), bit for bit.  d_out: w*h*3 or
+ * w*h*4 bytes per frame. */
+int rip_convert(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
+                int n_frames, int in_format, int out_format);
 
 /* K x K float32 convolution per channel in the reference's summation order, clamp-to-edge,
  * truncation.  channels: 1 (gray) or 4 (RGBA, all four channels blurred).  weights: host pointer
@@ -139,7 +152,8 @@ int rip_gauss(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out
 
 /* 3x3 Sobel magnitude, BORDER_REFLECT_101, round-half-even, saturate (OpenCV semantics).
  * in_format GRAY8 runs on the image as is; RGB8/RGBA8/BGR8/BGRA8 first convert with rip_gray's
- * arithmetic inside the same kernel.  d_out: w*h bytes per frame. */
+ * arithmetic inside the same kernel.  d_out: w*h bytes per frame.  NV12_COLOR: RIP_EUNSUPPORTED (rip_gray with
+ * RIP_GRAY_OUT_U8 first, then GRAY8); the same holds for rip_fused. */
 int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int in_format);
 

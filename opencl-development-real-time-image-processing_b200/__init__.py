@@ -20,11 +20,11 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("RIP_LIB_PATH") or os.path.join(_PKG, "librip_cuda.so")
 
 # ---- constants (include/rip_cuda.h) ----
-FMT_GRAY8, FMT_RGB8, FMT_RGBA8, FMT_BGR8, FMT_BGRA8, FMT_NV12 = 1, 3, 4, 5, 6, 7
+FMT_GRAY8, FMT_RGB8, FMT_RGBA8, FMT_BGR8, FMT_BGRA8, FMT_NV12, FMT_NV12_COLOR = 1, 3, 4, 5, 6, 7, 8
 OP_GRAY, OP_EDGE, OP_GAUSSIAN, OP_FUSED = 0, 1, 2, 3
 GRAY_OUT_U8, GRAY_OUT_RGBA = 0, 1
 MAX_KSIZE = 31
-CHANNELS = {FMT_GRAY8: 1, FMT_RGB8: 3, FMT_BGR8: 3, FMT_RGBA8: 4, FMT_BGRA8: 4, FMT_NV12: 1}
+CHANNELS = {FMT_GRAY8: 1, FMT_RGB8: 3, FMT_BGR8: 3, FMT_RGBA8: 4, FMT_BGRA8: 4, FMT_NV12: 1, FMT_NV12_COLOR: 1}
 
 # every symbol include/rip_cuda.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -36,7 +36,7 @@ ABI_SYMBOLS = [
     "rip_event_create", "rip_event_destroy", "rip_event_record", "rip_event_sync", "rip_event_elapsed_ns",
     "rip_malloc_device", "rip_free_device", "rip_malloc_pinned", "rip_free_pinned",
     "rip_memcpy_h2d_async", "rip_memcpy_d2h_async", "rip_memset_device_async",
-    "rip_gauss_weights", "rip_gray", "rip_gauss", "rip_sobel", "rip_fused", "rip_fused_workspace_bytes",
+    "rip_gauss_weights", "rip_gray", "rip_convert", "rip_gauss", "rip_sobel", "rip_fused", "rip_fused_workspace_bytes",
     "rip_launch_count", "rip_debug_slow_path_stats", "rip_debug_selftest", "rip_debug_set_option",
     "rip_out_bytes_per_frame", "rip_process_host", "rip_process_host_banded", "rip_shard_frames", "rip_band_rows",
     "rip_submit", "rip_ticket_done", "rip_collect", "rip_host_register", "rip_host_unregister",
@@ -106,6 +106,7 @@ def lib() -> C.CDLL:
         "rip_memset_device_async": ([C.c_int, vp, C.c_int, C.c_size_t, vp], C.c_int),
         "rip_gauss_weights": ([C.c_int, C.c_float, f32p], C.c_int),
         "rip_gray": ([C.c_int, vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int], C.c_int),
+        "rip_convert": ([C.c_int, vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int], C.c_int),
         "rip_gauss": ([C.c_int, vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, f32p], C.c_int),
         "rip_sobel": ([C.c_int, vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int], C.c_int),
         "rip_fused": ([C.c_int, vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, f32p,
@@ -321,6 +322,11 @@ def gray_dev(d_in: int, d_out: int, w: int, h: int, n: int, fmt: int, out_mode: 
     check(lib().rip_gray(device, stream, d_in, d_out, w, h, n, fmt, out_mode), "rip_gray")
 
 
+def convert_dev(d_in: int, d_out: int, w: int, h: int, n: int, in_fmt: int, out_fmt: int, device=0, stream=None):
+    """rip_convert: NV12_COLOR frames -> RGB8 / BGR8 / RGBA8 / BGRA8 (OpenCV's cvtColor arithmetic)."""
+    check(lib().rip_convert(device, stream, d_in, d_out, w, h, n, in_fmt, out_fmt), "rip_convert")
+
+
 def gauss_dev(d_in: int, d_out: int, w: int, h: int, n: int, channels: int, ksize: int, weights: np.ndarray,
               device=0, stream=None):
     weights = np.ascontiguousarray(weights, np.float32)
@@ -386,7 +392,7 @@ class Context:
             if a.ndim == 2:
                 a = a[None]
             n, h, w = a.shape
-            if fmt == FMT_NV12:
+            if fmt in (FMT_NV12, FMT_NV12_COLOR):
                 assert h % 3 == 0
                 h = h * 2 // 3
         else:
@@ -407,8 +413,8 @@ class Context:
 
     def process(self, frames: np.ndarray, op: int, fmt: int, *, gray_out=GRAY_OUT_U8, ksize=0, weights=None,
                 out: np.ndarray | None = None, banded: bool = False, prof: bool = False):
-        """frames: (N, H, W, C) or (H, W, C) / (H, W) u8 host array (pageable or pinned); NV12: (N, H*3/2, W) or
-        (H*3/2, W), the luma plane followed by the chroma plane."""
+        """frames: (N, H, W, C) or (H, W, C) / (H, W) u8 host array (pageable or pinned); NV12 / NV12_COLOR: (N, H*3/2, W)
+        or (H*3/2, W), the luma plane followed by the chroma plane."""
         a, d, n, h, w, shape, out, squeeze = self._shapes(frames, op, fmt, gray_out, ksize, weights, out)
         pr = (C.c_uint64 * 6)() if prof else None
         if banded:

@@ -23,6 +23,10 @@ void blur_sep_set_slow_counter(unsigned long long *d_counter);
 int launch_sobel(cudaStream_t s, const uint8_t *src, uint8_t *dst, int W, int H, int n_frames, int fmt,
                  int src_row0, int src_rows, int out_row0, int out_rows);
 
+// rip_nv12.cu -- RIP_FMT_NV12_COLOR frames (W and H even) decoded to an interleaved colour image or to the reference's gray
+enum Nv12Out { NV12_TO_RGB, NV12_TO_BGR, NV12_TO_RGBA, NV12_TO_BGRA, NV12_TO_GRAY, NV12_TO_GRAY_RGBA };
+int launch_nv12(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, Nv12Out to);
+
 // rip_fused.cu -- single-kernel gray -> 5x5 Gaussian -> Sobel (and gray -> Sobel)
 bool fused_supported(int W, int H, int fmt, int ksize /* 5, or 0 = no blur stage */, const uint8_t *d_in, const uint8_t *d_out);
 bool fused_plan_weights(const float *w25, float g[3], float *thr);

@@ -163,13 +163,15 @@ void Controller::_appendProfile(const uint64_t prof_ns[6], std::vector<cl_ulong>
     for (int i = 0; i < 6; i++) profiling_events->push_back(prof_ns[i]);
 }
 
-// bytes of one input frame in `fmt` (NV12: the luma plane followed by the half-height chroma plane), 0 = bad format / shape
+// bytes of one input frame in `fmt` (NV12 / NV12_COLOR: the luma plane followed by the half-height chroma plane), 0 = bad
+// format / shape
 static size_t in_frame_bytes(int fmt, int width, int height)
 {
     const size_t px = (size_t)width * height;
     switch (fmt) {
     case RIP_FMT_GRAY8: return px;
     case RIP_FMT_NV12: return (height & 1) ? 0 : px * 3 / 2;
+    case RIP_FMT_NV12_COLOR: return ((width | height) & 1) ? 0 : px * 3 / 2;
     case RIP_FMT_RGB8: case RIP_FMT_BGR8: return px * 3;
     case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return px * 4;
     default: return 0;
@@ -188,7 +190,7 @@ static unsigned char *prepare_output(const rip_op_desc &desc, const unsigned cha
     }
     const size_t in_frame = in_frame_bytes(desc.in_format, width, height);
     if (in_frame == 0) {
-        logger.log(std::string(what) + ": unsupported input format (NV12 needs an even height)", Logger::LogLevel::ERROR);
+        logger.log(std::string(what) + ": unsupported input format (NV12 needs an even height, NV12_COLOR an even width and height)", Logger::LogLevel::ERROR);
         return nullptr;
     }
     if (in_bytes != (size_t)-1 && in_bytes < in_frame * (size_t)n_frames) {
