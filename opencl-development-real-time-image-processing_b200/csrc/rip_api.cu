@@ -100,17 +100,21 @@ static int channels_of(int fmt)
 {
     switch (fmt) {
     case RIP_FMT_GRAY8: case RIP_FMT_NV12: return 1;   // (NV12: the luma plane is the image)
-    case RIP_FMT_RGB8: case RIP_FMT_BGR8: case RIP_FMT_NV12_COLOR: return 3;   // (NV12_COLOR: decoded to R, G, B; 1.5 bytes per pixel in)
+    case RIP_FMT_RGB8: case RIP_FMT_BGR8: return 3;
     case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return 4;
-    default: return 0;
+    default: return decodes_to_color(fmt) ? 3 : 0;   // (decoded to R, G, B; frame_bytes_of gives the bytes in)
     }
 }
 
 // bytes from one frame of a batch to the next
 static size_t frame_bytes_of(int fmt, int width, int height)
 {
-    if (fmt == RIP_FMT_NV12 || fmt == RIP_FMT_NV12_COLOR) return (size_t)width * height * 3 / 2;
-    return (size_t)width * height * channels_of(fmt);
+    const size_t px = (size_t)width * height;
+    switch (fmt) {
+    case RIP_FMT_NV12: case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return px * 3 / 2;
+    case RIP_FMT_YUYV: case RIP_FMT_UYVY: return px * 2;
+    default: return px * channels_of(fmt);
+    }
 }
 
 static int load_weights(Weights &dst, int ksize, const float *weights, const char *who)
@@ -138,7 +142,7 @@ struct BufSet {
     cudaStream_t stream = nullptr;
     void *d_in = nullptr, *d_out = nullptr;
     size_t in_cap = 0, out_cap = 0;
-    // NV12_COLOR frames decoded to RGBA8 (GAUSSIAN) or GRAY8 (EDGE / FUSED) for the kernel that follows
+    // frames of a decoded format decoded to RGBA8 (GAUSSIAN) or GRAY8 (EDGE / FUSED) for the kernel that follows
     void *d_mid = nullptr;
     size_t mid_cap = 0;
     // pinned staging for callers that hand in pageable memory (std::vector, cv::Mat): allocated on first need
@@ -661,9 +665,9 @@ extern "C" int rip_gray(int device, rip_stream stream, const uint8_t *d_in, uint
     if (out_mode != RIP_GRAY_OUT_U8 && out_mode != RIP_GRAY_OUT_RGBA) return fail(RIP_EINVAL, "rip_gray: bad out_mode %d", out_mode);
     DeviceGuard g(device);
     if (!g.ok) return fail(RIP_ENODEV, "cudaSetDevice(%d) failed", device);
-    if (in_format == RIP_FMT_NV12_COLOR)
-        return launch_nv12((cudaStream_t)stream, d_in, d_out, width, height, n_frames,
-                           out_mode == RIP_GRAY_OUT_RGBA ? NV12_TO_GRAY_RGBA : NV12_TO_GRAY);
+    if (decodes_to_color(in_format))
+        return launch_yuv((cudaStream_t)stream, d_in, d_out, width, height, n_frames, in_format,
+                          out_mode == RIP_GRAY_OUT_RGBA ? YUV_TO_GRAY_RGBA : YUV_TO_GRAY);
     return launch_gray((cudaStream_t)stream, d_in, d_out, (long long)width * height * n_frames, in_format, out_mode, device);
 }
 
@@ -672,24 +676,26 @@ extern "C" int rip_convert(int device, rip_stream stream, const uint8_t *d_in, u
 {
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_convert", d_in, d_out, width, height, n_frames)) return rc;
-    if (in_format != RIP_FMT_NV12_COLOR) return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (only RIP_FMT_NV12_COLOR)", in_format);
-    Nv12Out to;
+    if (!decodes_to_color(in_format))
+        return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (RIP_FMT_NV12_COLOR, YUYV, UYVY or I420)", in_format);
+    YuvOut to;
     switch (out_format) {
-    case RIP_FMT_RGB8: to = NV12_TO_RGB; break;
-    case RIP_FMT_BGR8: to = NV12_TO_BGR; break;
-    case RIP_FMT_RGBA8: to = NV12_TO_RGBA; break;
-    case RIP_FMT_BGRA8: to = NV12_TO_BGRA; break;
+    case RIP_FMT_RGB8: to = YUV_TO_RGB; break;
+    case RIP_FMT_BGR8: to = YUV_TO_BGR; break;
+    case RIP_FMT_RGBA8: to = YUV_TO_RGBA; break;
+    case RIP_FMT_BGRA8: to = YUV_TO_BGRA; break;
     default: return fail(RIP_EUNSUPPORTED, "rip_convert: output format %d (RGB8, BGR8, RGBA8 or BGRA8)", out_format);
     }
     DeviceGuard g(device);
     if (!g.ok) return fail(RIP_ENODEV, "cudaSetDevice(%d) failed", device);
-    return launch_nv12((cudaStream_t)stream, d_in, d_out, width, height, n_frames, to);
+    return launch_yuv((cudaStream_t)stream, d_in, d_out, width, height, n_frames, in_format, to);
 }
 
-static int nv12_color_needs_gray_first(const char *who)
+static int needs_gray_first(const char *who, int fmt)
 {
-    return fail(RIP_EUNSUPPORTED, "%s: RIP_FMT_NV12_COLOR is not taken here; decode with rip_gray(..., RIP_FMT_NV12_COLOR, RIP_GRAY_OUT_U8) "
-                "and pass the result as RIP_FMT_GRAY8", who);
+    const char *name = yuv_format_name(fmt);
+    return fail(RIP_EUNSUPPORTED, "%s: RIP_FMT_%s is not taken here; decode with rip_gray(..., RIP_FMT_%s, RIP_GRAY_OUT_U8) "
+                "and pass the result as RIP_FMT_GRAY8", who, name, name);
 }
 
 extern "C" int rip_gauss(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
@@ -709,7 +715,7 @@ extern "C" int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uin
 {
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_sobel", d_in, d_out, width, height, n_frames)) return rc;
-    if (in_format == RIP_FMT_NV12_COLOR) return nv12_color_needs_gray_first("rip_sobel");
+    if (decodes_to_color(in_format)) return needs_gray_first("rip_sobel", in_format);
     if (channels_of(in_format) == 0) return fail(RIP_EINVAL, "rip_sobel: unsupported input format %d", in_format);
     DeviceGuard g(device);
     if (!g.ok) return fail(RIP_ENODEV, "cudaSetDevice(%d) failed", device);
@@ -737,7 +743,7 @@ extern "C" int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uin
 {
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_fused", d_in, d_out, width, height, n_frames)) return rc;
-    if (in_format == RIP_FMT_NV12_COLOR) return nv12_color_needs_gray_first("rip_fused");
+    if (decodes_to_color(in_format)) return needs_gray_first("rip_fused", in_format);
     if (channels_of(in_format) == 0) return fail(RIP_EINVAL, "rip_fused: unsupported input format %d", in_format);
     Weights wts;
     if (int rc = load_weights(wts, ksize, weights, "rip_fused")) return rc;
@@ -831,7 +837,7 @@ extern "C" int rip_out_bytes_per_frame(const rip_op_desc *desc, int width, int h
     switch (desc->op) {
     case RIP_OP_GRAY: *bytes = desc->gray_out == RIP_GRAY_OUT_RGBA ? px * 4 : px; return RIP_OK;
     case RIP_OP_EDGE: case RIP_OP_FUSED: *bytes = px; return RIP_OK;
-    case RIP_OP_GAUSSIAN: *bytes = px * (desc->in_format == RIP_FMT_NV12_COLOR ? 4 : channels_of(desc->in_format)); return RIP_OK;
+    case RIP_OP_GAUSSIAN: *bytes = px * (decodes_to_color(desc->in_format) ? 4 : channels_of(desc->in_format)); return RIP_OK;
     default: return fail(RIP_EINVAL, "unknown op %d", desc->op);
     }
 }
@@ -850,8 +856,8 @@ int validate_desc(const rip_op_desc *desc, int *cn_out)
     case RIP_OP_EDGE:
         break;
     case RIP_OP_GAUSSIAN:
-        if (((cn != 1 && cn != 4) || desc->in_format == RIP_FMT_NV12) && desc->in_format != RIP_FMT_NV12_COLOR)
-            return fail(RIP_EINVAL, "GAUSSIAN runs on GRAY8, RGBA8/BGRA8 or NV12_COLOR input");
+        if (((cn != 1 && cn != 4) || desc->in_format == RIP_FMT_NV12) && !decodes_to_color(desc->in_format))
+            return fail(RIP_EINVAL, "GAUSSIAN runs on GRAY8, RGBA8/BGRA8, NV12_COLOR, YUYV, UYVY or I420 input");
         if (!desc->weights) return fail(RIP_EINVAL, "GAUSSIAN needs weights");
         break;
     case RIP_OP_FUSED:
@@ -890,14 +896,14 @@ int enqueue_op(const rip_ticket &t, int device, const BufSet &b, int n_frames, c
                              band->out_row0, band->out_rows, nullptr, 0);
         return rip_sobel_rows(device, s, in, out, t.W, t.H, d.in_format, band->in_row0, band->in_rows, band->out_row0, band->out_rows);
     }
-    if (d.in_format == RIP_FMT_NV12_COLOR && d.op != RIP_OP_GRAY) {
+    if (decodes_to_color(d.in_format) && d.op != RIP_OP_GRAY) {
         // decode into the chunk's middle buffer (RGBA8 for the blur, GRAY8 for Sobel / fused), then the existing kernel on it
         uint8_t *mid = (uint8_t *)b.d_mid;
         if (d.op == RIP_OP_GAUSSIAN) {
-            if (int rc = rip_convert(device, s, in, mid, t.W, t.H, n_frames, RIP_FMT_NV12_COLOR, RIP_FMT_RGBA8)) return rc;
+            if (int rc = rip_convert(device, s, in, mid, t.W, t.H, n_frames, d.in_format, RIP_FMT_RGBA8)) return rc;
             return rip_gauss(device, s, mid, out, t.W, t.H, n_frames, 4, d.ksize, d.weights);
         }
-        if (int rc = rip_gray(device, s, in, mid, t.W, t.H, n_frames, RIP_FMT_NV12_COLOR, RIP_GRAY_OUT_U8)) return rc;
+        if (int rc = rip_gray(device, s, in, mid, t.W, t.H, n_frames, d.in_format, RIP_GRAY_OUT_U8)) return rc;
         in = mid;
         if (d.op == RIP_OP_EDGE) return rip_sobel(device, s, in, out, t.W, t.H, n_frames, RIP_FMT_GRAY8);
         return rip_fused(device, s, in, out, t.W, t.H, n_frames, RIP_FMT_GRAY8, d.ksize, d.weights, 0, t.H, 0, t.H, nullptr, 0);
@@ -984,7 +990,7 @@ void issue_part(DevState &dev, Part *p)
         uint8_t *dst = band ? t.h_out + (size_t)t.W * p->out_row0 : t.h_out + (size_t)(p->f0 + c0) * t.out_frame_bytes;
         if ((rc = ensure(&b.d_in, &b.in_cap, in_bytes))) break;
         if ((rc = ensure(&b.d_out, &b.out_cap, out_bytes))) break;
-        if (t.desc.in_format == RIP_FMT_NV12_COLOR && t.desc.op != RIP_OP_GRAY &&
+        if (decodes_to_color(t.desc.in_format) && t.desc.op != RIP_OP_GRAY &&
             (rc = ensure(&b.d_mid, &b.mid_cap, (size_t)t.W * t.H * cf * (t.desc.op == RIP_OP_GAUSSIAN ? 4 : 1))))
             break;
         if (!t.in_pinned) {   // pageable source: stage through pinned memory (the copy overlaps the DMA of the previous chunk)
@@ -1122,12 +1128,12 @@ extern "C" int rip_submit(rip_ctx *ctx, const rip_op_desc *desc, const uint8_t *
     int cn = 0;
     if (int rc = validate_desc(desc, &cn)) return rc;
     if (desc->in_format == RIP_FMT_NV12 && (height & 1)) return fail(RIP_EINVAL, "NV12 frames need an even height (got %d)", height);
-    if (desc->in_format == RIP_FMT_NV12_COLOR && ((width | height) & 1))
-        return fail(RIP_EINVAL, "NV12_COLOR frames need an even width and height (got %d x %d)", width, height);
+    if (decodes_to_color(desc->in_format))
+        if (int rc = check_yuv_shape(desc->in_format, width, height)) return rc;
     const bool banded = (flags & RIP_SUBMIT_BANDED) != 0;
     if (banded) {
-        if (desc->in_format == RIP_FMT_NV12_COLOR)
-            return fail(RIP_EUNSUPPORTED, "row-band mode does not take NV12_COLOR (its bands carry luma rows only)");
+        if (decodes_to_color(desc->in_format))
+            return fail(RIP_EUNSUPPORTED, "row-band mode does not take %s (it decodes whole frames only)", yuv_format_name(desc->in_format));
         if (n_frames != 1) return fail(RIP_EINVAL, "row-band mode takes one frame per call (got %d)", n_frames);
         if (desc->op != RIP_OP_FUSED && desc->op != RIP_OP_EDGE) return fail(RIP_EUNSUPPORTED, "row-band mode supports FUSED and EDGE only");
     }

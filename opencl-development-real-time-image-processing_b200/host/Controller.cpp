@@ -163,15 +163,16 @@ void Controller::_appendProfile(const uint64_t prof_ns[6], std::vector<cl_ulong>
     for (int i = 0; i < 6; i++) profiling_events->push_back(prof_ns[i]);
 }
 
-// bytes of one input frame in `fmt` (NV12 / NV12_COLOR: the luma plane followed by the half-height chroma plane), 0 = bad
-// format / shape
+// bytes of one input frame in `fmt` (NV12 / NV12_COLOR / I420: the luma plane followed by chroma of half its size; YUYV /
+// UYVY: two bytes per pixel), 0 = bad format / shape
 static size_t in_frame_bytes(int fmt, int width, int height)
 {
     const size_t px = (size_t)width * height;
     switch (fmt) {
     case RIP_FMT_GRAY8: return px;
     case RIP_FMT_NV12: return (height & 1) ? 0 : px * 3 / 2;
-    case RIP_FMT_NV12_COLOR: return ((width | height) & 1) ? 0 : px * 3 / 2;
+    case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return ((width | height) & 1) ? 0 : px * 3 / 2;
+    case RIP_FMT_YUYV: case RIP_FMT_UYVY: return (width & 1) ? 0 : px * 2;
     case RIP_FMT_RGB8: case RIP_FMT_BGR8: return px * 3;
     case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return px * 4;
     default: return 0;
@@ -190,7 +191,8 @@ static unsigned char *prepare_output(const rip_op_desc &desc, const unsigned cha
     }
     const size_t in_frame = in_frame_bytes(desc.in_format, width, height);
     if (in_frame == 0) {
-        logger.log(std::string(what) + ": unsupported input format (NV12 needs an even height, NV12_COLOR an even width and height)", Logger::LogLevel::ERROR);
+        logger.log(std::string(what) + ": unsupported input format (NV12 needs an even height, NV12_COLOR and I420 an even width and height, "
+                   "YUYV and UYVY an even width)", Logger::LogLevel::ERROR);
         return nullptr;
     }
     if (in_bytes != (size_t)-1 && in_bytes < in_frame * (size_t)n_frames) {

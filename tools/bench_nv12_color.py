@@ -1,14 +1,16 @@
 #!/usr/bin/env python
-"""Times of the NV12_COLOR paths: the decode kernels on device-resident data, the decode's share of GAUSSIAN, and the end-to-end
-host pipeline with NV12_COLOR against RGBA8 input.
+"""Times of the decoded camera formats: the NV12_COLOR, YUYV, UYVY and I420 decode kernels on device-resident data (the NV12_COLOR
+legs are the same-session control for the others), the decode's share of GAUSSIAN, and the end-to-end host pipeline with
+NV12_COLOR and YUYV against RGBA8 / BGR8 input.
 
-    python tools/bench_nv12_color.py [--launches 21] > profiles/nv12_color_b200.txt
+    python tools/bench_nv12_color.py [--launches 21] > profiles/yuv_color_b200.txt
 
 Kernel legs: CUDA events around each launch, 3 warm-up launches, the median of --launches (>= 20) launches; 32 x 3840x2160
-frames are 398 MB of NV12 in and up to 1 GB out, far above the 126 MB L2.  Algorithmic bytes per pixel: 1.5 in + the output's
-bytes per pixel out.  The share of peak is against the 6.55 TB/s device-to-device copy peak measured on a B200 (DESIGN.md).
+frames are 398 MB of NV12 / I420 or 531 MB of YUYV / UYVY in and up to 1 GB out, far above the 126 MB L2.  Algorithmic bytes
+per pixel: 1.5 (4:2:0) or 2 (4:2:2) in + the output's bytes per pixel out.  The share of peak is against the 6.55 TB/s device-to-device copy peak measured on a B200 (DESIGN.md).
 End-to-end legs: rip_process_host from pinned host memory, wall clock over --e2e-steps blocking calls after 2 warm-up calls.
-A sample of every timed output (first, middle and last frame) is checked against tests/nv12_ref.py and the C oracle.
+A sample of every timed output (first, middle and last frame) is checked against tests/nv12_ref.py / tests/yuv_ref.py and the C
+oracle.
 """
 import argparse
 import os
@@ -22,6 +24,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     sys.path.insert(0, p)
 import nv12_ref as R  # noqa: E402
+import yuv_ref as YR  # noqa: E402
 import oracle as O  # noqa: E402
 import rip_b200 as rip  # noqa: E402
 
@@ -107,7 +110,39 @@ for mode, bpp in ((rip.GRAY_OUT_U8, 1), (rip.GRAY_OUT_RGBA, 4)):
         g = O.gray(R.decode(nv[i]), threads=0)
         got = d_out.download((H, W) if bpp == 1 else (H, W, 4), offset=i * H * W * bpp)
         check(f"gray frame {i}", got if bpp == 1 else got[..., 0], g)
-del d_in, d_out
+del d_in
+
+
+def packed_422(nv12, layout):
+    """The camera-like NV12 frames as YUYV / UYVY: the same luma, each chroma row serving two luma rows."""
+    out = np.empty((nv12.shape[0], H, W, 2), np.uint8)
+    for i, f in enumerate(nv12):
+        uv = np.repeat(f[H:].reshape(H // 2, W // 2, 2), 2, 0)
+        out[i] = YR.packed_from_planes(f[:H], uv[..., 0], uv[..., 1], layout)
+    return out
+
+
+# ---- the other layouts, 32 x 4K: YUYV / UYVY (4:2:2, 2 B/px in) and I420 (4:2:0 planar, 1.5 B/px in) ---------------------------
+LEGS = {"yuyv": (("rgba", "rgb"), True), "uyvy": (("rgba",), False), "i420": (("rgba",), True)}
+for layout, (orders, with_gray) in LEGS.items():
+    fmt = {"yuyv": rip.FMT_YUYV, "uyvy": rip.FMT_UYVY, "i420": rip.FMT_I420}[layout]
+    src = np.stack([YR.i420_from_nv12(f) for f in nv]) if layout == "i420" else packed_422(nv, layout)
+    in_b = src.nbytes / px
+    d_in = rip.DeviceBuffer(src.nbytes).upload(src)
+    for order in orders:
+        ofmt = {"rgba": rip.FMT_RGBA8, "rgb": rip.FMT_RGB8}[order]
+        us, best = timed(lambda: rip.convert_dev(d_in.ptr, d_out.ptr, W, H, N, fmt, ofmt))
+        row(f"rip_convert {layout.upper()} -> {order.upper()}8, {N} x {W}x{H}", us, best, px, in_b + len(order))
+        fb = H * W * len(order)
+        for i in sample:
+            check(f"convert {layout} {order} frame {i}", d_out.download((H, W, len(order)), offset=i * fb), YR.decode(src[i], layout, order))
+    if with_gray:
+        us, best = timed(lambda: rip.gray_dev(d_in.ptr, d_out.ptr, W, H, N, fmt, rip.GRAY_OUT_U8))
+        row(f"rip_gray {layout.upper()} -> u8, {N} x {W}x{H}", us, best, px, in_b + 1)
+        for i in sample:
+            check(f"gray {layout} frame {i}", d_out.download((H, W), offset=i * H * W), O.gray(YR.decode(src[i], layout), threads=0))
+    del d_in, src
+del d_out
 
 # ---- GAUSSIAN 5x5 on 16 x 1080p: decode + blur against the blur alone on RGBA8 ----------------------------------------------------
 N, H, W = 16, 1080, 1920
@@ -141,9 +176,14 @@ del d_nv, d_rgba, d_blur
 ctx = rip.Context([0])
 rgba = R.to_rgba(R.decode(nv))
 print(f"# end to end, rip_process_host, pinned host buffers, {N} x {W}x{H}, wall clock over {a.e2e_steps} calls", flush=True)
-for op, name, kw in ((rip.OP_GRAY, "GRAY", {}), (rip.OP_GAUSSIAN, "GAUSSIAN 5x5", {"ksize": 5, "weights": wt})):
+yuyv = packed_422(nv, "yuyv")
+bgr = R.decode(nv, "bgr")
+NAMES = {rip.FMT_NV12_COLOR: "NV12_COLOR", rip.FMT_YUYV: "YUYV", rip.FMT_BGR8: "BGR8", rip.FMT_RGBA8: "RGBA8"}
+for op, name, kw, inputs in ((rip.OP_GRAY, "GRAY", {}, ((rip.FMT_NV12_COLOR, nv), (rip.FMT_YUYV, yuyv), (rip.FMT_BGR8, bgr),
+                                                        (rip.FMT_RGBA8, rgba))),
+                             (rip.OP_GAUSSIAN, "GAUSSIAN 5x5", {"ksize": 5, "weights": wt}, ((rip.FMT_NV12_COLOR, nv), (rip.FMT_RGBA8, rgba)))):
     res = {}
-    for fmt, src in ((rip.FMT_NV12_COLOR, nv), (rip.FMT_RGBA8, rgba)):
+    for fmt, src in inputs:
         h_in = rip.PinnedBuffer(src.nbytes)
         a_in = h_in.array.reshape(src.shape)
         a_in[...] = src
@@ -158,12 +198,15 @@ for op, name, kw in ((rip.OP_GRAY, "GRAY", {}), (rip.OP_GAUSSIAN, "GAUSSIAN 5x5"
         dt = (time.perf_counter() - t0) / a.e2e_steps
         res[fmt] = (dt, a_out.copy())
         in_b = src.nbytes / px
-        print(f"  {name:13s} {'NV12_COLOR' if fmt == rip.FMT_NV12_COLOR else 'RGBA8':10s} {dt * 1e3:8.2f} ms/call  "
+        print(f"  {name:13s} {NAMES[fmt]:10s} {dt * 1e3:8.2f} ms/call  "
               f"{px / dt / 1e9:6.2f} Gpx/s  ({in_b:.1f} B/px in, {out_bpp} B/px out)", flush=True)
         del a_in, a_out
         h_in.free()
         h_out.free()
-    check(f"e2e {name}: NV12_COLOR vs RGBA8 of the decoded frames", res[rip.FMT_NV12_COLOR][1], res[rip.FMT_RGBA8][1])
-    print(f"  {name}: NV12_COLOR / RGBA8 speed {res[rip.FMT_RGBA8][0] / res[rip.FMT_NV12_COLOR][0]:.2f}x", flush=True)
+    for fmt in res:
+        check(f"e2e {name}: {NAMES[fmt]} vs RGBA8 of the decoded frames", res[fmt][1], res[rip.FMT_RGBA8][1])
+    for fmt in [f for f in res if f not in (rip.FMT_RGBA8, rip.FMT_BGR8)]:
+        for ref in [f for f in (rip.FMT_RGBA8, rip.FMT_BGR8) if f in res]:
+            print(f"  {name}: {NAMES[fmt]} / {NAMES[ref]} speed {res[ref][0] / res[fmt][0]:.2f}x", flush=True)
 ctx.close()
 print("# every sampled output equal to the reference")
