@@ -49,7 +49,8 @@ typedef struct rip_ticket rip_ticket;  /* one job in flight in the host-buffer p
 
 /* pixel formats of the interleaved u8 images */
 enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5, RIP_FMT_BGRA8 = 6, RIP_FMT_NV12 = 7,
-       RIP_FMT_NV12_COLOR = 8, RIP_FMT_YUYV = 9, RIP_FMT_UYVY = 10, RIP_FMT_I420 = 11 };
+       RIP_FMT_NV12_COLOR = 8, RIP_FMT_YUYV = 9, RIP_FMT_UYVY = 10, RIP_FMT_I420 = 11,
+       RIP_FMT_BAYER_RGGB8 = 12, RIP_FMT_BAYER_BGGR8 = 13, RIP_FMT_BAYER_GRBG8 = 14, RIP_FMT_BAYER_GBRG8 = 15 };
 /* RIP_FMT_NV12 (the reference's camera format, RT/RealtimeImageProcessing.cpp:153): per frame a W*H luma plane
  * followed by the W*H/2 interleaved chroma plane (frame = W*H*3/2 bytes, H even).  Accepted by the EDGE and FUSED
  * operations only; the luma plane is the gray image (one byte per pixel leaves HBM instead of three or four),
@@ -67,7 +68,14 @@ enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5,
  *   UYVY: the same with bytes U Y0 V Y1 (HDMI / SDI capture cards, many CSI sensors); W even, any H.
  *   I420: planar 4:2:0: the W*H luma plane, then the (W/2)*(H/2) U plane, then the V plane (frame = W*H*3/2 bytes);
  *         W and H even.  FFmpeg's yuv420p, GStreamer's I420.
- * None of the four has a luma-only meaning (RIP_FMT_NV12 is that for NV12). */
+ * None of the four has a luma-only meaning (RIP_FMT_NV12 is that for NV12).
+ * RIP_FMT_BAYER_RGGB8 / _BGGR8 / _GRBG8 / _GBRG8: 8-bit Bayer raw frames, W*H bytes per frame (one byte per pixel,
+ * row-major, frames consecutive), W >= 3 and H >= 3 of any parity; what machine-vision cameras (GenICam BayerRG8 ...) and
+ * raw CSI sensors (V4L2 SRGGB8 ...) deliver.  Named by the sensor's top-left 2x2, as V4L2 and GenICam name them; OpenCV
+ * names a pattern by the 2x2 at (1, 1), so the same result comes from its COLOR_BayerBG2RGB (RGGB), COLOR_BayerRG2RGB (BGGR),
+ * COLOR_BayerGB2RGB (GRBG) and COLOR_BayerGR2RGB (GBRG), and their 2BGR / 2RGBA / 2BGRA forms.  Demosaiced exactly as
+ * OpenCV's default (bilinear) cvtColor does it, border pixels copying their interior neighbour, and taken everywhere
+ * NV12_COLOR is, with the same results on the decoded image (GAUSSIAN: W*H*4 bytes out). */
 
 /* operations (the reference's METHOD strings "GRAYSCALE" / "GAUSSIAN" / "EDGE", plus "FUSED") */
 enum { RIP_OP_GRAY = 0, RIP_OP_EDGE = 1, RIP_OP_GAUSSIAN = 2, RIP_OP_FUSED = 3 };
@@ -141,14 +149,15 @@ int rip_gauss_weights(int ksize, float sigma, float *weights /* ksize*ksize, hos
  *      All asynchronous on `stream` of `device`. ---- */
 
 /* d_out[i] = (uchar)(0.299*r + 0.587*g + 0.114*b) (double, truncation).  in_format: RGB8 / RGBA8 /
- * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 (decoded in the same kernel).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
+ * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 / BAYER_* (decoded in the same kernel).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
  * RIP_GRAY_OUT_RGBA (w*h*4). */
 int rip_gray(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
              int height, int n_frames, int in_format, int out_mode);
 
 /* Colour conversion of whole frames: in_format RIP_FMT_NV12_COLOR or RIP_FMT_I420 (width and height even), RIP_FMT_YUYV or
- * RIP_FMT_UYVY (width even), out_format RGB8 / BGR8 / RGBA8 (alpha 255) / BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 /
- * _BGR / _RGBA / _BGRA, and the same for _I420, _YUYV, _UYVY), bit for bit.  d_out: w*h*3 or w*h*4 bytes per frame. */
+ * RIP_FMT_UYVY (width even), RIP_FMT_BAYER_* (width and height at least 3), out_format RGB8 / BGR8 / RGBA8 (alpha 255) /
+ * BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _BGR / _RGBA / _BGRA, and the same for _I420, _YUYV, _UYVY; the Bayer
+ * conversions listed with the formats), bit for bit.  d_out: w*h*3 or w*h*4 bytes per frame. */
 int rip_convert(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
                 int n_frames, int in_format, int out_format);
 
@@ -161,7 +170,7 @@ int rip_gauss(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out
 
 /* 3x3 Sobel magnitude, BORDER_REFLECT_101, round-half-even, saturate (OpenCV semantics).
  * in_format GRAY8 runs on the image as is; RGB8/RGBA8/BGR8/BGRA8 first convert with rip_gray's
- * arithmetic inside the same kernel.  d_out: w*h bytes per frame.  NV12_COLOR, YUYV, UYVY, I420: RIP_EUNSUPPORTED (rip_gray
+ * arithmetic inside the same kernel.  d_out: w*h bytes per frame.  NV12_COLOR, YUYV, UYVY, I420, BAYER_*: RIP_EUNSUPPORTED (rip_gray
  * with RIP_GRAY_OUT_U8 first, then GRAY8); the same holds for rip_fused. */
 int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int in_format);

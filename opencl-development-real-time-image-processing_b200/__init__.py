@@ -22,13 +22,16 @@ LIB_PATH = os.environ.get("RIP_LIB_PATH") or os.path.join(_PKG, "librip_cuda.so"
 # ---- constants (include/rip_cuda.h) ----
 FMT_GRAY8, FMT_RGB8, FMT_RGBA8, FMT_BGR8, FMT_BGRA8, FMT_NV12, FMT_NV12_COLOR = 1, 3, 4, 5, 6, 7, 8
 FMT_YUYV, FMT_UYVY, FMT_I420 = 9, 10, 11
+# 8-bit Bayer raw frames, named by the sensor's top-left 2x2 (V4L2 SRGGB8 / SBGGR8 / SGRBG8 / SGBRG8, GenICam BayerRG8 / ...)
+FMT_BAYER_RGGB8, FMT_BAYER_BGGR8, FMT_BAYER_GRBG8, FMT_BAYER_GBRG8 = 12, 13, 14, 15
 OP_GRAY, OP_EDGE, OP_GAUSSIAN, OP_FUSED = 0, 1, 2, 3
 GRAY_OUT_U8, GRAY_OUT_RGBA = 0, 1
 MAX_KSIZE = 31
-# bytes per pixel of the host array's last axis; 1 for the planar formats, whose frames are (H*3/2, W) arrays.  YUYV and UYVY
-# are (H, W, 2): the CV_8UC2 Mat that V4L2 capture returns with CAP_PROP_CONVERT_RGB off.
+# bytes per pixel of the host array's last axis; 1 for the planar formats, whose frames are (H*3/2, W) arrays, and for Bayer
+# frames, (H, W) arrays.  YUYV and UYVY are (H, W, 2): the CV_8UC2 Mat that V4L2 capture returns with CAP_PROP_CONVERT_RGB off.
 CHANNELS = {FMT_GRAY8: 1, FMT_RGB8: 3, FMT_BGR8: 3, FMT_RGBA8: 4, FMT_BGRA8: 4, FMT_NV12: 1, FMT_NV12_COLOR: 1,
-            FMT_YUYV: 2, FMT_UYVY: 2, FMT_I420: 1}
+            FMT_YUYV: 2, FMT_UYVY: 2, FMT_I420: 1,
+            FMT_BAYER_RGGB8: 1, FMT_BAYER_BGGR8: 1, FMT_BAYER_GRBG8: 1, FMT_BAYER_GBRG8: 1}
 
 # every symbol include/rip_cuda.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -323,13 +326,14 @@ class Event:
 
 # ---- device-resident ops on raw device pointers (ints) ----
 def gray_dev(d_in: int, d_out: int, w: int, h: int, n: int, fmt: int, out_mode: int = GRAY_OUT_U8, device=0, stream=None):
-    """rip_gray: the reference's gray of RGB8 / BGR8 / RGBA8 / BGRA8 frames, or of NV12_COLOR, YUYV, UYVY or I420 frames
-    decoded in the same kernel."""
+    """rip_gray: the reference's gray of RGB8 / BGR8 / RGBA8 / BGRA8 frames, or of NV12_COLOR, YUYV, UYVY, I420 or Bayer
+    frames decoded in the same kernel."""
     check(lib().rip_gray(device, stream, d_in, d_out, w, h, n, fmt, out_mode), "rip_gray")
 
 
 def convert_dev(d_in: int, d_out: int, w: int, h: int, n: int, in_fmt: int, out_fmt: int, device=0, stream=None):
-    """rip_convert: NV12_COLOR, YUYV, UYVY or I420 frames -> RGB8 / BGR8 / RGBA8 / BGRA8 (OpenCV's cvtColor arithmetic)."""
+    """rip_convert: NV12_COLOR, YUYV, UYVY, I420 or Bayer frames -> RGB8 / BGR8 / RGBA8 / BGRA8 (OpenCV's cvtColor
+    arithmetic; Bayer: its default bilinear demosaic)."""
     check(lib().rip_convert(device, stream, d_in, d_out, w, h, n, in_fmt, out_fmt), "rip_convert")
 
 
@@ -420,7 +424,8 @@ class Context:
     def process(self, frames: np.ndarray, op: int, fmt: int, *, gray_out=GRAY_OUT_U8, ksize=0, weights=None,
                 out: np.ndarray | None = None, banded: bool = False, prof: bool = False):
         """frames: (N, H, W, C) or (H, W, C) / (H, W) u8 host array (pageable or pinned); NV12 / NV12_COLOR / I420:
-        (N, H*3/2, W) or (H*3/2, W), the luma plane followed by the chroma planes; YUYV / UYVY: (N, H, W, 2) or (H, W, 2)."""
+        (N, H*3/2, W) or (H*3/2, W), the luma plane followed by the chroma planes; YUYV / UYVY: (N, H, W, 2) or (H, W, 2);
+        Bayer: (N, H, W) or (H, W), one raw byte per pixel."""
         a, d, n, h, w, shape, out, squeeze = self._shapes(frames, op, fmt, gray_out, ksize, weights, out)
         pr = (C.c_uint64 * 6)() if prof else None
         if banded:

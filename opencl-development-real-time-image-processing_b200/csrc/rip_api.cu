@@ -113,6 +113,7 @@ static size_t frame_bytes_of(int fmt, int width, int height)
     switch (fmt) {
     case RIP_FMT_NV12: case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return px * 3 / 2;
     case RIP_FMT_YUYV: case RIP_FMT_UYVY: return px * 2;
+    case RIP_FMT_BAYER_RGGB8: case RIP_FMT_BAYER_BGGR8: case RIP_FMT_BAYER_GRBG8: case RIP_FMT_BAYER_GBRG8: return px;
     default: return px * channels_of(fmt);
     }
 }
@@ -677,7 +678,7 @@ extern "C" int rip_convert(int device, rip_stream stream, const uint8_t *d_in, u
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_convert", d_in, d_out, width, height, n_frames)) return rc;
     if (!decodes_to_color(in_format))
-        return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (RIP_FMT_NV12_COLOR, YUYV, UYVY or I420)", in_format);
+        return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (RIP_FMT_NV12_COLOR, YUYV, UYVY, I420 or BAYER_*8)", in_format);
     YuvOut to;
     switch (out_format) {
     case RIP_FMT_RGB8: to = YUV_TO_RGB; break;
@@ -857,7 +858,7 @@ int validate_desc(const rip_op_desc *desc, int *cn_out)
         break;
     case RIP_OP_GAUSSIAN:
         if (((cn != 1 && cn != 4) || desc->in_format == RIP_FMT_NV12) && !decodes_to_color(desc->in_format))
-            return fail(RIP_EINVAL, "GAUSSIAN runs on GRAY8, RGBA8/BGRA8, NV12_COLOR, YUYV, UYVY or I420 input");
+            return fail(RIP_EINVAL, "GAUSSIAN runs on GRAY8, RGBA8/BGRA8, NV12_COLOR, YUYV, UYVY, I420 or Bayer input");
         if (!desc->weights) return fail(RIP_EINVAL, "GAUSSIAN needs weights");
         break;
     case RIP_OP_FUSED:

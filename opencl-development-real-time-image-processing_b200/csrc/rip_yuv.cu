@@ -1,5 +1,6 @@
 // rip_yuv.cu -- camera frames (RIP_FMT_NV12_COLOR, RIP_FMT_I420, RIP_FMT_YUYV, RIP_FMT_UYVY) decoded to colour, or straight
-// to the reference's gray.
+// to the reference's gray.  launch_yuv is also the entry for the Bayer formats, whose kernels are in rip_bayer.cu; the
+// output side of both (packing, gray, stores) is rip_decode.cuh.
 //
 // Colour is OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _I420 / _YUYV / _UYVY): BT.601 limited range in 20-bit fixed point.  The
 // four layouts differ only in where Y, U and V sit (one U,V pair per 2x2 block of luma for NV12 and I420, per horizontal
@@ -18,27 +19,10 @@
 // one cvt.pack.sat per two bytes (I2IP.U8.S32.SAT).  Widths that are not a multiple of 8 and unaligned buffers take
 // byte-granular kernels (one 2x2 block, or one pixel pair, per thread).  Frames ride in gridDim.y.  Memory-bound by intent:
 // 1.5 (4:2:0) or 2 (4:2:2) bytes per pixel in, 1..4 out.
-#include "rip_common.cuh"
-#include "rip_internal.h"
+#include "rip_decode.cuh"
 
 namespace rip {
 namespace {
-
-__constant__ uint32_t c_yuv_gray_down[2048] = {
-#include "rip_gray_table.inc"
-};
-
-// d = (c & 0xffff) << 16 | sat_u8(a) << 8 | sat_u8(b)
-__device__ __forceinline__ uint32_t i2ip(int a, int b, uint32_t c)
-{
-    uint32_t d;
-    asm("cvt.pack.sat.u8.s32.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-
-// bytes b0..b3 (low to high), each saturated to [0, 255]
-__device__ __forceinline__ uint32_t pack4(int b0, int b1, int b2, int b3) { return i2ip(b1, b0, i2ip(b3, b2, 0u)); }
-__device__ __forceinline__ uint32_t pack4(uint32_t b0, uint32_t b1, uint32_t b2, uint32_t b3) { return pack4((int)b0, (int)b1, (int)b2, (int)b3); }
 
 struct Chroma {
     int r, g, b;   // chroma part of each channel, with the rounding constant
@@ -50,55 +34,11 @@ __device__ __forceinline__ Chroma chroma_of(uint32_t U, uint32_t V)
     return {(1 << 19) + 1673527 * v, (1 << 19) - 852492 * v - 409993 * u, (1 << 19) + 2116026 * u};
 }
 
-// unsaturated R, G, B of one pixel (the >> is arithmetic, as in OpenCV)
-struct Rgb {
-    int r, g, b;
-};
-
 // Y16 = max(Y - 16, 0), already subtracted (four at a time, __vsubus4)
 __device__ __forceinline__ Rgb decode(uint32_t Y16, const Chroma &c)
 {
     const int y = (int)Y16 * 1220542;
     return {(y + c.r) >> 20, (y + c.g) >> 20, (y + c.b) >> 20};
-}
-
-constexpr float kInvK_up = 1.0000000474974513e-3f;   // 0x3A83126F: the float just ABOVE 1/1000
-constexpr float kInvK_dn = 9.9999993108212948e-4f;   // 0x3A83126E: the float just BELOW 1/1000
-
-// The reference's gray of a decoded pixel, from its saturated bytes (r, g, b, 0).  t = 299 r + 587 g + 114 b by two IDP.2A;
-// floor(t / 1000) as in the fused kernel: t's bit pattern read as a float is the denormal t * 2^-149, one multiply rounded
-// toward -inf by the float just above 1/1000 leaves floor(t / 1000) in the bit pattern, and a multiply-add rounded toward +inf
-// with the float just below 1/1000 is 1 exactly when t is a nonzero multiple of 1000 (rip_debug_selftest checks the same
-// arithmetic on all 2^24 triples).  Only there can the reference's double expression land one below t / 1000, as the (r, g)
-// table bit says.
-__device__ __forceinline__ uint32_t gray_of(uint32_t rgb0)
-{
-    const uint32_t t = __dp2a_hi(114u, rgb0, __dp2a_lo(299u | (587u << 16), rgb0, 0u));
-    const float tf = __uint_as_float(t);
-    const uint32_t q = __float_as_uint(__fmul_rd(tf, kInvK_up));
-    if (__float_as_uint(__fmaf_ru(tf, -kInvK_dn, __uint_as_float(q))) != 1u) return q;
-    const uint32_t key = rgb0 & 0xffffu;
-    return q - ((c_yuv_gray_down[key >> 5] >> (key & 31u)) & 1u);
-}
-
-template <int OUT> struct OutFmt;
-template <> struct OutFmt<YUV_TO_RGB> { static constexpr int bpp = 3; };
-template <> struct OutFmt<YUV_TO_BGR> { static constexpr int bpp = 3; };
-template <> struct OutFmt<YUV_TO_RGBA> { static constexpr int bpp = 4; };
-template <> struct OutFmt<YUV_TO_BGRA> { static constexpr int bpp = 4; };
-template <> struct OutFmt<YUV_TO_GRAY> { static constexpr int bpp = 1; };
-template <> struct OutFmt<YUV_TO_GRAY_RGBA> { static constexpr int bpp = 4; };
-
-// the output bytes of one pixel; bpp bytes, low byte first
-template <int OUT>
-__device__ __forceinline__ uint32_t pixel_word(const Rgb &p)
-{
-    if constexpr (OUT == YUV_TO_RGBA) return pack4(p.r, p.g, p.b, 255);
-    else if constexpr (OUT == YUV_TO_BGRA) return pack4(p.b, p.g, p.r, 255);
-    else if constexpr (OUT == YUV_TO_GRAY) return gray_of(pack4(p.r, p.g, p.b, 0));
-    else if constexpr (OUT == YUV_TO_GRAY_RGBA) return gray_of(pack4(p.r, p.g, p.b, 0)) * 0x010101u | 0xff000000u;
-    else if constexpr (OUT == YUV_TO_RGB) return pack4(p.r, p.g, p.b, 0);
-    else return pack4(p.b, p.g, p.r, 0);
 }
 
 // Eight pixels of one row.  Y: max(Y - 16, 0) of pixels 0..3 and 4..7, low byte first; UV: the U,V byte pairs (U low)
@@ -116,33 +56,9 @@ __device__ __forceinline__ void row_x8(uint32_t px[8], const uint32_t Y[2], cons
     }
 }
 
-// the eight pixels to o: 8-byte aligned (16-byte for 4 bytes per pixel)
-template <int OUT>
-__device__ __forceinline__ void store_x8(uint8_t *o, const uint32_t px[8])
-{
-    if constexpr (OutFmt<OUT>::bpp == 4) {
-        reinterpret_cast<uint4 *>(o)[0] = make_uint4(px[0], px[1], px[2], px[3]);
-        reinterpret_cast<uint4 *>(o)[1] = make_uint4(px[4], px[5], px[6], px[7]);
-    } else if constexpr (OutFmt<OUT>::bpp == 1) {
-        *reinterpret_cast<uint2 *>(o) = make_uint2(pack4(px[0], px[1], px[2], px[3]), pack4(px[4], px[5], px[6], px[7]));
-    } else {   // 24 bytes: the 3-byte pixels back to back
-        uint2 *o2 = reinterpret_cast<uint2 *>(o);
-        o2[0] = make_uint2(px[0] | px[1] << 24, px[1] >> 8 | px[2] << 16);
-        o2[1] = make_uint2(px[2] >> 16 | px[3] << 8, px[4] | px[5] << 24);
-        o2[2] = make_uint2(px[5] >> 8 | px[6] << 16, px[6] >> 16 | px[7] << 8);
-    }
-}
-
-// one pixel of luma Y (not yet reduced by 16), and its byte stores
+// one pixel of luma Y (not yet reduced by 16)
 template <int OUT>
 __device__ __forceinline__ uint32_t pixel_of(uint32_t Y, const Chroma &ch) { return pixel_word<OUT>(decode(max((int)Y - 16, 0), ch)); }
-
-template <int OUT>
-__device__ __forceinline__ void store_px(uint8_t *o, uint32_t v)
-{
-#pragma unroll
-    for (int b = 0; b < OutFmt<OUT>::bpp; b++) o[b] = (uint8_t)(v >> (8 * b));
-}
 
 // 4:2:0 chroma of frame f, after its W*H luma plane: NV12 interleaves U,V in one plane of W bytes per row; I420 keeps a U
 // plane and then a V plane, each of W/2 bytes per row and (W/2) * (H/2) bytes.  chroma_at is the U byte of pair `pair` of
@@ -308,6 +224,10 @@ const char *yuv_format_name(int fmt)
     case RIP_FMT_YUYV: return "YUYV";
     case RIP_FMT_UYVY: return "UYVY";
     case RIP_FMT_I420: return "I420";
+    case RIP_FMT_BAYER_RGGB8: return "BAYER_RGGB8";
+    case RIP_FMT_BAYER_BGGR8: return "BAYER_BGGR8";
+    case RIP_FMT_BAYER_GRBG8: return "BAYER_GRBG8";
+    case RIP_FMT_BAYER_GBRG8: return "BAYER_GBRG8";
     default: return "(not a YUV format)";
     }
 }
@@ -315,8 +235,11 @@ const char *yuv_format_name(int fmt)
 int check_yuv_shape(int fmt, int W, int H)
 {
     const char *name = yuv_format_name(fmt);
-    long long units;   // 2x2 blocks or pixel pairs of one frame
-    if (fmt == RIP_FMT_YUYV || fmt == RIP_FMT_UYVY) {
+    long long units;   // 2x2 blocks, pixel pairs or (Bayer) pixels of one frame
+    if (is_bayer(fmt)) {   // the demosaic's 3x3 neighbourhood
+        if (W < 3 || H < 3) return fail(RIP_EINVAL, "%s frames need a width and height of at least 3 (got %d x %d)", name, W, H);
+        units = (long long)W * H;
+    } else if (fmt == RIP_FMT_YUYV || fmt == RIP_FMT_UYVY) {
         if (W & 1) return fail(RIP_EINVAL, "%s frames need an even width (got %d x %d)", name, W, H);
         units = (long long)H * (W / 2);
     } else if (fmt == RIP_FMT_NV12_COLOR || fmt == RIP_FMT_I420) {
@@ -333,6 +256,7 @@ int check_yuv_shape(int fmt, int W, int H)
 int launch_yuv(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, int in_format, YuvOut to)
 {
     if (int rc = check_yuv_shape(in_format, W, H)) return rc;
+    if (is_bayer(in_format)) return launch_bayer(s, in, out, W, H, n_frames, in_format, to);
     switch (in_format) {
     case RIP_FMT_NV12_COLOR: return launch_fmt<RIP_FMT_NV12_COLOR>(s, in, out, W, H, n_frames, to);
     case RIP_FMT_I420: return launch_fmt<RIP_FMT_I420>(s, in, out, W, H, n_frames, to);

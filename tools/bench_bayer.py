@@ -1,0 +1,189 @@
+#!/usr/bin/env python
+"""Times of the Bayer demosaic: the decode kernels on device-resident data, the decode's share of GAUSSIAN, and the end-to-end
+host pipeline from Bayer against RGB8 and NV12_COLOR input.
+
+    python tools/bench_bayer.py [--launches 21] > profiles/bayer_b200.txt
+
+Kernel legs: CUDA events around each launch, 3 warm-up launches, the median of --launches (>= 20) launches; 32 x 3840x2160
+Bayer frames are 265 MB in and up to 1.06 GB out, far above the 126 MB L2.  Algorithmic bytes per pixel: 1 in + the output's
+bytes per pixel out.  The share of peak is against the 6.55 TB/s device-to-device copy peak measured on a B200 (DESIGN.md).
+The gray leg is compared, in the same run, with the two-kernel route a caller has without it: rip_convert to RGB8, then
+rip_gray on RGB8.
+End-to-end legs: rip_process_host from pinned host memory, wall clock over --e2e-steps blocking calls after 2 warm-up calls.
+A sample of every timed output (first, middle and last frame) is checked against tests/bayer_ref.py and the C oracle.
+"""
+import argparse
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
+    sys.path.insert(0, p)
+import bayer_ref as R  # noqa: E402
+import nv12_ref  # noqa: E402
+import oracle as O  # noqa: E402
+import rip_b200 as rip  # noqa: E402
+
+PEAK_GBS = 6550.0
+
+ap = argparse.ArgumentParser()
+ap.add_argument("--launches", type=int, default=21)
+ap.add_argument("--e2e-steps", type=int, default=10)
+a = ap.parse_args()
+assert a.launches >= 20
+if rip.device_count() < 1:
+    sys.exit("bench_bayer.py needs a CUDA device (there is no CPU fallback)")
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception as e:   # noqa: BLE001
+        q = f"nvidia-smi unavailable ({e})"
+    return f"{rip.device_info(0).name.decode()}; nvidia-smi: {q}"
+
+
+def timed(fn, n=a.launches, warm=3):
+    for _ in range(warm):
+        fn()
+    ts = []
+    for _ in range(n):
+        e0, e1 = rip.Event(), rip.Event()
+        e0.record()
+        fn()
+        e1.record()
+        e1.sync()
+        ts.append(e0.elapsed_ns(e1) / 1e3)
+    ts.sort()
+    return ts[len(ts) // 2], ts[0]
+
+
+def row(name, us, best, px, bpp, floor_note=True):
+    gbs = px * bpp / us / 1e3
+    floor = px * bpp / PEAK_GBS / 1e3
+    extra = f"  floor {floor:7.1f} us  {100 * gbs / PEAK_GBS:5.1f} % of {PEAK_GBS:.0f} GB/s" if floor_note else ""
+    print(f"{name:58s} {us:9.1f} us (best {best:8.1f})  {gbs:8.1f} GB/s ({bpp} B/px){extra}", flush=True)
+
+
+def camera_like(n, h, w, seed):
+    """Raw frames of a smooth scene with sensor noise (a demosaic is data-independent; the blur after it is not)."""
+    rng = np.random.default_rng(seed)
+    yy, xx = np.mgrid[0:h, 0:w].astype(np.float32)
+    one = np.clip(120 + 90 * np.sin(0.01 * xx + 0.007 * yy) + rng.integers(-3, 4, (h, w)), 0, 255).astype(np.uint8)
+    return np.stack([np.roll(one, 37 * i, axis=1) for i in range(n)])
+
+
+def check(name, got, want):
+    if not np.array_equal(got, want):
+        raise SystemExit(f"{name}: timed output differs from the reference ({int((got != want).sum())} bytes)")
+
+
+print(f"# {card()}")
+print(f"# median of {a.launches} launches after 3 warm-up launches (CUDA events); copy peak {PEAK_GBS:.0f} GB/s", flush=True)
+
+# ---- decode kernels, 32 x 4K RGGB ---------------------------------------------------------------------------------------------
+N, H, W = 32, 2160, 3840
+px = N * H * W
+FMT = rip.FMT_BAYER_RGGB8
+raw = camera_like(N, H, W, 1)
+d_in = rip.DeviceBuffer(raw.nbytes).upload(raw)
+d_out = rip.DeviceBuffer(px * 4)
+d_rgb = rip.DeviceBuffer(px * 3)
+sample = (0, N // 2, N - 1)
+want_rgb = {i: R.decode(raw[i], "rggb") for i in sample}
+for order, fmt in (("rgba", rip.FMT_RGBA8), ("rgb", rip.FMT_RGB8)):
+    us, best = timed(lambda: rip.convert_dev(d_in.ptr, d_out.ptr, W, H, N, FMT, fmt))
+    row(f"rip_convert BAYER_RGGB8 -> {order.upper()}8, {N} x {W}x{H}", us, best, px, 1 + len(order))
+    fb = H * W * len(order)
+    for i in sample:
+        want = want_rgb[i] if order == "rgb" else np.concatenate([want_rgb[i], np.full((H, W, 1), 255, np.uint8)], -1)
+        check(f"convert {order} frame {i}", d_out.download((H, W, len(order)), offset=i * fb), want)
+want_gray = {i: O.gray(want_rgb[i], threads=0) for i in sample}
+us_gray, best = timed(lambda: rip.gray_dev(d_in.ptr, d_out.ptr, W, H, N, FMT, rip.GRAY_OUT_U8))
+row(f"rip_gray BAYER_RGGB8 -> u8, {N} x {W}x{H}", us_gray, best, px, 2)
+for i in sample:
+    check(f"gray frame {i}", d_out.download((H, W), offset=i * H * W), want_gray[i])
+
+
+def two_kernels():
+    rip.convert_dev(d_in.ptr, d_rgb.ptr, W, H, N, FMT, rip.FMT_RGB8)
+    rip.gray_dev(d_rgb.ptr, d_out.ptr, W, H, N, rip.FMT_RGB8, rip.GRAY_OUT_U8)
+
+
+us_two, best = timed(two_kernels)
+row(f"rip_convert -> RGB8, then rip_gray RGB8 -> u8, {N} x {W}x{H}", us_two, best, px, 2, floor_note=False)
+print(f"  rip_gray on Bayer is {us_two / us_gray:.2f}x faster than the two-kernel route", flush=True)
+for i in sample:
+    check(f"two-kernel gray frame {i}", d_out.download((H, W), offset=i * H * W), want_gray[i])
+us, best = timed(lambda: rip.convert_dev(d_in.ptr, d_out.ptr, W, H, N, rip.FMT_BAYER_GBRG8, rip.FMT_RGBA8))
+row(f"rip_convert BAYER_GBRG8 -> RGBA8, {N} x {W}x{H}", us, best, px, 5)
+del d_in, d_out, d_rgb, raw
+
+# ---- GAUSSIAN 5x5 on 16 x 1080p: demosaic + blur against the blur alone on RGBA8 ---------------------------------------------------
+N, H, W = 16, 1080, 1920
+px = N * H * W
+raw = camera_like(N, H, W, 2)
+wt = rip.gauss_weights(5, 1.0)
+d_raw = rip.DeviceBuffer(raw.nbytes).upload(raw)
+d_rgba = rip.DeviceBuffer(px * 4)
+d_blur = rip.DeviceBuffer(px * 4)
+rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, FMT, rip.FMT_RGBA8)
+us_blur, best = timed(lambda: rip.gauss_dev(d_rgba.ptr, d_blur.ptr, W, H, N, 4, 5, wt))
+row(f"GAUSSIAN 5x5 blur alone, RGBA8, {N} x {W}x{H}", us_blur, best, px, 8)
+us_dec, best = timed(lambda: rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, FMT, rip.FMT_RGBA8))
+row(f"demosaic BAYER_RGGB8 -> RGBA8, {N} x {W}x{H}", us_dec, best, px, 5)
+
+
+def both():
+    rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, FMT, rip.FMT_RGBA8)
+    rip.gauss_dev(d_rgba.ptr, d_blur.ptr, W, H, N, 4, 5, wt)
+
+
+us_both, best = timed(both)
+row(f"demosaic + GAUSSIAN 5x5, BAYER_RGGB8, {N} x {W}x{H}", us_both, best, px, 5, floor_note=False)
+print(f"  demosaic adds {us_both - us_blur:.1f} us = {100 * (us_both - us_blur) / us_blur:.1f} % of the blur alone", flush=True)
+for i in (0, N - 1):
+    check(f"blur frame {i}", d_blur.download((H, W, 4), offset=i * H * W * 4),
+          O.blur(R.decode(raw[i], "rggb", "rgba"), 5, weights=wt, threads=0))
+del d_raw, d_rgba, d_blur
+
+# ---- end to end from pinned memory: Bayer against RGB8 (the same decoded image) and NV12_COLOR --------------------------------------
+ctx = rip.Context([0])
+rgb = R.decode(raw, "rggb")
+nv = np.empty((N, H * 3 // 2, W), np.uint8)
+nv[:, :H] = raw
+nv[:, H:] = 128   # neutral chroma; the NV12 leg is timed only
+print(f"# end to end, rip_process_host, pinned host buffers, {N} x {W}x{H}, wall clock over {a.e2e_steps} calls", flush=True)
+NAMES = {FMT: "BAYER_RGGB8", rip.FMT_RGB8: "RGB8", rip.FMT_NV12_COLOR: "NV12_COLOR"}
+for op, name, kw in ((rip.OP_GRAY, "GRAY", {}), (rip.OP_EDGE, "EDGE", {}), (rip.OP_FUSED, "FUSED 5x5", {"ksize": 5, "weights": wt})):
+    res = {}
+    for fmt, src in ((FMT, raw), (rip.FMT_RGB8, rgb), (rip.FMT_NV12_COLOR, nv)):
+        h_in = rip.PinnedBuffer(src.nbytes)
+        a_in = h_in.array.reshape(src.shape)
+        a_in[...] = src
+        h_out = rip.PinnedBuffer(px)
+        a_out = h_out.array.reshape((N, H, W))
+        for _ in range(2):
+            ctx.process(a_in, op, fmt, out=a_out, **kw)
+        t0 = time.perf_counter()
+        for _ in range(a.e2e_steps):
+            ctx.process(a_in, op, fmt, out=a_out, **kw)
+        dt = (time.perf_counter() - t0) / a.e2e_steps
+        res[fmt] = (dt, a_out.copy())
+        print(f"  {name:10s} {NAMES[fmt]:12s} {dt * 1e3:8.2f} ms/call  {px / dt / 1e9:6.2f} Gpx/s  "
+              f"({src.nbytes / px:.1f} B/px in, 1 B/px out)", flush=True)
+        del a_in, a_out
+        h_in.free()
+        h_out.free()
+    check(f"e2e {name}: BAYER_RGGB8 vs RGB8 of the decoded frames", res[FMT][1], res[rip.FMT_RGB8][1])
+    if op == rip.OP_GRAY:
+        check("e2e GRAY NV12_COLOR", res[rip.FMT_NV12_COLOR][1][0], O.gray(nv12_ref.decode(nv[0]), threads=0))
+    for ref in (rip.FMT_RGB8, rip.FMT_NV12_COLOR):
+        print(f"  {name}: BAYER_RGGB8 / {NAMES[ref]} speed {res[ref][0] / res[FMT][0]:.2f}x", flush=True)
+ctx.close()
+print("# every sampled output equal to the reference")
