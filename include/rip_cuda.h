@@ -50,7 +50,11 @@ typedef struct rip_ticket rip_ticket;  /* one job in flight in the host-buffer p
 /* pixel formats of the interleaved u8 images */
 enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5, RIP_FMT_BGRA8 = 6, RIP_FMT_NV12 = 7,
        RIP_FMT_NV12_COLOR = 8, RIP_FMT_YUYV = 9, RIP_FMT_UYVY = 10, RIP_FMT_I420 = 11,
-       RIP_FMT_BAYER_RGGB8 = 12, RIP_FMT_BAYER_BGGR8 = 13, RIP_FMT_BAYER_GRBG8 = 14, RIP_FMT_BAYER_GBRG8 = 15 };
+       RIP_FMT_BAYER_RGGB8 = 12, RIP_FMT_BAYER_BGGR8 = 13, RIP_FMT_BAYER_GRBG8 = 14, RIP_FMT_BAYER_GBRG8 = 15,
+       RIP_FMT_BAYER_RGGB10 = 16, RIP_FMT_BAYER_BGGR10 = 17, RIP_FMT_BAYER_GRBG10 = 18, RIP_FMT_BAYER_GBRG10 = 19,
+       RIP_FMT_BAYER_RGGB12 = 20, RIP_FMT_BAYER_BGGR12 = 21, RIP_FMT_BAYER_GRBG12 = 22, RIP_FMT_BAYER_GBRG12 = 23,
+       RIP_FMT_BAYER_RGGB14 = 24, RIP_FMT_BAYER_BGGR14 = 25, RIP_FMT_BAYER_GRBG14 = 26, RIP_FMT_BAYER_GBRG14 = 27,
+       RIP_FMT_BAYER_RGGB16 = 28, RIP_FMT_BAYER_BGGR16 = 29, RIP_FMT_BAYER_GRBG16 = 30, RIP_FMT_BAYER_GBRG16 = 31 };
 /* RIP_FMT_NV12 (the reference's camera format, RT/RealtimeImageProcessing.cpp:153): per frame a W*H luma plane
  * followed by the W*H/2 interleaved chroma plane (frame = W*H*3/2 bytes, H even).  Accepted by the EDGE and FUSED
  * operations only; the luma plane is the gray image (one byte per pixel leaves HBM instead of three or four),
@@ -75,7 +79,16 @@ enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5,
  * names a pattern by the 2x2 at (1, 1), so the same result comes from its COLOR_BayerBG2RGB (RGGB), COLOR_BayerRG2RGB (BGGR),
  * COLOR_BayerGB2RGB (GRBG) and COLOR_BayerGR2RGB (GBRG), and their 2BGR / 2RGBA / 2BGRA forms.  Demosaiced exactly as
  * OpenCV's default (bilinear) cvtColor does it, border pixels copying their interior neighbour, and taken everywhere
- * NV12_COLOR is, with the same results on the decoded image (GAUSSIAN: W*H*4 bytes out). */
+ * NV12_COLOR is, with the same results on the decoded image (GAUSSIAN: W*H*4 bytes out).
+ * RIP_FMT_BAYER_<pattern>10 / 12 / 14 / 16 (codes 16-31, patterns in the same order as 12-15 within each depth): Bayer raw
+ * frames of b = 10, 12, 14 or 16 bits per sample, W*H little-endian 16-bit words per frame (2*W*H bytes, row-major, frames
+ * consecutive), W >= 3 and H >= 3 of any parity; what V4L2 SRGGB10 / 12 / 14 / 16 ... and GenICam BayerRG10 / 12 / 14 / 16 ...
+ * (unpacked) deliver.  Samples are LSB-aligned, as V4L2 and GenICam store them; a stream whose samples are MSB-aligned is a
+ * 16-bit stream to this decode (use the *16 code).  The decode is OpenCV's cvtColor(COLOR_Bayer**2RGB) on the CV_16U frame
+ * (the 8-bit formulas on the full samples, the same pattern names) followed by convertTo(CV_8U, 1.0 / (1 << (b - 8))): each
+ * channel divided by 2^(b-8), rounded half to even, saturated (a full-scale sample gives 255; padding bits above bit b-1 are
+ * used as they are, and saturate); alpha 255.  Taken everywhere the 8-bit Bayer formats are, with the same results on that
+ * 8-bit image.  Packed RAW10 / RAW12 are not taken. */
 
 /* operations (the reference's METHOD strings "GRAYSCALE" / "GAUSSIAN" / "EDGE", plus "FUSED") */
 enum { RIP_OP_GRAY = 0, RIP_OP_EDGE = 1, RIP_OP_GAUSSIAN = 2, RIP_OP_FUSED = 3 };
@@ -149,15 +162,17 @@ int rip_gauss_weights(int ksize, float sigma, float *weights /* ksize*ksize, hos
  *      All asynchronous on `stream` of `device`. ---- */
 
 /* d_out[i] = (uchar)(0.299*r + 0.587*g + 0.114*b) (double, truncation).  in_format: RGB8 / RGBA8 /
- * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 / BAYER_* (decoded in the same kernel).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
+ * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 / BAYER_* of any depth (decoded in the same kernel; 16-bit samples:
+ * 2*w*h bytes in per frame, any alignment).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
  * RIP_GRAY_OUT_RGBA (w*h*4). */
 int rip_gray(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
              int height, int n_frames, int in_format, int out_mode);
 
 /* Colour conversion of whole frames: in_format RIP_FMT_NV12_COLOR or RIP_FMT_I420 (width and height even), RIP_FMT_YUYV or
- * RIP_FMT_UYVY (width even), RIP_FMT_BAYER_* (width and height at least 3), out_format RGB8 / BGR8 / RGBA8 (alpha 255) /
- * BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _BGR / _RGBA / _BGRA, and the same for _I420, _YUYV, _UYVY; the Bayer
- * conversions listed with the formats), bit for bit.  d_out: w*h*3 or w*h*4 bytes per frame. */
+ * RIP_FMT_UYVY (width even), RIP_FMT_BAYER_* of 8 to 16 bits (width and height at least 3), out_format RGB8 / BGR8 / RGBA8
+ * (alpha 255) / BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _BGR / _RGBA / _BGRA, and the same for _I420, _YUYV, _UYVY;
+ * the Bayer conversions listed with the formats, followed for 10 to 16 bits by convertTo(CV_8U, 1.0 / (1 << (b - 8)))),
+ * bit for bit.  d_in and d_out may have any alignment.  d_out: w*h*3 or w*h*4 bytes per frame. */
 int rip_convert(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
                 int n_frames, int in_format, int out_format);
 

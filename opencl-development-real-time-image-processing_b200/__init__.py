@@ -24,14 +24,24 @@ FMT_GRAY8, FMT_RGB8, FMT_RGBA8, FMT_BGR8, FMT_BGRA8, FMT_NV12, FMT_NV12_COLOR = 
 FMT_YUYV, FMT_UYVY, FMT_I420 = 9, 10, 11
 # 8-bit Bayer raw frames, named by the sensor's top-left 2x2 (V4L2 SRGGB8 / SBGGR8 / SGRBG8 / SGBRG8, GenICam BayerRG8 / ...)
 FMT_BAYER_RGGB8, FMT_BAYER_BGGR8, FMT_BAYER_GRBG8, FMT_BAYER_GBRG8 = 12, 13, 14, 15
+# 10- to 16-bit Bayer raw frames, one little-endian uint16 per sample, LSB-aligned (V4L2 SRGGB10 ... SGBRG16, GenICam
+# BayerRG10 ... BayerGB16, unpacked); MSB-aligned samples are a 16-bit stream
+FMT_BAYER_RGGB10, FMT_BAYER_BGGR10, FMT_BAYER_GRBG10, FMT_BAYER_GBRG10 = 16, 17, 18, 19
+FMT_BAYER_RGGB12, FMT_BAYER_BGGR12, FMT_BAYER_GRBG12, FMT_BAYER_GBRG12 = 20, 21, 22, 23
+FMT_BAYER_RGGB14, FMT_BAYER_BGGR14, FMT_BAYER_GRBG14, FMT_BAYER_GBRG14 = 24, 25, 26, 27
+FMT_BAYER_RGGB16, FMT_BAYER_BGGR16, FMT_BAYER_GRBG16, FMT_BAYER_GBRG16 = 28, 29, 30, 31
+# the formats whose host arrays are uint16 (every other format takes uint8)
+FMTS_U16 = frozenset(range(FMT_BAYER_RGGB10, FMT_BAYER_GBRG16 + 1))
 OP_GRAY, OP_EDGE, OP_GAUSSIAN, OP_FUSED = 0, 1, 2, 3
 GRAY_OUT_U8, GRAY_OUT_RGBA = 0, 1
 MAX_KSIZE = 31
-# bytes per pixel of the host array's last axis; 1 for the planar formats, whose frames are (H*3/2, W) arrays, and for Bayer
-# frames, (H, W) arrays.  YUYV and UYVY are (H, W, 2): the CV_8UC2 Mat that V4L2 capture returns with CAP_PROP_CONVERT_RGB off.
+# elements per pixel of the host array's last axis; 1 for the planar formats, whose frames are (H*3/2, W) arrays, and for Bayer
+# frames, (H, W) arrays (uint16 for 10 to 16 bits).  YUYV and UYVY are (H, W, 2): the CV_8UC2 Mat that V4L2 capture returns
+# with CAP_PROP_CONVERT_RGB off.
 CHANNELS = {FMT_GRAY8: 1, FMT_RGB8: 3, FMT_BGR8: 3, FMT_RGBA8: 4, FMT_BGRA8: 4, FMT_NV12: 1, FMT_NV12_COLOR: 1,
             FMT_YUYV: 2, FMT_UYVY: 2, FMT_I420: 1,
-            FMT_BAYER_RGGB8: 1, FMT_BAYER_BGGR8: 1, FMT_BAYER_GRBG8: 1, FMT_BAYER_GBRG8: 1}
+            FMT_BAYER_RGGB8: 1, FMT_BAYER_BGGR8: 1, FMT_BAYER_GRBG8: 1, FMT_BAYER_GBRG8: 1,
+            **{f: 1 for f in FMTS_U16}}
 
 # every symbol include/rip_cuda.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -327,13 +337,13 @@ class Event:
 # ---- device-resident ops on raw device pointers (ints) ----
 def gray_dev(d_in: int, d_out: int, w: int, h: int, n: int, fmt: int, out_mode: int = GRAY_OUT_U8, device=0, stream=None):
     """rip_gray: the reference's gray of RGB8 / BGR8 / RGBA8 / BGRA8 frames, or of NV12_COLOR, YUYV, UYVY, I420 or Bayer
-    frames decoded in the same kernel."""
+    frames (8 to 16 bits) decoded in the same kernel."""
     check(lib().rip_gray(device, stream, d_in, d_out, w, h, n, fmt, out_mode), "rip_gray")
 
 
 def convert_dev(d_in: int, d_out: int, w: int, h: int, n: int, in_fmt: int, out_fmt: int, device=0, stream=None):
     """rip_convert: NV12_COLOR, YUYV, UYVY, I420 or Bayer frames -> RGB8 / BGR8 / RGBA8 / BGRA8 (OpenCV's cvtColor
-    arithmetic; Bayer: its default bilinear demosaic)."""
+    arithmetic; Bayer: its default bilinear demosaic, then for 10 to 16 bits convertTo(CV_8U, 1 / 2^(bits - 8)))."""
     check(lib().rip_convert(device, stream, d_in, d_out, w, h, n, in_fmt, out_fmt), "rip_convert")
 
 
@@ -396,7 +406,12 @@ class Context:
 
     def _shapes(self, frames: np.ndarray, op, fmt, gray_out, ksize, weights, out):
         a = frames
-        assert a.dtype == np.uint8 and a.flags["C_CONTIGUOUS"]
+        if fmt in FMTS_U16:
+            assert a.dtype == np.dtype("<u2"), \
+                f"format {fmt} (10- to 16-bit Bayer) takes native little-endian uint16 arrays, got {a.dtype.str}"
+        else:
+            assert a.dtype == np.uint8, f"format {fmt} takes uint8 arrays, got {a.dtype}"
+        assert a.flags["C_CONTIGUOUS"]
         cn = CHANNELS[fmt]
         if cn == 1:
             if a.ndim == 2:
@@ -425,7 +440,8 @@ class Context:
                 out: np.ndarray | None = None, banded: bool = False, prof: bool = False):
         """frames: (N, H, W, C) or (H, W, C) / (H, W) u8 host array (pageable or pinned); NV12 / NV12_COLOR / I420:
         (N, H*3/2, W) or (H*3/2, W), the luma plane followed by the chroma planes; YUYV / UYVY: (N, H, W, 2) or (H, W, 2);
-        Bayer: (N, H, W) or (H, W), one raw byte per pixel."""
+        Bayer: (N, H, W) or (H, W), one raw byte per pixel (uint8) for the 8-bit formats, one little-endian uint16 per pixel
+        for 10 to 16 bits.  Every other format takes uint8."""
         a, d, n, h, w, shape, out, squeeze = self._shapes(frames, op, fmt, gray_out, ksize, weights, out)
         pr = (C.c_uint64 * 6)() if prof else None
         if banded:

@@ -1,5 +1,6 @@
 // rip_bayer.cu -- 8-bit Bayer raw frames (RIP_FMT_BAYER_RGGB8, _BGGR8, _GRBG8, _GBRG8) demosaiced to colour, or straight to
-// the reference's gray.  launch_yuv (rip_yuv.cu) checks the shape and calls launch_bayer.
+// the reference's gray, and the same for 10- to 16-bit samples (RIP_FMT_BAYER_RGGB10 ... _GBRG16; their section below).
+// launch_yuv (rip_yuv.cu) checks the shape and calls launch_bayer.
 //
 // The demosaic is OpenCV's default (bilinear) cvtColor(COLOR_Bayer**2RGB), bit for bit.  For an interior pixel with raw
 // byte c, h the sum of its left and right neighbours, v the sum of the pixels above and below, n = h + v and d the sum of the
@@ -145,46 +146,187 @@ bayer_kernel_x1(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, int W
     store_px<OUT>(out + (frame + (size_t)y * W + x) * OutFmt<OUT>::bpp, pixel_word<OUT>(rgb));
 }
 
-template <int OUT, int FMT>
-int launch_t(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames)
+// ---- 10- to 16-bit samples (RIP_FMT_BAYER_RGGB10 ... _GBRG16): W*H little-endian 16-bit words per frame, LSB-aligned ------
+// The decode is OpenCV's cvtColor(COLOR_Bayer**2RGB) on the CV_16U frame followed by convertTo(CV_8U, 1.0 / 2^shift), with
+// shift = bits - 8: the same formulas on the full 16-bit samples, then each channel divided by 2^shift, rounded half to even
+// and saturated (a full-scale 10-bit 1023 gives 255.75, so 256, so 255; padding bits above the depth are used as they are).
+// The sums stay in 32-bit lanes (four 16-bit samples need 18 bits).  The pattern and the output are template parameters, as
+// above; the shift is a kernel argument, so the four depths share one kernel per pattern and output.
+
+// v / 2^shift rounded half to even, for shift >= 1 (the saturation is pack4's); half_m1 = 2^(shift - 1) - 1
+__device__ __forceinline__ int reduce16(int v, int shift, int half_m1) { return (v + half_m1 + ((v >> shift) & 1)) >> shift; }
+
+__device__ __forceinline__ Rgb reduce16(const Rgb &p, int shift, int half_m1)
 {
-    const uintptr_t out_align = OutFmt<OUT>::bpp == 4 ? 15u : 7u;
-    const bool x8 = (W & 7) == 0 && (reinterpret_cast<uintptr_t>(in) & 7u) == 0 && (reinterpret_cast<uintptr_t>(out) & out_align) == 0;
+    return {reduce16(p.r, shift, half_m1), reduce16(p.g, shift, half_m1), reduce16(p.b, shift, half_m1)};
+}
+
+// One raw row as seen by a thread: its 8 samples (two per word, low half first), and the sample on either side.
+struct Row16 {
+    uint4 w;
+    uint32_t l, r;
+};
+
+// sample j of the row, j = -1 .. 8
+__device__ __forceinline__ int at(const Row16 &q, int j)
+{
+    if (j < 0) return (int)q.l;
+    if (j > 7) return (int)q.r;
+    const uint32_t word = j < 2 ? q.w.x : j < 4 ? q.w.y : j < 6 ? q.w.z : q.w.w;
+    return (int)((word >> (16 * (j & 1))) & 0xffffu);
+}
+
+// row_x8 for 16-bit samples: the same sums and sites, then the reduction to 8 bits
+template <int OUT, int FMT, int P>
+__device__ __forceinline__ void row16_x8(uint32_t px[8], const Row16 &a, const Row16 &m, const Row16 &b, int shift, int half_m1)
+{
+    using Pat = Pattern<FMT>;
+    int vs[10];
+#pragma unroll
+    for (int j = 0; j < 10; j++) vs[j] = at(a, j - 1) + at(b, j - 1);
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const int h = at(m, i - 1) + at(m, i + 1);
+        const Rgb rgb = site(P == Pat::ry, (i & 1) == Pat::rx, at(m, i), h, vs[i + 1], vs[i] + vs[i + 2]);
+        px[i] = pixel_word<OUT>(reduce16(rgb, shift, half_m1));
+    }
+}
+
+// bayer_kernel_x8's shape for 16-bit samples (W % 8 == 0, input 16-byte aligned, output as there): a row pair x 8 columns per
+// thread, one 128-bit load per raw row, and the halo samples of the four rows in two shuffles each way (rows 0, 1 and rows
+// 2, 3 share a word), the warp's two edge lanes loading theirs.  FMT is the 8-bit code of the same pattern.
+template <int OUT, int FMT>
+__global__ void __launch_bounds__(256)
+bayer16_kernel_x8(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, int W, int H, int f0, int shift)
+{
+    constexpr int BPP = OutFmt<OUT>::bpp;
+    const int cols = W >> 3, pairs = (H + 1) >> 1;
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    const int c = u % cols;
+    const bool live = u / cols < pairs;
+    const int y0 = 2 * min(u / cols, pairs - 1);
+    const int s0 = min(max(y0, 1), H - 2);
+    const int s1 = min(max(y0 + 1, 1), H - 2);
+    const size_t frame = ((size_t)f0 + blockIdx.y) * W * H;   // in pixels
+    const uint16_t *base = reinterpret_cast<const uint16_t *>(in) + frame + 8 * c;
+    const int lane = threadIdx.x & 31;
+    uint4 w[4];   // raw rows s0 - 1 .. s0 + 2
+#pragma unroll
+    for (int i = 0; i < 4; i++) w[i] = __ldg(reinterpret_cast<const uint4 *>(base + (size_t)min(s0 - 1 + i, H - 1) * W));
+    // halo words: the last samples (left halo of lane + 1) or first samples (right halo of lane - 1) of rows 0, 1 and of 2, 3
+    uint32_t left01 = __shfl_up_sync(0xffffffffu, __byte_perm(w[0].w, w[1].w, 0x7632), 1);
+    uint32_t left23 = __shfl_up_sync(0xffffffffu, __byte_perm(w[2].w, w[3].w, 0x7632), 1);
+    uint32_t right01 = __shfl_down_sync(0xffffffffu, __byte_perm(w[0].x, w[1].x, 0x5410), 1);
+    uint32_t right23 = __shfl_down_sync(0xffffffffu, __byte_perm(w[2].x, w[3].x, 0x5410), 1);
+    if (lane == 0 && c > 0) {   // samples -2, -1 of each row; keep -1
+        uint32_t e[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++) e[i] = __ldg(reinterpret_cast<const uint32_t *>(base + (size_t)min(s0 - 1 + i, H - 1) * W - 2));
+        left01 = __byte_perm(e[0], e[1], 0x7632);
+        left23 = __byte_perm(e[2], e[3], 0x7632);
+    }
+    if (lane == 31 && c < cols - 1) {   // samples 8, 9 of each row; keep 8
+        uint32_t e[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++) e[i] = __ldg(reinterpret_cast<const uint32_t *>(base + (size_t)min(s0 - 1 + i, H - 1) * W + 8));
+        right01 = __byte_perm(e[0], e[1], 0x5410);
+        right23 = __byte_perm(e[2], e[3], 0x5410);
+    }
+    const Row16 q[4] = {{w[0], left01 & 0xffffu, right01 & 0xffffu}, {w[1], left01 >> 16, right01 >> 16},
+                        {w[2], left23 & 0xffffu, right23 & 0xffffu}, {w[3], left23 >> 16, right23 >> 16}};
+    const int half_m1 = (1 << (shift - 1)) - 1;
+    uint8_t *o = out + (frame + (size_t)y0 * W + 8 * c) * BPP;
+    const size_t next_row = (size_t)W * BPP;
+    uint32_t px[8];
+    if (s0 & 1) row16_x8<OUT, FMT, 1>(px, q[0], q[1], q[2], shift, half_m1);
+    else row16_x8<OUT, FMT, 0>(px, q[0], q[1], q[2], shift, half_m1);
+    if (c == 0) px[0] = px[1];
+    if (c == cols - 1) px[7] = px[6];
+    if (live) {
+        store_x8<OUT>(o, px);
+        if (s1 == s0 && y0 + 1 < H) store_x8<OUT>(o + next_row, px);
+    }
+    if (s1 != s0) {
+        row16_x8<OUT, FMT, 1>(px, q[1], q[2], q[3], shift, half_m1);
+        if (c == 0) px[0] = px[1];
+        if (c == cols - 1) px[7] = px[6];
+        if (live) store_x8<OUT>(o + next_row, px);
+    }
+}
+
+// any W, H >= 3, any alignment (odd byte addresses included): one pixel per thread, each sample from two byte loads
+template <int OUT, int FMT>
+__global__ void __launch_bounds__(256)
+bayer16_kernel_x1(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, int W, int H, int f0, int shift)
+{
+    using Pat = Pattern<FMT>;
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    const int y = u / W, x = u - y * W;
+    if (y >= H) return;
+    const size_t frame = ((size_t)f0 + blockIdx.y) * W * H;
+    const int ys = min(max(y, 1), H - 2), xs = min(max(x, 1), W - 2);
+    const uint8_t *p = in + 2 * (frame + (size_t)ys * W + xs);
+    const auto at = [p](ptrdiff_t i) { return (int)__ldg(p + 2 * i) | (int)__ldg(p + 2 * i + 1) << 8; };
+    const int h = at(-1) + at(1), v = at(-W) + at(W);
+    const int d = at(-W - 1) + at(-W + 1) + at(W - 1) + at(W + 1);
+    const Rgb rgb = site((ys & 1) == Pat::ry, (xs & 1) == Pat::rx, at(0), h, v, d);
+    store_px<OUT>(out + (frame + (size_t)y * W + x) * OutFmt<OUT>::bpp, pixel_word<OUT>(reduce16(rgb, shift, (1 << (shift - 1)) - 1)));
+}
+
+// shift: bits per sample - 8; 0 = 8-bit samples
+template <int OUT, int FMT>
+int launch_t(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, int shift)
+{
+    const uintptr_t in_align = shift ? 15u : 7u, out_align = OutFmt<OUT>::bpp == 4 ? 15u : 7u;
+    const bool x8 = (W & 7) == 0 && (reinterpret_cast<uintptr_t>(in) & in_align) == 0 && (reinterpret_cast<uintptr_t>(out) & out_align) == 0;
     const long long units = x8 ? (long long)((H + 1) / 2) * (W / 8) : (long long)H * W;   // threads per frame
     const dim3 block(256);
     for (int f0 = 0; f0 < n_frames; f0 += 65535) {
         const dim3 grid((unsigned)((units + 255) / 256), (unsigned)min(n_frames - f0, 65535));
-        if (x8) bayer_kernel_x8<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0);
-        else bayer_kernel_x1<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0);
+        if (shift == 0) {
+            if (x8) bayer_kernel_x8<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0);
+            else bayer_kernel_x1<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0);
+        } else {
+            if (x8) bayer16_kernel_x8<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0, shift);
+            else bayer16_kernel_x1<OUT, FMT><<<grid, block, 0, s>>>(in, out, W, H, f0, shift);
+        }
         RIP_LAUNCH_CHECK();
     }
     return RIP_OK;
 }
 
 template <int FMT>
-int launch_fmt(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, YuvOut to)
+int launch_fmt(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, YuvOut to, int shift)
 {
     switch (to) {
-    case YUV_TO_RGB: return launch_t<YUV_TO_RGB, FMT>(s, in, out, W, H, n_frames);
-    case YUV_TO_BGR: return launch_t<YUV_TO_BGR, FMT>(s, in, out, W, H, n_frames);
-    case YUV_TO_RGBA: return launch_t<YUV_TO_RGBA, FMT>(s, in, out, W, H, n_frames);
-    case YUV_TO_BGRA: return launch_t<YUV_TO_BGRA, FMT>(s, in, out, W, H, n_frames);
-    case YUV_TO_GRAY: return launch_t<YUV_TO_GRAY, FMT>(s, in, out, W, H, n_frames);
-    case YUV_TO_GRAY_RGBA: return launch_t<YUV_TO_GRAY_RGBA, FMT>(s, in, out, W, H, n_frames);
+    case YUV_TO_RGB: return launch_t<YUV_TO_RGB, FMT>(s, in, out, W, H, n_frames, shift);
+    case YUV_TO_BGR: return launch_t<YUV_TO_BGR, FMT>(s, in, out, W, H, n_frames, shift);
+    case YUV_TO_RGBA: return launch_t<YUV_TO_RGBA, FMT>(s, in, out, W, H, n_frames, shift);
+    case YUV_TO_BGRA: return launch_t<YUV_TO_BGRA, FMT>(s, in, out, W, H, n_frames, shift);
+    case YUV_TO_GRAY: return launch_t<YUV_TO_GRAY, FMT>(s, in, out, W, H, n_frames, shift);
+    case YUV_TO_GRAY_RGBA: return launch_t<YUV_TO_GRAY_RGBA, FMT>(s, in, out, W, H, n_frames, shift);
     }
     return fail(RIP_EINVAL, "Bayer decode: bad output %d", (int)to);
 }
 
 }  // namespace
 
+// Every Bayer code is routed by name to the kernels of its pattern (the 8-bit code) and its depth (the shift); anything
+// else is an error, never a default pattern.
 int launch_bayer(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, int in_format, YuvOut to)
 {
+    const int shift = bayer_bits(in_format) - 8;
     switch (in_format) {
-    case RIP_FMT_BAYER_RGGB8: return launch_fmt<RIP_FMT_BAYER_RGGB8>(s, in, out, W, H, n_frames, to);
-    case RIP_FMT_BAYER_BGGR8: return launch_fmt<RIP_FMT_BAYER_BGGR8>(s, in, out, W, H, n_frames, to);
-    case RIP_FMT_BAYER_GRBG8: return launch_fmt<RIP_FMT_BAYER_GRBG8>(s, in, out, W, H, n_frames, to);
-    default: return launch_fmt<RIP_FMT_BAYER_GBRG8>(s, in, out, W, H, n_frames, to);
+    case RIP_FMT_BAYER_RGGB8: case RIP_FMT_BAYER_RGGB10: case RIP_FMT_BAYER_RGGB12: case RIP_FMT_BAYER_RGGB14: case RIP_FMT_BAYER_RGGB16:
+        return launch_fmt<RIP_FMT_BAYER_RGGB8>(s, in, out, W, H, n_frames, to, shift);
+    case RIP_FMT_BAYER_BGGR8: case RIP_FMT_BAYER_BGGR10: case RIP_FMT_BAYER_BGGR12: case RIP_FMT_BAYER_BGGR14: case RIP_FMT_BAYER_BGGR16:
+        return launch_fmt<RIP_FMT_BAYER_BGGR8>(s, in, out, W, H, n_frames, to, shift);
+    case RIP_FMT_BAYER_GRBG8: case RIP_FMT_BAYER_GRBG10: case RIP_FMT_BAYER_GRBG12: case RIP_FMT_BAYER_GRBG14: case RIP_FMT_BAYER_GRBG16:
+        return launch_fmt<RIP_FMT_BAYER_GRBG8>(s, in, out, W, H, n_frames, to, shift);
+    case RIP_FMT_BAYER_GBRG8: case RIP_FMT_BAYER_GBRG10: case RIP_FMT_BAYER_GBRG12: case RIP_FMT_BAYER_GBRG14: case RIP_FMT_BAYER_GBRG16:
+        return launch_fmt<RIP_FMT_BAYER_GBRG8>(s, in, out, W, H, n_frames, to, shift);
     }
+    return fail(RIP_EINVAL, "Bayer decode: input format %d is not a Bayer format", in_format);
 }
 
 }  // namespace rip

@@ -228,6 +228,22 @@ const char *yuv_format_name(int fmt)
     case RIP_FMT_BAYER_BGGR8: return "BAYER_BGGR8";
     case RIP_FMT_BAYER_GRBG8: return "BAYER_GRBG8";
     case RIP_FMT_BAYER_GBRG8: return "BAYER_GBRG8";
+    case RIP_FMT_BAYER_RGGB10: return "BAYER_RGGB10";
+    case RIP_FMT_BAYER_BGGR10: return "BAYER_BGGR10";
+    case RIP_FMT_BAYER_GRBG10: return "BAYER_GRBG10";
+    case RIP_FMT_BAYER_GBRG10: return "BAYER_GBRG10";
+    case RIP_FMT_BAYER_RGGB12: return "BAYER_RGGB12";
+    case RIP_FMT_BAYER_BGGR12: return "BAYER_BGGR12";
+    case RIP_FMT_BAYER_GRBG12: return "BAYER_GRBG12";
+    case RIP_FMT_BAYER_GBRG12: return "BAYER_GBRG12";
+    case RIP_FMT_BAYER_RGGB14: return "BAYER_RGGB14";
+    case RIP_FMT_BAYER_BGGR14: return "BAYER_BGGR14";
+    case RIP_FMT_BAYER_GRBG14: return "BAYER_GRBG14";
+    case RIP_FMT_BAYER_GBRG14: return "BAYER_GBRG14";
+    case RIP_FMT_BAYER_RGGB16: return "BAYER_RGGB16";
+    case RIP_FMT_BAYER_BGGR16: return "BAYER_BGGR16";
+    case RIP_FMT_BAYER_GRBG16: return "BAYER_GRBG16";
+    case RIP_FMT_BAYER_GBRG16: return "BAYER_GBRG16";
     default: return "(not a YUV format)";
     }
 }

@@ -3,6 +3,11 @@
 host pipeline from Bayer against RGB8 and NV12_COLOR input.
 
     python tools/bench_bayer.py [--launches 21] > profiles/bayer_b200.txt
+    python tools/bench_bayer.py --raw16 [--launches 21] > profiles/bayer16_b200.txt
+
+--raw16 times the 10- to 16-bit formats instead (2 bytes per pixel in): the kernel legs on 32 x 3840x2160 BAYER_RGGB12 and
+BAYER_RGGB16, the demosaic's share of GAUSSIAN 5x5 on 16 x 1920x1080 BAYER_RGGB12, and the end-to-end legs from BAYER_RGGB12
+against RGB8 of the same decoded image and against BAYER_RGGB8; outputs are checked against tests/bayer16_ref.py.
 
 Kernel legs: CUDA events around each launch, 3 warm-up launches, the median of --launches (>= 20) launches; 32 x 3840x2160
 Bayer frames are 265 MB in and up to 1.06 GB out, far above the 126 MB L2.  Algorithmic bytes per pixel: 1 in + the output's
@@ -23,6 +28,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     sys.path.insert(0, p)
+import bayer16_ref as R16  # noqa: E402
 import bayer_ref as R  # noqa: E402
 import nv12_ref  # noqa: E402
 import oracle as O  # noqa: E402
@@ -33,6 +39,7 @@ PEAK_GBS = 6550.0
 ap = argparse.ArgumentParser()
 ap.add_argument("--launches", type=int, default=21)
 ap.add_argument("--e2e-steps", type=int, default=10)
+ap.add_argument("--raw16", action="store_true", help="time the 10- to 16-bit formats instead of the 8-bit ones")
 a = ap.parse_args()
 assert a.launches >= 20
 if rip.device_count() < 1:
@@ -83,8 +90,122 @@ def check(name, got, want):
         raise SystemExit(f"{name}: timed output differs from the reference ({int((got != want).sum())} bytes)")
 
 
+def camera_like16(n, h, w, bits, seed):
+    """camera_like at `bits` bits per sample: the same kind of scene, with the sensor noise of the deeper samples."""
+    rng = np.random.default_rng(seed)
+    yy, xx = np.mgrid[0:h, 0:w].astype(np.float32)
+    top = (1 << bits) - 1
+    one = np.clip(top * (0.47 + 0.35 * np.sin(0.01 * xx + 0.007 * yy)) + rng.integers(-3 << (bits - 8), 4 << (bits - 8), (h, w)),
+                  0, top).astype(np.uint16)
+    return np.stack([np.roll(one, 37 * i, axis=1) for i in range(n)])
+
+
+def raw16_legs():
+    # ---- decode kernels, 32 x 4K RGGB at 12 and at 16 bits: 2 B/px in --------------------------------------------------------
+    N, H, W = 32, 2160, 3840
+    px = N * H * W
+    d_out = rip.DeviceBuffer(px * 4)
+    d_rgb = rip.DeviceBuffer(px * 3)
+    sample = (0, N // 2, N - 1)
+    for bits in (12, 16):
+        fmt, name = getattr(rip, f"FMT_BAYER_RGGB{bits}"), f"BAYER_RGGB{bits}"
+        raw = camera_like16(N, H, W, bits, bits)
+        d_in = rip.DeviceBuffer(raw.nbytes).upload(raw)
+        want_rgb = {i: R16.decode(raw[i], "rggb", bits) for i in sample}
+        for order, ofmt in (("rgba", rip.FMT_RGBA8), ("rgb", rip.FMT_RGB8)):
+            us, best = timed(lambda: rip.convert_dev(d_in.ptr, d_out.ptr, W, H, N, fmt, ofmt))
+            row(f"rip_convert {name} -> {order.upper()}8, {N} x {W}x{H}", us, best, px, 2 + len(order))
+            fb = H * W * len(order)
+            for i in sample:
+                want = want_rgb[i] if order == "rgb" else np.concatenate([want_rgb[i], np.full((H, W, 1), 255, np.uint8)], -1)
+                check(f"convert {name} {order} frame {i}", d_out.download((H, W, len(order)), offset=i * fb), want)
+        want_gray = {i: O.gray(want_rgb[i], threads=0) for i in sample}
+        us_gray, best = timed(lambda: rip.gray_dev(d_in.ptr, d_out.ptr, W, H, N, fmt, rip.GRAY_OUT_U8))
+        row(f"rip_gray {name} -> u8, {N} x {W}x{H}", us_gray, best, px, 3)
+        for i in sample:
+            check(f"gray {name} frame {i}", d_out.download((H, W), offset=i * H * W), want_gray[i])
+
+        def two_kernels():
+            rip.convert_dev(d_in.ptr, d_rgb.ptr, W, H, N, fmt, rip.FMT_RGB8)
+            rip.gray_dev(d_rgb.ptr, d_out.ptr, W, H, N, rip.FMT_RGB8, rip.GRAY_OUT_U8)
+
+        us_two, best = timed(two_kernels)
+        row(f"rip_convert -> RGB8, then rip_gray RGB8 -> u8, {name}", us_two, best, px, 3, floor_note=False)
+        print(f"  rip_gray on {name} is {us_two / us_gray:.2f}x faster than the two-kernel route", flush=True)
+        for i in sample:
+            check(f"two-kernel gray {name} frame {i}", d_out.download((H, W), offset=i * H * W), want_gray[i])
+        d_in.free()
+        del raw
+    d_out.free()
+    d_rgb.free()
+
+    # ---- GAUSSIAN 5x5 on 16 x 1080p: demosaic + blur against the blur alone on RGBA8 ------------------------------------------
+    N, H, W = 16, 1080, 1920
+    px = N * H * W
+    fmt = rip.FMT_BAYER_RGGB12
+    raw = camera_like16(N, H, W, 12, 2)
+    wt = rip.gauss_weights(5, 1.0)
+    d_raw = rip.DeviceBuffer(raw.nbytes).upload(raw)
+    d_rgba = rip.DeviceBuffer(px * 4)
+    d_blur = rip.DeviceBuffer(px * 4)
+    rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, fmt, rip.FMT_RGBA8)
+    us_blur, best = timed(lambda: rip.gauss_dev(d_rgba.ptr, d_blur.ptr, W, H, N, 4, 5, wt))
+    row(f"GAUSSIAN 5x5 blur alone, RGBA8, {N} x {W}x{H}", us_blur, best, px, 8)
+    us_dec, best = timed(lambda: rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, fmt, rip.FMT_RGBA8))
+    row(f"demosaic BAYER_RGGB12 -> RGBA8, {N} x {W}x{H}", us_dec, best, px, 6)
+
+    def both():
+        rip.convert_dev(d_raw.ptr, d_rgba.ptr, W, H, N, fmt, rip.FMT_RGBA8)
+        rip.gauss_dev(d_rgba.ptr, d_blur.ptr, W, H, N, 4, 5, wt)
+
+    us_both, best = timed(both)
+    row(f"demosaic + GAUSSIAN 5x5, BAYER_RGGB12, {N} x {W}x{H}", us_both, best, px, 6, floor_note=False)
+    print(f"  demosaic adds {us_both - us_blur:.1f} us = {100 * (us_both - us_blur) / us_blur:.1f} % of the blur alone", flush=True)
+    for i in (0, N - 1):
+        check(f"blur frame {i}", d_blur.download((H, W, 4), offset=i * H * W * 4),
+              O.blur(R16.decode(raw[i], "rggb", 12, "rgba"), 5, weights=wt, threads=0))
+    d_raw.free()
+    d_rgba.free()
+    d_blur.free()
+
+    # ---- end to end from pinned memory: BAYER_RGGB12 against RGB8 (the same decoded image) and BAYER_RGGB8 -------------------
+    ctx = rip.Context([0])
+    rgb = R16.decode(raw, "rggb", 12)
+    raw8 = camera_like(N, H, W, 2)
+    print(f"# end to end, rip_process_host, pinned host buffers, {N} x {W}x{H}, wall clock over {a.e2e_steps} calls", flush=True)
+    names = {fmt: "BAYER_RGGB12", rip.FMT_RGB8: "RGB8", rip.FMT_BAYER_RGGB8: "BAYER_RGGB8"}
+    for op, name, kw in ((rip.OP_GRAY, "GRAY", {}), (rip.OP_EDGE, "EDGE", {}), (rip.OP_FUSED, "FUSED 5x5", {"ksize": 5, "weights": wt})):
+        res = {}
+        for f, src in ((fmt, raw), (rip.FMT_RGB8, rgb), (rip.FMT_BAYER_RGGB8, raw8)):
+            h_in = rip.PinnedBuffer(src.nbytes)
+            a_in = h_in.array.view(src.dtype).reshape(src.shape)
+            a_in[...] = src
+            h_out = rip.PinnedBuffer(px)
+            a_out = h_out.array.reshape((N, H, W))
+            for _ in range(2):
+                ctx.process(a_in, op, f, out=a_out, **kw)
+            t0 = time.perf_counter()
+            for _ in range(a.e2e_steps):
+                ctx.process(a_in, op, f, out=a_out, **kw)
+            dt = (time.perf_counter() - t0) / a.e2e_steps
+            res[f] = (dt, a_out.copy())
+            print(f"  {name:10s} {names[f]:12s} {dt * 1e3:8.2f} ms/call  {px / dt / 1e9:6.2f} Gpx/s  "
+                  f"({src.nbytes / px:.1f} B/px in, 1 B/px out)", flush=True)
+            del a_in, a_out
+            h_in.free()
+            h_out.free()
+        check(f"e2e {name}: BAYER_RGGB12 vs RGB8 of the decoded frames", res[fmt][1], res[rip.FMT_RGB8][1])
+        for ref in (rip.FMT_RGB8, rip.FMT_BAYER_RGGB8):
+            print(f"  {name}: BAYER_RGGB12 / {names[ref]} speed {res[ref][0] / res[fmt][0]:.2f}x", flush=True)
+    ctx.close()
+    print("# every sampled output equal to the reference")
+
+
 print(f"# {card()}")
 print(f"# median of {a.launches} launches after 3 warm-up launches (CUDA events); copy peak {PEAK_GBS:.0f} GB/s", flush=True)
+if a.raw16:
+    raw16_legs()
+    sys.exit(0)
 
 # ---- decode kernels, 32 x 4K RGGB ---------------------------------------------------------------------------------------------
 N, H, W = 32, 2160, 3840
