@@ -400,8 +400,10 @@ class Context:
     def _desc(self, op, fmt, gray_out=GRAY_OUT_U8, ksize=0, weights=None):
         d = OpDesc()
         d.op, d.in_format, d.gray_out, d.ksize = op, fmt, gray_out, ksize
-        self._w = None if weights is None else np.ascontiguousarray(weights, np.float32)
-        d.weights = _f32p(self._w)
+        # the descriptor keeps its weights alive: two threads calling process() on one Context must not free each other's
+        # weights while the C call reads them
+        d.keep_weights = None if weights is None else np.ascontiguousarray(weights, np.float32)
+        d.weights = _f32p(d.keep_weights)
         return d
 
     def _shapes(self, frames: np.ndarray, op, fmt, gray_out, ksize, weights, out):
