@@ -15,6 +15,9 @@
  *     asynchronous on their stream; pointers named d_* are device pointers on the stream's device.
  *   - images are interleaved u8, row-major, tightly packed (pitch = width * channels); batches are
  *     n_frames consecutive frames.
+ *   - device buffers may start at any byte: rip_gray, rip_convert, rip_sobel and rip_fused take any alignment of d_in
+ *     and d_out (aligned buffers run the wider kernels, with the same results).  The one exception is RGBA rip_gauss
+ *     (channels = 4), whose d_in and d_out must be 4-byte aligned; otherwise it returns RIP_EINVAL and writes nothing.
  *   - results are defined by the reference's CPU paths (bit-exact): gray = Comparator.cpp:30-45,
  *     blur = GaussianBlur.cpp:231-261, Sobel = EdgeDetection.cpp:219-240, fused = their
  *     composition with a u8 image between stages.
@@ -177,15 +180,17 @@ int rip_convert(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_o
                 int n_frames, int in_format, int out_format);
 
 /* K x K float32 convolution per channel in the reference's summation order, clamp-to-edge,
- * truncation.  channels: 1 (gray) or 4 (RGBA, all four channels blurred).  weights: host pointer
- * to ksize*ksize floats (copied before the call returns).  ksize odd, 1..RIP_MAX_KSIZE. */
+ * truncation.  channels: 1 (gray, any alignment) or 4 (RGBA, all four channels blurred; d_in and d_out
+ * 4-byte aligned, else RIP_EINVAL).  weights: host pointer to ksize*ksize floats (copied before the call
+ * returns).  ksize odd, 1..RIP_MAX_KSIZE. */
 #define RIP_MAX_KSIZE 31
 int rip_gauss(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int channels, int ksize, const float *weights);
 
 /* 3x3 Sobel magnitude, BORDER_REFLECT_101, round-half-even, saturate (OpenCV semantics).
  * in_format GRAY8 runs on the image as is; RGB8/RGBA8/BGR8/BGRA8 first convert with rip_gray's
- * arithmetic inside the same kernel.  d_out: w*h bytes per frame.  NV12_COLOR, YUYV, UYVY, I420, BAYER_*: RIP_EUNSUPPORTED (rip_gray
+ * arithmetic inside the same kernel; NV12 (even height, any width) runs on the luma plane of each frame.  d_out: w*h bytes
+ * per frame.  NV12_COLOR, YUYV, UYVY, I420, BAYER_*: RIP_EUNSUPPORTED (rip_gray
  * with RIP_GRAY_OUT_U8 first, then GRAY8); the same holds for rip_fused. */
 int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
               int height, int n_frames, int in_format);
@@ -194,7 +199,9 @@ int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out
  * shape and kernel size.  Processes output rows [out_row0, out_row0 + out_rows) of
  * frames whose true height is `height`; d_in holds input rows [in_row0, in_row0 + in_rows) of each
  * frame (a row band with halo: it must cover out rows extended by ksize/2 + 1 rows each side, clipped to
- * the image).  For whole frames pass in_row0 = out_row0 = 0 and in_rows = out_rows = height.
+ * the image, and may hold more rows than that, up to the whole frame; a band that misses a needed row, or
+ * reaches past row height - 1, fails with RIP_EINVAL).  For whole frames pass in_row0 = out_row0 = 0 and
+ * in_rows = out_rows = height.
  * d_out holds out_rows * width bytes per frame.  d_workspace and workspace_bytes are unused (pass
  * NULL, 0); they stay in the signature for ABI compatibility. */
 int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,

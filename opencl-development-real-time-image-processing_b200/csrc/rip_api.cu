@@ -719,15 +719,13 @@ extern "C" int rip_sobel(int device, rip_stream stream, const uint8_t *d_in, uin
     if (int rc = check_image("rip_sobel", d_in, d_out, width, height, n_frames)) return rc;
     if (decodes_to_color(in_format)) return needs_gray_first("rip_sobel", in_format);
     if (channels_of(in_format) == 0) return fail(RIP_EINVAL, "rip_sobel: unsupported input format %d", in_format);
+    if (in_format == RIP_FMT_NV12 && (height & 1)) return fail(RIP_EINVAL, "rip_sobel: NV12 frames need an even height (got %d)", height);
     DeviceGuard g(device);
     if (!g.ok) return fail(RIP_ENODEV, "cudaSetDevice(%d) failed", device);
     if (fused_supported(width, height, in_format, 0, d_in, d_out))
         return launch_fused((cudaStream_t)stream, d_in, d_out, width, height, n_frames, in_format, false, nullptr, 0, height, 0,
                             height, device);
-    if (in_format == RIP_FMT_NV12 && n_frames > 1)
-        return fail(RIP_EUNSUPPORTED, "rip_sobel: NV12 batches need width %% 4 == 0, an even height and 4-byte aligned buffers");
-    return launch_sobel((cudaStream_t)stream, d_in, d_out, width, height, n_frames, in_format == RIP_FMT_NV12 ? RIP_FMT_GRAY8 : in_format, 0,
-                        height, 0, height);
+    return launch_sobel((cudaStream_t)stream, d_in, d_out, width, height, n_frames, in_format, 0, height, 0, height);
 }
 
 extern "C" int rip_fused_workspace_bytes(int width, int in_rows, int n_frames, int ksize, size_t *bytes)
@@ -747,6 +745,7 @@ extern "C" int rip_fused(int device, rip_stream stream, const uint8_t *d_in, uin
     if (int rc = check_image("rip_fused", d_in, d_out, width, height, n_frames)) return rc;
     if (decodes_to_color(in_format)) return needs_gray_first("rip_fused", in_format);
     if (channels_of(in_format) == 0) return fail(RIP_EINVAL, "rip_fused: unsupported input format %d", in_format);
+    if (in_format == RIP_FMT_NV12 && (height & 1)) return fail(RIP_EINVAL, "rip_fused: NV12 frames need an even height (got %d)", height);
     Weights wts;
     if (int rc = load_weights(wts, ksize, weights, "rip_fused")) return rc;
     const int half = ksize / 2;
@@ -880,7 +879,7 @@ int rip_sobel_rows(int device, cudaStream_t s, const uint8_t *d_in, uint8_t *d_o
     if (!g.ok) return fail(RIP_ENODEV, "cudaSetDevice(%d) failed", device);
     if (fused_supported(W, H, fmt, 0, d_in, d_out))
         return launch_fused(s, d_in, d_out, W, H, 1, fmt, false, nullptr, in_row0, in_rows, out_row0, out_rows, device);
-    return launch_sobel(s, d_in, d_out, W, H, 1, fmt == RIP_FMT_NV12 ? RIP_FMT_GRAY8 : fmt, in_row0, in_rows, out_row0, out_rows);
+    return launch_sobel(s, d_in, d_out, W, H, 1, fmt, in_row0, in_rows, out_row0, out_rows);
 }
 
 // ---- the worker side ----------------------------------------------------------------------------------------

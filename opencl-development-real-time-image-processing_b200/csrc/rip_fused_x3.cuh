@@ -721,6 +721,7 @@ __device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, const X2Params &
             s = s == (uint32_t)NB - 1u ? 0u : s + 1u;
         }
     }
+    const int r_main0 = r;
 #pragma unroll 1
     for (; r + NB - 1 <= r_main_last; r += NB) {
         if constexpr (BLUR) {
@@ -735,7 +736,11 @@ __device__ __forceinline__ void run_rows_x2(WarpX<NPX, CN> &st, const X2Params &
             for (int k = 0; k < NB; k++) step_x2<NPX, CN, BGR, BLUR, false, STATS, 0, NB>(st, ra[k], xp, geo, r + k);
         }
     }
-    if constexpr (BLUR) geo.slot = (geo.ringB - geo.ring_lane) / kRowB + 2u;   // newest row: last slot of the half written last
+    // newest row: last slot of the half written last.  Only if a trip ran: a segment of one output row leaves the head at r_last
+    // with the newest row in slot 1 (neither 2 nor 5), and no trip follows -- the tail must keep the head's slot.
+    if constexpr (BLUR) {
+        if (r != r_main0) geo.slot = (geo.ringB - geo.ring_lane) / kRowB + 2u;
+    }
 #pragma unroll 1
     for (; r <= geo.r_last; r++) {
         step_x2<NPX, CN, BGR, BLUR, true, STATS, -1, NB>(st, geo.raw_lane + geo.rs * kRawB, xp, geo, r);

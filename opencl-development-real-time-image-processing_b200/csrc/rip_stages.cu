@@ -223,11 +223,11 @@ constexpr int SOB_TW = 64, SOB_TH = 16, SOB_SW = SOB_TW + 2 + 2 /* pad to a mult
 template <int CN, bool BGR>
 __global__ void __launch_bounds__(256)
 sobel_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, int W, int H, int src_row0, int src_rows,
-             int out_row0, int out_rows)
+             int out_row0, int out_rows, size_t in_frame_bytes)
 {
     __shared__ uint8_t tile[(SOB_TH + 2) * SOB_SW];
     const int x0 = blockIdx.x * SOB_TW, y0 = out_row0 + blockIdx.y * SOB_TH;
-    const uint8_t *fsrc = src + (size_t)blockIdx.z * src_rows * W * CN;
+    const uint8_t *fsrc = src + (size_t)blockIdx.z * in_frame_bytes;
     uint8_t *fdst = dst + (size_t)blockIdx.z * out_rows * W;
     const int y_end = min(out_row0 + out_rows, H);
 
@@ -274,14 +274,19 @@ int launch_sobel(cudaStream_t s, const uint8_t *src, uint8_t *dst, int W, int H,
                  int src_row0, int src_rows, int out_row0, int out_rows)
 {
     const dim3 block(256);
+    const int cn = fmt == RIP_FMT_RGB8 || fmt == RIP_FMT_BGR8 ? 3 : fmt == RIP_FMT_RGBA8 || fmt == RIP_FMT_BGRA8 ? 4 : 1;
+    // whole NV12 frames carry their chroma plane behind the luma plane; row bands are passed as plain luma rows
+    const size_t in_frame_bytes = (fmt == RIP_FMT_NV12 && src_row0 == 0 && src_rows == H) ? (size_t)W * H * 3 / 2 : (size_t)src_rows * W * cn;
     // frames ride in gridDim.z (<= 65535): batches of tiny frames go out in slabs
     for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
         const dim3 grid((W + SOB_TW - 1) / SOB_TW, (out_rows + SOB_TH - 1) / SOB_TH, min(n_frames - f0, kMaxGridZ));
+        const uint8_t *fs = src + (size_t)f0 * in_frame_bytes;
         uint8_t *fd = dst + (size_t)f0 * out_rows * W;
 #define RIP_SOBEL_CASE(F, CN, BGR) \
-    case F: sobel_kernel<CN, BGR><<<grid, block, 0, s>>>(src + (size_t)f0 * src_rows * W * CN, fd, W, H, src_row0, src_rows, out_row0, out_rows); break;
+    case F: sobel_kernel<CN, BGR><<<grid, block, 0, s>>>(fs, fd, W, H, src_row0, src_rows, out_row0, out_rows, in_frame_bytes); break;
         switch (fmt) {
             RIP_SOBEL_CASE(RIP_FMT_GRAY8, 1, false)
+            RIP_SOBEL_CASE(RIP_FMT_NV12, 1, false)
             RIP_SOBEL_CASE(RIP_FMT_RGB8, 3, false)
             RIP_SOBEL_CASE(RIP_FMT_BGR8, 3, true)
             RIP_SOBEL_CASE(RIP_FMT_RGBA8, 4, false)
