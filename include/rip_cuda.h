@@ -57,7 +57,15 @@ enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5,
        RIP_FMT_BAYER_RGGB10 = 16, RIP_FMT_BAYER_BGGR10 = 17, RIP_FMT_BAYER_GRBG10 = 18, RIP_FMT_BAYER_GBRG10 = 19,
        RIP_FMT_BAYER_RGGB12 = 20, RIP_FMT_BAYER_BGGR12 = 21, RIP_FMT_BAYER_GRBG12 = 22, RIP_FMT_BAYER_GBRG12 = 23,
        RIP_FMT_BAYER_RGGB14 = 24, RIP_FMT_BAYER_BGGR14 = 25, RIP_FMT_BAYER_GRBG14 = 26, RIP_FMT_BAYER_GBRG14 = 27,
-       RIP_FMT_BAYER_RGGB16 = 28, RIP_FMT_BAYER_BGGR16 = 29, RIP_FMT_BAYER_GRBG16 = 30, RIP_FMT_BAYER_GBRG16 = 31 };
+       RIP_FMT_BAYER_RGGB16 = 28, RIP_FMT_BAYER_BGGR16 = 29, RIP_FMT_BAYER_GRBG16 = 30, RIP_FMT_BAYER_GBRG16 = 31,
+       RIP_FMT_BAYER_RGGB10P_MIPI = 40, RIP_FMT_BAYER_BGGR10P_MIPI = 41, RIP_FMT_BAYER_GRBG10P_MIPI = 42,
+       RIP_FMT_BAYER_GBRG10P_MIPI = 43,
+       RIP_FMT_BAYER_RGGB12P_MIPI = 44, RIP_FMT_BAYER_BGGR12P_MIPI = 45, RIP_FMT_BAYER_GRBG12P_MIPI = 46,
+       RIP_FMT_BAYER_GBRG12P_MIPI = 47,
+       RIP_FMT_BAYER_RGGB10P_GENICAM = 48, RIP_FMT_BAYER_BGGR10P_GENICAM = 49, RIP_FMT_BAYER_GRBG10P_GENICAM = 50,
+       RIP_FMT_BAYER_GBRG10P_GENICAM = 51,
+       RIP_FMT_BAYER_RGGB12P_GENICAM = 52, RIP_FMT_BAYER_BGGR12P_GENICAM = 53, RIP_FMT_BAYER_GRBG12P_GENICAM = 54,
+       RIP_FMT_BAYER_GBRG12P_GENICAM = 55 };
 /* RIP_FMT_NV12 (the reference's camera format, RT/RealtimeImageProcessing.cpp:153): per frame a W*H luma plane
  * followed by the W*H/2 interleaved chroma plane (frame = W*H*3/2 bytes, H even).  Accepted by the EDGE and FUSED
  * operations only; the luma plane is the gray image (one byte per pixel leaves HBM instead of three or four),
@@ -91,7 +99,30 @@ enum { RIP_FMT_GRAY8 = 1, RIP_FMT_RGB8 = 3, RIP_FMT_RGBA8 = 4, RIP_FMT_BGR8 = 5,
  * (the 8-bit formulas on the full samples, the same pattern names) followed by convertTo(CV_8U, 1.0 / (1 << (b - 8))): each
  * channel divided by 2^(b-8), rounded half to even, saturated (a full-scale sample gives 255; padding bits above bit b-1 are
  * used as they are, and saturate); alpha 255.  Taken everywhere the 8-bit Bayer formats are, with the same results on that
- * 8-bit image.  Packed RAW10 / RAW12 are not taken. */
+ * 8-bit image.
+ * Packed 10- and 12-bit Bayer raw frames (codes 40-55, patterns in the order of 12-15 within each packing): rows of exactly
+ * W*5/4 bytes (10-bit) or W*3/2 bytes (12-bit), no row padding, frames consecutive (H*W*5/4 or H*W*3/2 bytes each), any
+ * alignment; W a multiple of 4 (10-bit) or of 2 (12-bit) and at least 4, H at least 3 (else RIP_EINVAL).
+ *   RIP_FMT_BAYER_<pattern>10P_MIPI (40-43): MIPI CSI-2 RAW10 (V4L2 SRGGB10P ..., libcamera SRGGB10_CSI2P ...), 4 pixels in
+ *     5 bytes:
+ *         byte 0      byte 1      byte 2      byte 3      byte 4
+ *         P0[9:2]     P1[9:2]     P2[9:2]     P3[9:2]     P3[1:0] P2[1:0] P1[1:0] P0[1:0]   (bit 7 ... bit 0)
+ *   RIP_FMT_BAYER_<pattern>12P_MIPI (44-47): MIPI CSI-2 RAW12 (V4L2 SRGGB12P ..., libcamera SRGGB12_CSI2P ...), 2 pixels in
+ *     3 bytes:
+ *         byte 0      byte 1      byte 2
+ *         P0[11:4]    P1[11:4]    P1[3:0] P0[3:0]                                         (bit 7 ... bit 0)
+ *   RIP_FMT_BAYER_<pattern>10P_GENICAM (48-51), RIP_FMT_BAYER_<pattern>12P_GENICAM (52-55): GenICam PFNC BayerRG10p /
+ *     BayerRG12p ... (and BayerBG, BayerGR, BayerGB), an LSB-first bit stream: pixel i occupies stream bits b*i .. b*i+b-1,
+ *     stream bit k is bit k % 8 of byte k / 8.  At 10 bits:
+ *         byte 0      byte 1              byte 2              byte 3              byte 4
+ *         P0[7:0]     P1[5:0] P0[9:8]     P2[3:0] P1[9:6]     P3[1:0] P2[9:4]     P3[9:2]   (bit 7 ... bit 0)
+ *     at 12 bits:
+ *         byte 0      byte 1              byte 2
+ *         P0[7:0]     P1[3:0] P0[11:8]    P1[11:4]                                        (bit 7 ... bit 0)
+ *     A width off these multiples would start rows inside a byte.
+ * The decode unpacks the b-bit samples and applies exactly the decode of RIP_FMT_BAYER_<pattern>10 / 12 (cvtColor on the
+ * 16-bit frame, then convertTo(CV_8U, 1.0 / (1 << (b - 8)))); packed samples have no padding bits, so full scale (1023 /
+ * 4095) gives 255.  Taken everywhere the other Bayer formats are, with the same results on that 8-bit image. */
 
 /* operations (the reference's METHOD strings "GRAYSCALE" / "GAUSSIAN" / "EDGE", plus "FUSED") */
 enum { RIP_OP_GRAY = 0, RIP_OP_EDGE = 1, RIP_OP_GAUSSIAN = 2, RIP_OP_FUSED = 3 };
@@ -165,16 +196,18 @@ int rip_gauss_weights(int ksize, float sigma, float *weights /* ksize*ksize, hos
  *      All asynchronous on `stream` of `device`. ---- */
 
 /* d_out[i] = (uchar)(0.299*r + 0.587*g + 0.114*b) (double, truncation).  in_format: RGB8 / RGBA8 /
- * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 / BAYER_* of any depth (decoded in the same kernel; 16-bit samples:
- * 2*w*h bytes in per frame, any alignment).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
+ * BGR8 / BGRA8, or NV12_COLOR / YUYV / UYVY / I420 / BAYER_* of any depth or packing (decoded in the same kernel; 16-bit
+ * samples: 2*w*h bytes in per frame, packed: w*h*5/4 or w*h*3/2; any alignment).  out_mode: RIP_GRAY_OUT_U8 (w*h bytes per frame) or
  * RIP_GRAY_OUT_RGBA (w*h*4). */
 int rip_gray(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width,
              int height, int n_frames, int in_format, int out_mode);
 
 /* Colour conversion of whole frames: in_format RIP_FMT_NV12_COLOR or RIP_FMT_I420 (width and height even), RIP_FMT_YUYV or
- * RIP_FMT_UYVY (width even), RIP_FMT_BAYER_* of 8 to 16 bits (width and height at least 3), out_format RGB8 / BGR8 / RGBA8
+ * RIP_FMT_UYVY (width even), RIP_FMT_BAYER_* of 8 to 16 bits (width and height at least 3) or packed at 10 and 12 bits
+ * (width a multiple of 4 or 2 and at least 4, height at least 3), out_format RGB8 / BGR8 / RGBA8
  * (alpha 255) / BGRA8: OpenCV's cvtColor(COLOR_YUV2RGB_NV12 / _BGR / _RGBA / _BGRA, and the same for _I420, _YUYV, _UYVY;
- * the Bayer conversions listed with the formats, followed for 10 to 16 bits by convertTo(CV_8U, 1.0 / (1 << (b - 8)))),
+ * the Bayer conversions listed with the formats, followed for 10 to 16 bits and packed samples by
+ * convertTo(CV_8U, 1.0 / (1 << (b - 8)))),
  * bit for bit.  d_in and d_out may have any alignment.  d_out: w*h*3 or w*h*4 bytes per frame. */
 int rip_convert(int device, rip_stream stream, const uint8_t *d_in, uint8_t *d_out, int width, int height,
                 int n_frames, int in_format, int out_format);

@@ -32,16 +32,32 @@ FMT_BAYER_RGGB14, FMT_BAYER_BGGR14, FMT_BAYER_GRBG14, FMT_BAYER_GBRG14 = 24, 25,
 FMT_BAYER_RGGB16, FMT_BAYER_BGGR16, FMT_BAYER_GRBG16, FMT_BAYER_GBRG16 = 28, 29, 30, 31
 # the formats whose host arrays are uint16 (every other format takes uint8)
 FMTS_U16 = frozenset(range(FMT_BAYER_RGGB10, FMT_BAYER_GBRG16 + 1))
+# packed 10- and 12-bit Bayer raw frames, rows of W*5/4 or W*3/2 bytes with no padding: MIPI CSI-2 RAW10 / RAW12 (V4L2
+# SRGGB10P / SRGGB12P ..., libcamera *10_CSI2P / *12_CSI2P) and GenICam's LSB-first bit streams (BayerRG10p / BayerRG12p ...)
+FMT_BAYER_RGGB10P_MIPI, FMT_BAYER_BGGR10P_MIPI, FMT_BAYER_GRBG10P_MIPI, FMT_BAYER_GBRG10P_MIPI = 40, 41, 42, 43
+FMT_BAYER_RGGB12P_MIPI, FMT_BAYER_BGGR12P_MIPI, FMT_BAYER_GRBG12P_MIPI, FMT_BAYER_GBRG12P_MIPI = 44, 45, 46, 47
+FMT_BAYER_RGGB10P_GENICAM, FMT_BAYER_BGGR10P_GENICAM, FMT_BAYER_GRBG10P_GENICAM, FMT_BAYER_GBRG10P_GENICAM = 48, 49, 50, 51
+FMT_BAYER_RGGB12P_GENICAM, FMT_BAYER_BGGR12P_GENICAM, FMT_BAYER_GRBG12P_GENICAM, FMT_BAYER_GBRG12P_GENICAM = 52, 53, 54, 55
+# the packed formats: their host arrays are uint8 (N, H, row_bytes), and W is derived from row_bytes
+FMTS_PACKED = frozenset(range(FMT_BAYER_RGGB10P_MIPI, FMT_BAYER_GBRG12P_GENICAM + 1))
+
+
+def packed_bits(fmt: int) -> int:
+    """Bits per sample of a packed Bayer format: 10 or 12."""
+    assert fmt in FMTS_PACKED, f"format {fmt} is not a packed Bayer format"
+    return 10 if (fmt - FMT_BAYER_RGGB10P_MIPI) % 8 < 4 else 12
+
+
 OP_GRAY, OP_EDGE, OP_GAUSSIAN, OP_FUSED = 0, 1, 2, 3
 GRAY_OUT_U8, GRAY_OUT_RGBA = 0, 1
 MAX_KSIZE = 31
 # elements per pixel of the host array's last axis; 1 for the planar formats, whose frames are (H*3/2, W) arrays, and for Bayer
-# frames, (H, W) arrays (uint16 for 10 to 16 bits).  YUYV and UYVY are (H, W, 2): the CV_8UC2 Mat that V4L2 capture returns
-# with CAP_PROP_CONVERT_RGB off.
+# frames, (H, W) arrays (uint16 for 10 to 16 bits; packed: (H, row_bytes) uint8).  YUYV and UYVY are (H, W, 2): the CV_8UC2
+# Mat that V4L2 capture returns with CAP_PROP_CONVERT_RGB off.
 CHANNELS = {FMT_GRAY8: 1, FMT_RGB8: 3, FMT_BGR8: 3, FMT_RGBA8: 4, FMT_BGRA8: 4, FMT_NV12: 1, FMT_NV12_COLOR: 1,
             FMT_YUYV: 2, FMT_UYVY: 2, FMT_I420: 1,
             FMT_BAYER_RGGB8: 1, FMT_BAYER_BGGR8: 1, FMT_BAYER_GRBG8: 1, FMT_BAYER_GBRG8: 1,
-            **{f: 1 for f in FMTS_U16}}
+            **{f: 1 for f in FMTS_U16}, **{f: 1 for f in FMTS_PACKED}}
 
 # every symbol include/rip_cuda.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -337,13 +353,14 @@ class Event:
 # ---- device-resident ops on raw device pointers (ints) ----
 def gray_dev(d_in: int, d_out: int, w: int, h: int, n: int, fmt: int, out_mode: int = GRAY_OUT_U8, device=0, stream=None):
     """rip_gray: the reference's gray of RGB8 / BGR8 / RGBA8 / BGRA8 frames, or of NV12_COLOR, YUYV, UYVY, I420 or Bayer
-    frames (8 to 16 bits) decoded in the same kernel."""
+    frames (8 to 16 bits, or packed at 10 and 12) decoded in the same kernel."""
     check(lib().rip_gray(device, stream, d_in, d_out, w, h, n, fmt, out_mode), "rip_gray")
 
 
 def convert_dev(d_in: int, d_out: int, w: int, h: int, n: int, in_fmt: int, out_fmt: int, device=0, stream=None):
     """rip_convert: NV12_COLOR, YUYV, UYVY, I420 or Bayer frames -> RGB8 / BGR8 / RGBA8 / BGRA8 (OpenCV's cvtColor
-    arithmetic; Bayer: its default bilinear demosaic, then for 10 to 16 bits convertTo(CV_8U, 1 / 2^(bits - 8)))."""
+    arithmetic; Bayer: its default bilinear demosaic, then for 10 to 16 bits convertTo(CV_8U, 1 / 2^(bits - 8)); packed
+    samples are unpacked first)."""
     check(lib().rip_convert(device, stream, d_in, d_out, w, h, n, in_fmt, out_fmt), "rip_convert")
 
 
@@ -422,6 +439,12 @@ class Context:
             if fmt in (FMT_NV12, FMT_NV12_COLOR, FMT_I420):
                 assert h % 3 == 0
                 h = h * 2 // 3
+            elif fmt in FMTS_PACKED:   # the last axis is the row's bytes: 4 pixels in 5 (10-bit) or 2 in 3 (12-bit)
+                bits = packed_bits(fmt)
+                group = 5 if bits == 10 else 3
+                assert w % group == 0, \
+                    f"format {fmt} ({bits}-bit packed Bayer) takes rows of a multiple of {group} bytes, got {w}"
+                w = w * 8 // bits
         else:
             if a.ndim == 3:
                 a = a[None]
@@ -443,7 +466,8 @@ class Context:
         """frames: (N, H, W, C) or (H, W, C) / (H, W) u8 host array (pageable or pinned); NV12 / NV12_COLOR / I420:
         (N, H*3/2, W) or (H*3/2, W), the luma plane followed by the chroma planes; YUYV / UYVY: (N, H, W, 2) or (H, W, 2);
         Bayer: (N, H, W) or (H, W), one raw byte per pixel (uint8) for the 8-bit formats, one little-endian uint16 per pixel
-        for 10 to 16 bits.  Every other format takes uint8."""
+        for 10 to 16 bits; packed Bayer: (N, H, row_bytes) or (H, row_bytes) uint8, the row's packed bytes (W*5/4 at 10 bits,
+        W*3/2 at 12), W derived from row_bytes.  Every other format takes uint8."""
         a, d, n, h, w, shape, out, squeeze = self._shapes(frames, op, fmt, gray_out, ksize, weights, out)
         pr = (C.c_uint64 * 6)() if prof else None
         if banded:

@@ -114,6 +114,7 @@ static size_t frame_bytes_of(int fmt, int width, int height)
     case RIP_FMT_NV12: case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return px * 3 / 2;
     case RIP_FMT_YUYV: case RIP_FMT_UYVY: return px * 2;
     default:
+        if (is_packed_bayer(fmt)) return px * bayer_bits(fmt) / 8;   // (W is a multiple of 4 at 10 bits, of 2 at 12)
         if (is_bayer(fmt)) return bayer_bits(fmt) == 8 ? px : px * 2;   // (10 to 16 bits: one 16-bit word per sample)
         return px * channels_of(fmt);
     }
@@ -679,7 +680,7 @@ extern "C" int rip_convert(int device, rip_stream stream, const uint8_t *d_in, u
     if (int rc = check_device(device)) return rc;
     if (int rc = check_image("rip_convert", d_in, d_out, width, height, n_frames)) return rc;
     if (!decodes_to_color(in_format))
-        return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (RIP_FMT_NV12_COLOR, YUYV, UYVY, I420 or BAYER_*8 ... BAYER_*16)", in_format);
+        return fail(RIP_EUNSUPPORTED, "rip_convert: input format %d (RIP_FMT_NV12_COLOR, YUYV, UYVY, I420, BAYER_*8 ... BAYER_*16 or BAYER_*P_*)", in_format);
     YuvOut to;
     switch (out_format) {
     case RIP_FMT_RGB8: to = YUV_TO_RGB; break;

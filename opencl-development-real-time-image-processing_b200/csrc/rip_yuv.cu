@@ -244,6 +244,22 @@ const char *yuv_format_name(int fmt)
     case RIP_FMT_BAYER_BGGR16: return "BAYER_BGGR16";
     case RIP_FMT_BAYER_GRBG16: return "BAYER_GRBG16";
     case RIP_FMT_BAYER_GBRG16: return "BAYER_GBRG16";
+    case RIP_FMT_BAYER_RGGB10P_MIPI: return "BAYER_RGGB10P_MIPI";
+    case RIP_FMT_BAYER_BGGR10P_MIPI: return "BAYER_BGGR10P_MIPI";
+    case RIP_FMT_BAYER_GRBG10P_MIPI: return "BAYER_GRBG10P_MIPI";
+    case RIP_FMT_BAYER_GBRG10P_MIPI: return "BAYER_GBRG10P_MIPI";
+    case RIP_FMT_BAYER_RGGB12P_MIPI: return "BAYER_RGGB12P_MIPI";
+    case RIP_FMT_BAYER_BGGR12P_MIPI: return "BAYER_BGGR12P_MIPI";
+    case RIP_FMT_BAYER_GRBG12P_MIPI: return "BAYER_GRBG12P_MIPI";
+    case RIP_FMT_BAYER_GBRG12P_MIPI: return "BAYER_GBRG12P_MIPI";
+    case RIP_FMT_BAYER_RGGB10P_GENICAM: return "BAYER_RGGB10P_GENICAM";
+    case RIP_FMT_BAYER_BGGR10P_GENICAM: return "BAYER_BGGR10P_GENICAM";
+    case RIP_FMT_BAYER_GRBG10P_GENICAM: return "BAYER_GRBG10P_GENICAM";
+    case RIP_FMT_BAYER_GBRG10P_GENICAM: return "BAYER_GBRG10P_GENICAM";
+    case RIP_FMT_BAYER_RGGB12P_GENICAM: return "BAYER_RGGB12P_GENICAM";
+    case RIP_FMT_BAYER_BGGR12P_GENICAM: return "BAYER_BGGR12P_GENICAM";
+    case RIP_FMT_BAYER_GRBG12P_GENICAM: return "BAYER_GRBG12P_GENICAM";
+    case RIP_FMT_BAYER_GBRG12P_GENICAM: return "BAYER_GBRG12P_GENICAM";
     default: return "(not a YUV format)";
     }
 }
@@ -252,7 +268,18 @@ int check_yuv_shape(int fmt, int W, int H)
 {
     const char *name = yuv_format_name(fmt);
     long long units;   // 2x2 blocks, pixel pairs or (Bayer) pixels of one frame
-    if (is_bayer(fmt)) {   // the demosaic's 3x3 neighbourhood
+    if (is_packed_bayer(fmt)) {   // whole bytes per row (no padding), and the demosaic's 3x3 neighbourhood
+        const int bits = bayer_bits(fmt), per = bits == 10 ? 4 : 2;   // pixels per whole number of bytes
+        if (W < 4 || W % per || H < 3) {
+            if (bayer_packing(fmt) == BAYER_GENICAM)
+                return fail(RIP_EINVAL, "%s frames need a width that is a multiple of %d and at least 4, and a height of at least 3 "
+                            "(got %d x %d): rows are W*%d/8 bytes with no padding, and a width that is not a multiple of %d "
+                            "would start rows inside a byte", name, per, W, H, bits, per);
+            return fail(RIP_EINVAL, "%s frames need a width that is a multiple of %d and at least 4, and a height of at least 3 "
+                        "(got %d x %d): rows are W*%d/8 bytes with no padding", name, per, W, H, bits);
+        }
+        units = (long long)W * H;
+    } else if (is_bayer(fmt)) {   // the demosaic's 3x3 neighbourhood
         if (W < 3 || H < 3) return fail(RIP_EINVAL, "%s frames need a width and height of at least 3 (got %d x %d)", name, W, H);
         units = (long long)W * H;
     } else if (fmt == RIP_FMT_YUYV || fmt == RIP_FMT_UYVY) {

@@ -164,7 +164,8 @@ void Controller::_appendProfile(const uint64_t prof_ns[6], std::vector<cl_ulong>
 }
 
 // bytes of one input frame in `fmt` (NV12 / NV12_COLOR / I420: the luma plane followed by chroma of half its size; YUYV /
-// UYVY: two bytes per pixel; Bayer: one byte per pixel at 8 bits, one 16-bit word at 10 to 16), 0 = bad format / shape
+// UYVY: two bytes per pixel; Bayer: one byte per pixel at 8 bits, one 16-bit word at 10 to 16, packed: W*5/4 or W*3/2 bytes
+// per row), 0 = bad format / shape
 static size_t in_frame_bytes(int fmt, int width, int height)
 {
     const size_t px = (size_t)width * height;
@@ -180,6 +181,14 @@ static size_t in_frame_bytes(int fmt, int width, int height)
     case RIP_FMT_BAYER_RGGB14: case RIP_FMT_BAYER_BGGR14: case RIP_FMT_BAYER_GRBG14: case RIP_FMT_BAYER_GBRG14:
     case RIP_FMT_BAYER_RGGB16: case RIP_FMT_BAYER_BGGR16: case RIP_FMT_BAYER_GRBG16: case RIP_FMT_BAYER_GBRG16:
         return (width < 3 || height < 3) ? 0 : px * 2;
+    case RIP_FMT_BAYER_RGGB10P_MIPI: case RIP_FMT_BAYER_BGGR10P_MIPI: case RIP_FMT_BAYER_GRBG10P_MIPI: case RIP_FMT_BAYER_GBRG10P_MIPI:
+    case RIP_FMT_BAYER_RGGB10P_GENICAM: case RIP_FMT_BAYER_BGGR10P_GENICAM: case RIP_FMT_BAYER_GRBG10P_GENICAM:
+    case RIP_FMT_BAYER_GBRG10P_GENICAM:
+        return (width < 4 || width % 4 || height < 3) ? 0 : px * 5 / 4;
+    case RIP_FMT_BAYER_RGGB12P_MIPI: case RIP_FMT_BAYER_BGGR12P_MIPI: case RIP_FMT_BAYER_GRBG12P_MIPI: case RIP_FMT_BAYER_GBRG12P_MIPI:
+    case RIP_FMT_BAYER_RGGB12P_GENICAM: case RIP_FMT_BAYER_BGGR12P_GENICAM: case RIP_FMT_BAYER_GRBG12P_GENICAM:
+    case RIP_FMT_BAYER_GBRG12P_GENICAM:
+        return (width < 4 || width % 2 || height < 3) ? 0 : px * 3 / 2;
     case RIP_FMT_RGB8: case RIP_FMT_BGR8: return px * 3;
     case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return px * 4;
     default: return 0;
@@ -199,7 +208,8 @@ static unsigned char *prepare_output(const rip_op_desc &desc, const unsigned cha
     const size_t in_frame = in_frame_bytes(desc.in_format, width, height);
     if (in_frame == 0) {
         logger.log(std::string(what) + ": unsupported input format (NV12 needs an even height, NV12_COLOR and I420 an even width and height, "
-                   "YUYV and UYVY an even width, Bayer of 8 to 16 bits a width and height of at least 3)", Logger::LogLevel::ERROR);
+                   "YUYV and UYVY an even width, Bayer of 8 to 16 bits a width and height of at least 3, packed 10- / 12-bit Bayer a "
+                   "width of at least 4 that is a multiple of 4 / 2 and a height of at least 3)", Logger::LogLevel::ERROR);
         return nullptr;
     }
     if (in_bytes != (size_t)-1 && in_bytes < in_frame * (size_t)n_frames) {

@@ -4,6 +4,7 @@ host pipeline from Bayer against RGB8 and NV12_COLOR input.
 
     python tools/bench_bayer.py [--launches 21] > profiles/bayer_b200.txt
     python tools/bench_bayer.py --raw16 [--launches 21] > profiles/bayer16_b200.txt
+    python tools/bench_bayer.py --packed [--launches 21] > profiles/bayer_packed_b200.txt
 
 --raw16 times the 10- to 16-bit formats instead (2 bytes per pixel in): the kernel legs on 32 x 3840x2160 BAYER_RGGB12 and
 BAYER_RGGB16, the demosaic's share of GAUSSIAN 5x5 on 16 x 1920x1080 BAYER_RGGB12, and the end-to-end legs from BAYER_RGGB12
@@ -14,6 +15,12 @@ Bayer frames are 265 MB in and up to 1.06 GB out, far above the 126 MB L2.  Algo
 bytes per pixel out.  The share of peak is against the 6.55 TB/s device-to-device copy peak measured on a B200 (DESIGN.md).
 The gray leg is compared, in the same run, with the two-kernel route a caller has without it: rip_convert to RGB8, then
 rip_gray on RGB8.
+--packed times the packed 10- and 12-bit formats (MIPI CSI-2 and GenICam, 1.25 or 1.5 bytes per pixel in): the kernel legs on
+32 x 3840x2160 RGGB in each layout beside the unpacked code of the same samples (BAYER_RGGB10 / 12), and the end-to-end legs
+of 16 x 1920x1080 from each layout against BAYER_RGGB12 and BAYER_RGGB8.  Kernel legs: the first, middle and last frame of
+every output against tests/bayer16_ref.py and the C oracle.  End-to-end legs: the first and last frame of every leg (packed or
+not) against the oracle, and every packed leg in full against the unpacked code on the same samples.
+
 End-to-end legs: rip_process_host from pinned host memory, wall clock over --e2e-steps blocking calls after 2 warm-up calls.
 A sample of every timed output (first, middle and last frame) is checked against tests/bayer_ref.py and the C oracle.
 """
@@ -29,6 +36,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     sys.path.insert(0, p)
 import bayer16_ref as R16  # noqa: E402
+import bayer_packed_ref as RP  # noqa: E402
 import bayer_ref as R  # noqa: E402
 import nv12_ref  # noqa: E402
 import oracle as O  # noqa: E402
@@ -40,6 +48,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--launches", type=int, default=21)
 ap.add_argument("--e2e-steps", type=int, default=10)
 ap.add_argument("--raw16", action="store_true", help="time the 10- to 16-bit formats instead of the 8-bit ones")
+ap.add_argument("--packed", action="store_true", help="time the packed 10- and 12-bit formats instead of the 8-bit ones")
 a = ap.parse_args()
 assert a.launches >= 20
 if rip.device_count() < 1:
@@ -201,10 +210,121 @@ def raw16_legs():
     print("# every sampled output equal to the reference")
 
 
+PACKED_FMT = {"mipi10": "10P_MIPI", "mipi12": "12P_MIPI", "genicam10": "10P_GENICAM", "genicam12": "12P_GENICAM"}
+
+
+def packed_frames(n, h, w, layout, seed):
+    """camera_like16 samples, packed: one frame packed, the others its rolls by 40 columns (a whole number of bytes in every
+    layout), so that 32 4K frames need no packing pass of their own.  Returns (packed, samples)."""
+    bits = RP.bits_of(layout)
+    one = camera_like16(1, h, w, bits, seed)[0]
+    p1 = RP.pack(one, layout)
+    step = RP.row_bytes(layout, 40)
+    packed = np.stack([np.roll(p1, step * i, axis=1) for i in range(n)])
+    samples = np.stack([np.roll(one, 40 * i, axis=1) for i in range(n)])
+    return packed, samples
+
+
+def packed_legs():
+    # ---- decode kernels, 32 x 4K RGGB in each layout, beside the unpacked code of the same samples ----------------------------
+    N, H, W = 32, 2160, 3840
+    px = N * H * W
+    d_out = rip.DeviceBuffer(px * 4)
+    sample = (0, N // 2, N - 1)
+    for layout in RP.LAYOUTS:
+        bits = RP.bits_of(layout)
+        packed, samples = packed_frames(N, H, W, layout, bits)
+        assert np.array_equal(RP.unpack(packed[N - 1], layout), samples[N - 1])
+        fmt, name = getattr(rip, f"FMT_BAYER_RGGB{PACKED_FMT[layout]}"), f"BAYER_RGGB{PACKED_FMT[layout]}"
+        u16, u16_name = getattr(rip, f"FMT_BAYER_RGGB{bits}"), f"BAYER_RGGB{bits}"
+        d_in = rip.DeviceBuffer(packed.nbytes).upload(packed)
+        d_u16 = rip.DeviceBuffer(samples.nbytes).upload(samples)
+        bpp_in = bits / 8
+        want_rgb = {i: R16.decode(samples[i], "rggb", bits) for i in sample}
+        want_gray = {i: O.gray(want_rgb[i], threads=0) for i in sample}
+        for order, ofmt in (("rgba", rip.FMT_RGBA8), ("rgb", rip.FMT_RGB8), ("gray", None)):
+            nb = 1 if order == "gray" else len(order)
+            res = {}
+            for f, nm, src, b_in in ((fmt, name, d_in, bpp_in), (u16, u16_name, d_u16, 2)):
+                if order == "gray":
+                    us, best = timed(lambda: rip.gray_dev(src.ptr, d_out.ptr, W, H, N, f, rip.GRAY_OUT_U8))
+                else:
+                    us, best = timed(lambda: rip.convert_dev(src.ptr, d_out.ptr, W, H, N, f, ofmt))
+                res[f] = us
+                label = "rip_gray" if order == "gray" else "rip_convert"
+                row(f"{label} {nm} -> {order.upper()}{'8' if order != 'gray' else ' u8'}, {N} x {W}x{H}", us, best, px, b_in + nb)
+                for i in sample:
+                    shape = (H, W) if order == "gray" else (H, W, nb)
+                    got = d_out.download(shape, offset=i * H * W * nb)
+                    if order == "gray":
+                        want = want_gray[i]
+                    else:
+                        want = want_rgb[i] if order == "rgb" else np.concatenate([want_rgb[i], np.full((H, W, 1), 255, np.uint8)], -1)
+                    check(f"{label} {nm} {order} frame {i}", got, want)
+            print(f"  {order}: {name} / {u16_name} time {res[fmt] / res[u16]:.2f}", flush=True)
+        d_in.free()
+        d_u16.free()
+        del packed, samples
+    d_out.free()
+
+    # ---- end to end from pinned memory, 16 x 1080p: each layout against BAYER_RGGB12 and BAYER_RGGB8 -------------------------
+    N, H, W = 16, 1080, 1920
+    px = N * H * W
+    wt = rip.gauss_weights(5, 1.0)
+    ctx = rip.Context([0])
+    # (format, name, host frames, the unpacked code and samples of the same frames or None, decoded RGB of frame i)
+    srcs = []
+    for layout in RP.LAYOUTS:
+        bits = RP.bits_of(layout)
+        packed, samples = packed_frames(N, H, W, layout, 2)
+        srcs.append((getattr(rip, f"FMT_BAYER_RGGB{PACKED_FMT[layout]}"), f"BAYER_RGGB{PACKED_FMT[layout]}", packed,
+                     (getattr(rip, f"FMT_BAYER_RGGB{bits}"), samples),
+                     lambda i, s=samples, b=bits: R16.decode(s[i], "rggb", b)))
+    raw12, raw8 = camera_like16(N, H, W, 12, 2), camera_like(N, H, W, 2)
+    srcs.append((rip.FMT_BAYER_RGGB12, "BAYER_RGGB12", raw12, None, lambda i: R16.decode(raw12[i], "rggb", 12)))
+    srcs.append((rip.FMT_BAYER_RGGB8, "BAYER_RGGB8", raw8, None, lambda i: R.decode(raw8[i], "rggb")))
+    print(f"# end to end, rip_process_host, pinned host buffers, {N} x {W}x{H}, wall clock over {a.e2e_steps} calls", flush=True)
+    for op, name, kw in ((rip.OP_GRAY, "GRAY", {}), (rip.OP_EDGE, "EDGE", {}), (rip.OP_FUSED, "FUSED 5x5", {"ksize": 5, "weights": wt})):
+        res = {}
+        for f, nm, src, ref, rgb_of in srcs:
+            h_in = rip.PinnedBuffer(src.nbytes)
+            a_in = h_in.array.view(src.dtype).reshape(src.shape)
+            a_in[...] = src
+            h_out = rip.PinnedBuffer(px)
+            a_out = h_out.array.reshape((N, H, W))
+            for _ in range(2):
+                ctx.process(a_in, op, f, out=a_out, **kw)
+            t0 = time.perf_counter()
+            for _ in range(a.e2e_steps):
+                ctx.process(a_in, op, f, out=a_out, **kw)
+            dt = (time.perf_counter() - t0) / a.e2e_steps
+            res[nm] = dt
+            print(f"  {name:10s} {nm:26s} {dt * 1e3:8.2f} ms/call  {px / dt / 1e9:6.2f} Gpx/s  "
+                  f"({src.nbytes / px:.2f} B/px in, 1 B/px out)", flush=True)
+            if ref is not None:
+                check(f"e2e {name} {nm} vs the unpacked code", a_out, ctx.process(ref[1], op, ref[0], **kw))
+            for i in (0, N - 1):
+                rgb = rgb_of(i)
+                want = O.gray(rgb, threads=0) if op == rip.OP_GRAY else \
+                    O.sobel(O.gray(rgb, threads=0), threads=0) if op == rip.OP_EDGE else O.fused(rgb, 5, weights=wt, threads=0)
+                check(f"e2e {name} {nm} frame {i} vs the oracle", a_out[i], want)
+            del a_in, a_out
+            h_in.free()
+            h_out.free()
+        for nm in [x[1] for x in srcs[:4]]:
+            print(f"  {name}: {nm} speed against BAYER_RGGB12 {res['BAYER_RGGB12'] / res[nm]:.2f}x, "
+                  f"against BAYER_RGGB8 {res['BAYER_RGGB8'] / res[nm]:.2f}x", flush=True)
+    ctx.close()
+    print("# every sampled output equal to the reference")
+
+
 print(f"# {card()}")
 print(f"# median of {a.launches} launches after 3 warm-up launches (CUDA events); copy peak {PEAK_GBS:.0f} GB/s", flush=True)
 if a.raw16:
     raw16_legs()
+    sys.exit(0)
+if a.packed:
+    packed_legs()
     sys.exit(0)
 
 # ---- decode kernels, 32 x 4K RGGB ---------------------------------------------------------------------------------------------
