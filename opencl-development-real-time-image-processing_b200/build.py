@@ -74,10 +74,10 @@ def build_host(force: bool = False, verbose: bool = False) -> str | None:
     if not srcs:
         return None
     deps = srcs + glob.glob(os.path.join(HOST, "*.hpp")) + glob.glob(os.path.join(HOST, "*.h")) + \
-        glob.glob(os.path.join(INCLUDE, "*.h"))
+        glob.glob(os.path.join(INCLUDE, "*.h")) + [os.path.join(CSRC, "rip_formats.h")]
     if force or _stale(LIB_HOST, deps) or _stale(LIB_HOST, [LIB_CUDA]):
         cmd = [_host_cxx(), "-O2", "-std=c++17", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-pthread",
-               "-I", INCLUDE, "-I", HOST, "-I", os.path.join(os.path.dirname(os.path.dirname(_nvcc())), "include"),
+               "-I", INCLUDE, "-I", HOST, "-I", CSRC, "-I", os.path.join(os.path.dirname(os.path.dirname(_nvcc())), "include"),
                "-o", LIB_HOST, *srcs,
                "-L", PKG, "-lrip_cuda", "-Wl,-rpath,$ORIGIN"]
         res = subprocess.run(cmd, capture_output=True, text=True)

@@ -96,28 +96,11 @@ static int check_device(int device)
     return RIP_OK;
 }
 
+// 0 = not a format
 static int channels_of(int fmt)
 {
-    switch (fmt) {
-    case RIP_FMT_GRAY8: case RIP_FMT_NV12: return 1;   // (NV12: the luma plane is the image)
-    case RIP_FMT_RGB8: case RIP_FMT_BGR8: return 3;
-    case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return 4;
-    default: return decodes_to_color(fmt) ? 3 : 0;   // (decoded to R, G, B; frame_bytes_of gives the bytes in)
-    }
-}
-
-// bytes from one frame of a batch to the next
-static size_t frame_bytes_of(int fmt, int width, int height)
-{
-    const size_t px = (size_t)width * height;
-    switch (fmt) {
-    case RIP_FMT_NV12: case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return px * 3 / 2;
-    case RIP_FMT_YUYV: case RIP_FMT_UYVY: return px * 2;
-    default:
-        if (is_packed_bayer(fmt)) return px * bayer_bits(fmt) / 8;   // (W is a multiple of 4 at 10 bits, of 2 at 12)
-        if (is_bayer(fmt)) return bayer_bits(fmt) == 8 ? px : px * 2;   // (10 to 16 bits: one 16-bit word per sample)
-        return px * channels_of(fmt);
-    }
+    const Format *f = format_of(fmt);
+    return f ? f->channels : 0;
 }
 
 static int load_weights(Weights &dst, int ksize, const float *weights, const char *who)
@@ -696,7 +679,7 @@ extern "C" int rip_convert(int device, rip_stream stream, const uint8_t *d_in, u
 
 static int needs_gray_first(const char *who, int fmt)
 {
-    const char *name = yuv_format_name(fmt);
+    const char *name = format_of(fmt)->name;
     return fail(RIP_EUNSUPPORTED, "%s: RIP_FMT_%s is not taken here; decode with rip_gray(..., RIP_FMT_%s, RIP_GRAY_OUT_U8) "
                 "and pass the result as RIP_FMT_GRAY8", who, name, name);
 }
@@ -849,8 +832,9 @@ namespace {
 int validate_desc(const rip_op_desc *desc, int *cn_out)
 {
     if (!desc) return fail(RIP_EINVAL, "rip_process_host: NULL descriptor");
-    const int cn = channels_of(desc->in_format);
-    if (cn == 0) return fail(RIP_EINVAL, "rip_process_host: unsupported input format %d", desc->in_format);
+    const Format *f = format_of(desc->in_format);
+    if (!f) return fail(RIP_EINVAL, "rip_process_host: unsupported input format %d", desc->in_format);
+    const int cn = f->channels;
     switch (desc->op) {
     case RIP_OP_GRAY:
         if (cn < 3) return fail(RIP_EINVAL, "GRAYSCALE needs a colour input");
@@ -858,7 +842,7 @@ int validate_desc(const rip_op_desc *desc, int *cn_out)
     case RIP_OP_EDGE:
         break;
     case RIP_OP_GAUSSIAN:
-        if (((cn != 1 && cn != 4) || desc->in_format == RIP_FMT_NV12) && !decodes_to_color(desc->in_format))
+        if (!(f->layout == LAYOUT_INTERLEAVED && (cn == 1 || cn == 4)) && !decodes_to_color(desc->in_format))
             return fail(RIP_EINVAL, "GAUSSIAN runs on GRAY8, RGBA8/BGRA8, NV12_COLOR, YUYV, UYVY, I420 or Bayer input");
         if (!desc->weights) return fail(RIP_EINVAL, "GAUSSIAN needs weights");
         break;
@@ -1135,7 +1119,7 @@ extern "C" int rip_submit(rip_ctx *ctx, const rip_op_desc *desc, const uint8_t *
     const bool banded = (flags & RIP_SUBMIT_BANDED) != 0;
     if (banded) {
         if (decodes_to_color(desc->in_format))
-            return fail(RIP_EUNSUPPORTED, "row-band mode does not take %s (it decodes whole frames only)", yuv_format_name(desc->in_format));
+            return fail(RIP_EUNSUPPORTED, "row-band mode does not take %s (it decodes whole frames only)", format_of(desc->in_format)->name);
         if (n_frames != 1) return fail(RIP_EINVAL, "row-band mode takes one frame per call (got %d)", n_frames);
         if (desc->op != RIP_OP_FUSED && desc->op != RIP_OP_EDGE) return fail(RIP_EUNSUPPORTED, "row-band mode supports FUSED and EDGE only");
     }
@@ -1149,7 +1133,7 @@ extern "C" int rip_submit(rip_ctx *ctx, const rip_op_desc *desc, const uint8_t *
         t->desc.weights = t->weights.data();
     }
     t->W = width; t->H = height; t->cn = cn;
-    t->in_frame_bytes = frame_bytes_of(desc->in_format, width, height);
+    t->in_frame_bytes = frame_bytes(*format_of(desc->in_format), width, height);   // (validate_desc checked the format)
     if (int rc = rip_out_bytes_per_frame(desc, width, height, &t->out_frame_bytes)) return rc;
     t->h_in = h_in; t->h_out = h_out;
     t->in_pinned = is_pinned(h_in);

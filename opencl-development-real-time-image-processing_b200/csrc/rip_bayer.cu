@@ -500,24 +500,16 @@ int launch_fmt(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, in
 
 }  // namespace
 
-// Every Bayer code is routed by name to the kernels of its pattern (the 8-bit code), its depth (the shift) and its packing;
-// anything else is an error, never a default pattern.
+// Every Bayer code is routed by its row to the kernels of its pattern (the 8-bit code), its depth (the shift) and its
+// packing; anything else is an error, never a default pattern.
 int launch_bayer(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, int in_format, YuvOut to)
 {
-    const int shift = bayer_bits(in_format) - 8, packing = bayer_packing(in_format);
-    switch (in_format) {
-    case RIP_FMT_BAYER_RGGB8: case RIP_FMT_BAYER_RGGB10: case RIP_FMT_BAYER_RGGB12: case RIP_FMT_BAYER_RGGB14: case RIP_FMT_BAYER_RGGB16:
-    case RIP_FMT_BAYER_RGGB10P_MIPI: case RIP_FMT_BAYER_RGGB12P_MIPI: case RIP_FMT_BAYER_RGGB10P_GENICAM: case RIP_FMT_BAYER_RGGB12P_GENICAM:
-        return launch_fmt<RIP_FMT_BAYER_RGGB8>(s, in, out, W, H, n_frames, to, shift, packing);
-    case RIP_FMT_BAYER_BGGR8: case RIP_FMT_BAYER_BGGR10: case RIP_FMT_BAYER_BGGR12: case RIP_FMT_BAYER_BGGR14: case RIP_FMT_BAYER_BGGR16:
-    case RIP_FMT_BAYER_BGGR10P_MIPI: case RIP_FMT_BAYER_BGGR12P_MIPI: case RIP_FMT_BAYER_BGGR10P_GENICAM: case RIP_FMT_BAYER_BGGR12P_GENICAM:
-        return launch_fmt<RIP_FMT_BAYER_BGGR8>(s, in, out, W, H, n_frames, to, shift, packing);
-    case RIP_FMT_BAYER_GRBG8: case RIP_FMT_BAYER_GRBG10: case RIP_FMT_BAYER_GRBG12: case RIP_FMT_BAYER_GRBG14: case RIP_FMT_BAYER_GRBG16:
-    case RIP_FMT_BAYER_GRBG10P_MIPI: case RIP_FMT_BAYER_GRBG12P_MIPI: case RIP_FMT_BAYER_GRBG10P_GENICAM: case RIP_FMT_BAYER_GRBG12P_GENICAM:
-        return launch_fmt<RIP_FMT_BAYER_GRBG8>(s, in, out, W, H, n_frames, to, shift, packing);
-    case RIP_FMT_BAYER_GBRG8: case RIP_FMT_BAYER_GBRG10: case RIP_FMT_BAYER_GBRG12: case RIP_FMT_BAYER_GBRG14: case RIP_FMT_BAYER_GBRG16:
-    case RIP_FMT_BAYER_GBRG10P_MIPI: case RIP_FMT_BAYER_GBRG12P_MIPI: case RIP_FMT_BAYER_GBRG10P_GENICAM: case RIP_FMT_BAYER_GBRG12P_GENICAM:
-        return launch_fmt<RIP_FMT_BAYER_GBRG8>(s, in, out, W, H, n_frames, to, shift, packing);
+    const Format *f = format_of(in_format);
+    switch (f ? f->pattern : -1) {
+    case 0: return launch_fmt<RIP_FMT_BAYER_RGGB8>(s, in, out, W, H, n_frames, to, f->bits - 8, f->packing);
+    case 1: return launch_fmt<RIP_FMT_BAYER_BGGR8>(s, in, out, W, H, n_frames, to, f->bits - 8, f->packing);
+    case 2: return launch_fmt<RIP_FMT_BAYER_GRBG8>(s, in, out, W, H, n_frames, to, f->bits - 8, f->packing);
+    case 3: return launch_fmt<RIP_FMT_BAYER_GBRG8>(s, in, out, W, H, n_frames, to, f->bits - 8, f->packing);
     }
     return fail(RIP_EINVAL, "Bayer decode: input format %d is not a Bayer format", in_format);
 }

@@ -75,11 +75,9 @@ bool fused_supported(int W, int H, int fmt, int ksize, const uint8_t *d_in, cons
 {
     if (ksize != 0 && ksize != 5) return false;
     if (W < 4 || (W & 3) || H < 2) return false;
-    const int cn = (fmt == RIP_FMT_RGB8 || fmt == RIP_FMT_BGR8) ? 3 : (fmt == RIP_FMT_RGBA8 || fmt == RIP_FMT_BGRA8) ? 4 :
-                   (fmt == RIP_FMT_GRAY8 || fmt == RIP_FMT_NV12) ? 1 : 0;
-    if (cn == 0) return false;
-    if (fmt == RIP_FMT_NV12 && (H & 1)) return false;
-    const uintptr_t in_align = cn == 4 ? 15u : 3u;
+    const Format *f = format_of(fmt);
+    if (!f || decodes_to_color(fmt) || !shape_ok(*f, W, H)) return false;
+    const uintptr_t in_align = f->channels == 4 ? 15u : 3u;
     if ((reinterpret_cast<uintptr_t>(d_in) & in_align) || (reinterpret_cast<uintptr_t>(d_out) & 3u)) return false;
     return true;
 }
@@ -266,10 +264,10 @@ int launch_fused(cudaStream_t s, const uint8_t *d_in, uint8_t *d_out, int W, int
             return fail(RIP_EUNSUPPORTED, "rip_fused: weights are not a non-negative symmetric separable 5x5 kernel");
         memcpy(p.w, weights25, sizeof(float) * 25);
     }
-    const int cn = (fmt == RIP_FMT_RGB8 || fmt == RIP_FMT_BGR8) ? 3 : (fmt == RIP_FMT_GRAY8 || fmt == RIP_FMT_NV12) ? 1 : 4;
+    const Format &f = *format_of(fmt);   // (fused_supported() checked the format)
     // whole NV12 frames carry their chroma plane behind the luma plane; row bands are passed as plain luma rows
-    p.in_frame_bytes = (fmt == RIP_FMT_NV12 && in_row0 == 0 && in_rows == H) ? (size_t)W * H * 3 / 2 : (size_t)in_rows * W * cn;
-    if (x2_npx(W, cn, d_in, d_out) == 8) return launch_fused_x2_n<8>(s, p, n_frames, fmt, with_blur, band, g, device);
+    p.in_frame_bytes = (in_row0 == 0 && in_rows == H) ? frame_bytes(f, W, H) : (size_t)in_rows * W * f.channels;
+    if (x2_npx(W, f.channels, d_in, d_out) == 8) return launch_fused_x2_n<8>(s, p, n_frames, fmt, with_blur, band, g, device);
     return launch_fused_x2_n<4>(s, p, n_frames, fmt, with_blur, band, g, device);
 }
 

@@ -112,9 +112,9 @@ int launch_fused_tile(cudaStream_t s, const uint8_t *d_in, uint8_t *d_out, int W
     p.src = d_in; p.dst = d_out; p.W = W; p.H = H;
     p.in_row0 = in_row0; p.in_rows = in_rows; p.out_row0 = out_row0; p.out_rows = out_rows;
     p.ksize = ksize;
-    const int cn = (fmt == RIP_FMT_RGB8 || fmt == RIP_FMT_BGR8) ? 3 : (fmt == RIP_FMT_RGBA8 || fmt == RIP_FMT_BGRA8) ? 4 : 1;
+    const Format &f = *format_of(fmt);   // (rip_fused checked the format)
     // whole NV12 frames carry their chroma plane behind the luma plane; row bands are passed as plain luma rows
-    p.in_frame_bytes = (fmt == RIP_FMT_NV12 && in_row0 == 0 && in_rows == H) ? (size_t)W * H * 3 / 2 : (size_t)in_rows * W * cn;
+    p.in_frame_bytes = (in_row0 == 0 && in_rows == H) ? frame_bytes(f, W, H) : (size_t)in_rows * W * f.channels;
     // frames ride in gridDim.z (<= 65535): batches of tiny frames go out in slabs
     for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
         const dim3 grid((W + FT_TW - 1) / FT_TW, (out_rows + FT_TH - 1) / FT_TH, min(n_frames - f0, kMaxGridZ));

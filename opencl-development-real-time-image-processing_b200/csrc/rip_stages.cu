@@ -274,9 +274,9 @@ int launch_sobel(cudaStream_t s, const uint8_t *src, uint8_t *dst, int W, int H,
                  int src_row0, int src_rows, int out_row0, int out_rows)
 {
     const dim3 block(256);
-    const int cn = fmt == RIP_FMT_RGB8 || fmt == RIP_FMT_BGR8 ? 3 : fmt == RIP_FMT_RGBA8 || fmt == RIP_FMT_BGRA8 ? 4 : 1;
+    const Format &f = *format_of(fmt);   // (rip_sobel checked the format)
     // whole NV12 frames carry their chroma plane behind the luma plane; row bands are passed as plain luma rows
-    const size_t in_frame_bytes = (fmt == RIP_FMT_NV12 && src_row0 == 0 && src_rows == H) ? (size_t)W * H * 3 / 2 : (size_t)src_rows * W * cn;
+    const size_t in_frame_bytes = (src_row0 == 0 && src_rows == H) ? frame_bytes(f, W, H) : (size_t)src_rows * W * f.channels;
     // frames ride in gridDim.z (<= 65535): batches of tiny frames go out in slabs
     for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
         const dim3 grid((W + SOB_TW - 1) / SOB_TW, (out_rows + SOB_TH - 1) / SOB_TH, min(n_frames - f0, kMaxGridZ));

@@ -217,89 +217,34 @@ int launch_fmt(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, in
 
 }  // namespace
 
-const char *yuv_format_name(int fmt)
-{
-    switch (fmt) {
-    case RIP_FMT_NV12_COLOR: return "NV12_COLOR";
-    case RIP_FMT_YUYV: return "YUYV";
-    case RIP_FMT_UYVY: return "UYVY";
-    case RIP_FMT_I420: return "I420";
-    case RIP_FMT_BAYER_RGGB8: return "BAYER_RGGB8";
-    case RIP_FMT_BAYER_BGGR8: return "BAYER_BGGR8";
-    case RIP_FMT_BAYER_GRBG8: return "BAYER_GRBG8";
-    case RIP_FMT_BAYER_GBRG8: return "BAYER_GBRG8";
-    case RIP_FMT_BAYER_RGGB10: return "BAYER_RGGB10";
-    case RIP_FMT_BAYER_BGGR10: return "BAYER_BGGR10";
-    case RIP_FMT_BAYER_GRBG10: return "BAYER_GRBG10";
-    case RIP_FMT_BAYER_GBRG10: return "BAYER_GBRG10";
-    case RIP_FMT_BAYER_RGGB12: return "BAYER_RGGB12";
-    case RIP_FMT_BAYER_BGGR12: return "BAYER_BGGR12";
-    case RIP_FMT_BAYER_GRBG12: return "BAYER_GRBG12";
-    case RIP_FMT_BAYER_GBRG12: return "BAYER_GBRG12";
-    case RIP_FMT_BAYER_RGGB14: return "BAYER_RGGB14";
-    case RIP_FMT_BAYER_BGGR14: return "BAYER_BGGR14";
-    case RIP_FMT_BAYER_GRBG14: return "BAYER_GRBG14";
-    case RIP_FMT_BAYER_GBRG14: return "BAYER_GBRG14";
-    case RIP_FMT_BAYER_RGGB16: return "BAYER_RGGB16";
-    case RIP_FMT_BAYER_BGGR16: return "BAYER_BGGR16";
-    case RIP_FMT_BAYER_GRBG16: return "BAYER_GRBG16";
-    case RIP_FMT_BAYER_GBRG16: return "BAYER_GBRG16";
-    case RIP_FMT_BAYER_RGGB10P_MIPI: return "BAYER_RGGB10P_MIPI";
-    case RIP_FMT_BAYER_BGGR10P_MIPI: return "BAYER_BGGR10P_MIPI";
-    case RIP_FMT_BAYER_GRBG10P_MIPI: return "BAYER_GRBG10P_MIPI";
-    case RIP_FMT_BAYER_GBRG10P_MIPI: return "BAYER_GBRG10P_MIPI";
-    case RIP_FMT_BAYER_RGGB12P_MIPI: return "BAYER_RGGB12P_MIPI";
-    case RIP_FMT_BAYER_BGGR12P_MIPI: return "BAYER_BGGR12P_MIPI";
-    case RIP_FMT_BAYER_GRBG12P_MIPI: return "BAYER_GRBG12P_MIPI";
-    case RIP_FMT_BAYER_GBRG12P_MIPI: return "BAYER_GBRG12P_MIPI";
-    case RIP_FMT_BAYER_RGGB10P_GENICAM: return "BAYER_RGGB10P_GENICAM";
-    case RIP_FMT_BAYER_BGGR10P_GENICAM: return "BAYER_BGGR10P_GENICAM";
-    case RIP_FMT_BAYER_GRBG10P_GENICAM: return "BAYER_GRBG10P_GENICAM";
-    case RIP_FMT_BAYER_GBRG10P_GENICAM: return "BAYER_GBRG10P_GENICAM";
-    case RIP_FMT_BAYER_RGGB12P_GENICAM: return "BAYER_RGGB12P_GENICAM";
-    case RIP_FMT_BAYER_BGGR12P_GENICAM: return "BAYER_BGGR12P_GENICAM";
-    case RIP_FMT_BAYER_GRBG12P_GENICAM: return "BAYER_GRBG12P_GENICAM";
-    case RIP_FMT_BAYER_GBRG12P_GENICAM: return "BAYER_GBRG12P_GENICAM";
-    default: return "(not a YUV format)";
-    }
-}
-
 int check_yuv_shape(int fmt, int W, int H)
 {
-    const char *name = yuv_format_name(fmt);
-    long long units;   // 2x2 blocks, pixel pairs or (Bayer) pixels of one frame
-    if (is_packed_bayer(fmt)) {   // whole bytes per row (no padding), and the demosaic's 3x3 neighbourhood
-        const int bits = bayer_bits(fmt), per = bits == 10 ? 4 : 2;   // pixels per whole number of bytes
-        if (W < 4 || W % per || H < 3) {
-            if (bayer_packing(fmt) == BAYER_GENICAM)
-                return fail(RIP_EINVAL, "%s frames need a width that is a multiple of %d and at least 4, and a height of at least 3 "
-                            "(got %d x %d): rows are W*%d/8 bytes with no padding, and a width that is not a multiple of %d "
-                            "would start rows inside a byte", name, per, W, H, bits, per);
+    if (!decodes_to_color(fmt)) return fail(RIP_EINVAL, "YUV decode: input format %d is not decoded to colour", fmt);
+    const Format &f = *format_of(fmt);
+    if (!shape_ok(f, W, H)) {
+        if (f.packing == BAYER_GENICAM)
             return fail(RIP_EINVAL, "%s frames need a width that is a multiple of %d and at least 4, and a height of at least 3 "
-                        "(got %d x %d): rows are W*%d/8 bytes with no padding", name, per, W, H, bits);
-        }
-        units = (long long)W * H;
-    } else if (is_bayer(fmt)) {   // the demosaic's 3x3 neighbourhood
-        if (W < 3 || H < 3) return fail(RIP_EINVAL, "%s frames need a width and height of at least 3 (got %d x %d)", name, W, H);
-        units = (long long)W * H;
-    } else if (fmt == RIP_FMT_YUYV || fmt == RIP_FMT_UYVY) {
-        if (W & 1) return fail(RIP_EINVAL, "%s frames need an even width (got %d x %d)", name, W, H);
-        units = (long long)H * (W / 2);
-    } else if (fmt == RIP_FMT_NV12_COLOR || fmt == RIP_FMT_I420) {
-        if ((W & 1) || (H & 1)) return fail(RIP_EINVAL, "%s frames need an even width and height (got %d x %d)", name, W, H);
-        units = (long long)(H / 2) * (W / 2);
-    } else {
-        return fail(RIP_EINVAL, "YUV decode: input format %d is not decoded to colour", fmt);
+                        "(got %d x %d): rows are W*%d/8 bytes with no padding, and a width that is not a multiple of %d "
+                        "would start rows inside a byte", f.name, f.w_mul, W, H, f.bits, f.w_mul);
+        if (f.packing == BAYER_MIPI)
+            return fail(RIP_EINVAL, "%s frames need a width that is a multiple of %d and at least 4, and a height of at least 3 "
+                        "(got %d x %d): rows are W*%d/8 bytes with no padding", f.name, f.w_mul, W, H, f.bits);
+        if (f.layout == LAYOUT_BAYER)
+            return fail(RIP_EINVAL, "%s frames need a width and height of at least 3 (got %d x %d)", f.name, W, H);
+        if (f.layout == LAYOUT_YUV422) return fail(RIP_EINVAL, "%s frames need an even width (got %d x %d)", f.name, W, H);
+        return fail(RIP_EINVAL, "%s frames need an even width and height (got %d x %d)", f.name, W, H);
     }
+    // threads of the x1 / x2 kernels per frame: one per Bayer pixel, 4:2:2 pixel pair or 4:2:0 2x2 block
+    const long long units = f.layout == LAYOUT_BAYER ? (long long)W * H : (long long)(H / f.h_mul) * (W / f.w_mul);
     if (units > 0x7fffff00ll)   // (thread indices are 32-bit)
-        return fail(RIP_EINVAL, "%s frame of %d x %d is too large", name, W, H);
+        return fail(RIP_EINVAL, "%s frame of %d x %d is too large", f.name, W, H);
     return RIP_OK;
 }
 
 int launch_yuv(cudaStream_t s, const uint8_t *in, uint8_t *out, int W, int H, int n_frames, int in_format, YuvOut to)
 {
     if (int rc = check_yuv_shape(in_format, W, H)) return rc;
-    if (is_bayer(in_format)) return launch_bayer(s, in, out, W, H, n_frames, in_format, to);
+    if (format_of(in_format)->layout == LAYOUT_BAYER) return launch_bayer(s, in, out, W, H, n_frames, in_format, to);
     switch (in_format) {
     case RIP_FMT_NV12_COLOR: return launch_fmt<RIP_FMT_NV12_COLOR>(s, in, out, W, H, n_frames, to);
     case RIP_FMT_I420: return launch_fmt<RIP_FMT_I420>(s, in, out, W, H, n_frames, to);

@@ -9,6 +9,8 @@
 #include <cstring>
 #include <iostream>
 
+#include "rip_formats.h"
+
 namespace {
 
 rip_platform_rec g_platform{0};
@@ -163,36 +165,11 @@ void Controller::_appendProfile(const uint64_t prof_ns[6], std::vector<cl_ulong>
     for (int i = 0; i < 6; i++) profiling_events->push_back(prof_ns[i]);
 }
 
-// bytes of one input frame in `fmt` (NV12 / NV12_COLOR / I420: the luma plane followed by chroma of half its size; YUYV /
-// UYVY: two bytes per pixel; Bayer: one byte per pixel at 8 bits, one 16-bit word at 10 to 16, packed: W*5/4 or W*3/2 bytes
-// per row), 0 = bad format / shape
+// bytes of one input frame in `fmt` (its row in rip_formats.h), 0 = bad format / shape
 static size_t in_frame_bytes(int fmt, int width, int height)
 {
-    const size_t px = (size_t)width * height;
-    switch (fmt) {
-    case RIP_FMT_GRAY8: return px;
-    case RIP_FMT_NV12: return (height & 1) ? 0 : px * 3 / 2;
-    case RIP_FMT_NV12_COLOR: case RIP_FMT_I420: return ((width | height) & 1) ? 0 : px * 3 / 2;
-    case RIP_FMT_YUYV: case RIP_FMT_UYVY: return (width & 1) ? 0 : px * 2;
-    case RIP_FMT_BAYER_RGGB8: case RIP_FMT_BAYER_BGGR8: case RIP_FMT_BAYER_GRBG8: case RIP_FMT_BAYER_GBRG8:
-        return (width < 3 || height < 3) ? 0 : px;
-    case RIP_FMT_BAYER_RGGB10: case RIP_FMT_BAYER_BGGR10: case RIP_FMT_BAYER_GRBG10: case RIP_FMT_BAYER_GBRG10:
-    case RIP_FMT_BAYER_RGGB12: case RIP_FMT_BAYER_BGGR12: case RIP_FMT_BAYER_GRBG12: case RIP_FMT_BAYER_GBRG12:
-    case RIP_FMT_BAYER_RGGB14: case RIP_FMT_BAYER_BGGR14: case RIP_FMT_BAYER_GRBG14: case RIP_FMT_BAYER_GBRG14:
-    case RIP_FMT_BAYER_RGGB16: case RIP_FMT_BAYER_BGGR16: case RIP_FMT_BAYER_GRBG16: case RIP_FMT_BAYER_GBRG16:
-        return (width < 3 || height < 3) ? 0 : px * 2;
-    case RIP_FMT_BAYER_RGGB10P_MIPI: case RIP_FMT_BAYER_BGGR10P_MIPI: case RIP_FMT_BAYER_GRBG10P_MIPI: case RIP_FMT_BAYER_GBRG10P_MIPI:
-    case RIP_FMT_BAYER_RGGB10P_GENICAM: case RIP_FMT_BAYER_BGGR10P_GENICAM: case RIP_FMT_BAYER_GRBG10P_GENICAM:
-    case RIP_FMT_BAYER_GBRG10P_GENICAM:
-        return (width < 4 || width % 4 || height < 3) ? 0 : px * 5 / 4;
-    case RIP_FMT_BAYER_RGGB12P_MIPI: case RIP_FMT_BAYER_BGGR12P_MIPI: case RIP_FMT_BAYER_GRBG12P_MIPI: case RIP_FMT_BAYER_GBRG12P_MIPI:
-    case RIP_FMT_BAYER_RGGB12P_GENICAM: case RIP_FMT_BAYER_BGGR12P_GENICAM: case RIP_FMT_BAYER_GRBG12P_GENICAM:
-    case RIP_FMT_BAYER_GBRG12P_GENICAM:
-        return (width < 4 || width % 2 || height < 3) ? 0 : px * 3 / 2;
-    case RIP_FMT_RGB8: case RIP_FMT_BGR8: return px * 3;
-    case RIP_FMT_RGBA8: case RIP_FMT_BGRA8: return px * 4;
-    default: return 0;
-    }
+    const rip::Format *f = rip::format_of(fmt);
+    return f && rip::shape_ok(*f, width, height) ? rip::frame_bytes(*f, width, height) : 0;
 }
 
 // Validates the shapes and sizes the result container: resized in place (no zero-filled temporary per call), unless it
